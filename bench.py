@@ -62,12 +62,30 @@ def parse_args():
     ap.add_argument("--e2e-depth", type=int, default=1, help="batches in flight in the end-to-end measurement (JxlB200DecodeBatchSubmit / Wait); 1 = synchronous calls")
     ap.add_argument("--cpu-sample", type=int, default=2, help="images in the bounded CPU-baseline sample")
     ap.add_argument("--no-mixed", action="store_true", help="skip the second (variable-block) workload")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the pixels decoded in the last timed step of each timed path to DIR/<path>.npy "
+                    "(float32, one row per file of the step, the same seeded byte positions of every image; DIR/sample_index.npy holds them)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def describe(args, world):
     per = "%d files per step sharded over %d rank(s)" % (args.batch, world) if args.scaling == "strong" else "%d files per step per GPU" % args.batch
     return "batch of synthetic %dx%d RGB8 files, %s (%d distinct images repeated), decoded to interleaved RGB8, no collective; " % (args.width, args.height, per, args.distinct)
+
+
+DUMP_PATHS = 3                   # timed paths dumped: dct8 device, dct8 e2e, mixed device
+DUMP_BYTES = 48 << 20            # the samples of every path plus their index: the dump stays under 64 MB with the .npy headers
+
+
+def dump_sample_index(n_bytes, n_files):
+    """Byte offsets sampled from every decoded image: one seeded offset in each of K equal stripes of the image, K sized so that the
+    samples of every path over the whole job's files (float32) and the index itself (float64) fit DUMP_BYTES. Depends only on the arguments."""
+    import numpy as np
+    k = max(1, min(n_bytes, DUMP_BYTES // (4 * DUMP_PATHS * n_files + 8)))
+    stripe = n_bytes // k
+    return np.arange(k, dtype=np.int64) * stripe + np.random.default_rng(0).integers(0, stripe, k)
 
 
 # ------------------------------------------------------------------------------------------------ input files (CPU, deterministic)
@@ -244,7 +262,8 @@ def main():
         raise SystemExit("bench.py needs a GPU: " + why)
     B = len(mine)
     out_bytes_one = W * H * 3
-    total_mp_step = (args.batch if args.scaling == "strong" else args.batch * world) * W * H / 1e6
+    files_per_step = args.batch if args.scaling == "strong" else args.batch * world
+    total_mp_step = files_per_step * W * H / 1e6
     dev_out = [torch.empty(out_bytes_one, dtype=torch.uint8, device="cuda") for _ in range(B)]
     # --e2e-depth N > 1: the end-to-end steps are submitted asynchronously with N batches in flight, each writing its own set of host buffers
     # (measured in r02: two batches in flight are SLOWER than synchronous calls, 378 vs 260 ms per step — profiles/r02_e2e_pipeline.md)
@@ -257,6 +276,7 @@ def main():
         host_pinned = False
     host_out_sets = [[t.numpy() for t in host_out[k * B:(k + 1) * B]] for k in range(E2E_DEPTH)]
     host_out_np = host_out_sets[0]
+    dump_index = dump_sample_index(out_bytes_one, files_per_step) if args.dump_outputs else None
 
     def barrier():
         torch.cuda.synchronize()
@@ -314,6 +334,9 @@ def main():
         launches = P.kernel_launch_count() - launches0
         clocks = sampler.stop()
         r = {"files": files, "ms_dev": ms_dev, "launches": launches, "clocks": clocks, "comp_bytes": sum(len(f) for f in files), "value": total_mp_step * steps / (ms_dev / 1e3)}
+        if dump_index is not None:   # dev_out is reused by the next workload: sample it now, outside the timed region
+            idx = torch.from_numpy(dump_index).cuda()
+            r["dump_device"] = torch.stack([t[idx] for t in dev_out]).float().cpu().numpy()
         if with_host:
             for _ in range(max(1, warmup // 2)):
                 step_host()
@@ -321,6 +344,8 @@ def main():
             r["ms_host"] = timed(step_host, steps, drain_host)
             r["last_host_set"] = (submitted[0] - 1) % E2E_DEPTH
             r["e2e"] = total_mp_step * steps / (r["ms_host"] / 1e3)
+            if dump_index is not None:
+                r["dump_e2e"] = np.stack([o[dump_index] for o in host_out_sets[r["last_host_set"]]]).astype(np.float32)
         return r
 
     head = measure("dct8", args.steps, args.warmup, True)
@@ -344,7 +369,17 @@ def main():
             verified, max_err = None, "unavailable: %s" % e
     mixed = None
     if not args.no_mixed:
-        mixed = measure("mixed", max(2, args.steps // 2), 2, False)
+        mixed = measure("mixed", args.steps, 2, False)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        suffix = ".rank%d" % rank if world > 1 else ""
+        dumps = {"dct8_device": head["dump_device"], "dct8_e2e": head["dump_e2e"]}
+        if mixed is not None:
+            dumps["mixed_device"] = mixed["dump_device"]
+        for name, arr in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + suffix + ".npy"), arr)
+        if rank == 0:
+            np.save(os.path.join(args.dump_outputs, "sample_index.npy"), dump_index.astype(np.float64))
 
     launches = head["launches"]
     if dist is not None:
@@ -369,7 +404,7 @@ def main():
     line["e2e"]["h2d_bytes_per_step"], line["e2e"]["d2h_bytes_per_step"] = int(tb[0].item()), int(tb[1].item())
     if mixed is not None:
         line["workloads"] = {"dct8": {"value": head["value"], "bpp": 8.0 * comp_bytes / (B * W * H), "what": WORKLOADS["dct8"]["label"]},
-                             "mixed": {"value": mixed["value"], "bpp": 8.0 * mixed["comp_bytes"] / (B * W * H), "ms_per_step": mixed["ms_dev"] / max(2, args.steps // 2),
+                             "mixed": {"value": mixed["value"], "bpp": 8.0 * mixed["comp_bytes"] / (B * W * H), "ms_per_step": mixed["ms_dev"] / args.steps,
                                        "ratio_to_dct8": mixed["value"] / head["value"], "what": WORKLOADS["mixed"]["label"], "block_mix": BLOCK_MIX.get("mixed")}}
         line["workloads"]["dct8"]["block_mix"] = BLOCK_MIX.get("dct8")
 
