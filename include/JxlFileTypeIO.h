@@ -170,8 +170,18 @@ JXLFT_API EncoderStatus JXLFT_CALL JxlB200AssembleBands(uint32_t width, uint32_t
 
 /* Instrumentation for bench.py / tests: per-stage device times (ms) of the last single-image decode on this thread
  * (h2d, lf, ac, recon, filters, output, d2h, total), number of kernels launched by this process, and raw stage dumps of
- * one decode for parity tests (which: 0 = planes in the XYB buffer, 1 = planes in the ping-pong buffer, 3 = LF planes;
- * 4 = int16 coefficients as floats). Returns the element count written (<= capacity) or 0. */
+ * one VarDCT decode for parity tests. Each call decodes the whole file, then copies one buffer out as floats:
+ *   which = 4: the quantised AC coefficients, [group][channel X, Y, B][65536] (int16 values), cell-chunked: coefficient k of the
+ *              cell (by, bx) of a group at ((by * 32 + bx) * 64 + k), a varblock's storage position p in its (p / 64)-th covered cell
+ *              in raster order; cells outside the image are zero. Two-pass files hold the sum of both passes.
+ *   which = 3: the LF planes the reconstruction reads, [3][yblocks][xblocks], after dequantisation, chroma-from-luma and adaptive
+ *              LF smoothing (unsmoothed when the frame skips it or has at most 2 block rows or columns).
+ *   which = 0: the XYB buffer, [3][ypad][xpad] (padded to whole 8x8 blocks). It holds the reconstruction (dequantisation, CfL, LLF
+ *              and inverse transforms, before gaborish and EPF) whenever the fused render ran or the frame has no restoration filter;
+ *              with JXLB200_UNFUSED set and a filter on, the unfused filter kernels leave filtered planes in it.
+ *   which = 1: the second plane buffer (filter ping-pong and large-transform scratch): contents depend on the path taken.
+ * dims2 receives (xpad, ypad) for which = 0 and 1. Returns the element count written (<= capacity), or 0 when the file is not
+ * VarDCT, the decode failed or the buffer is too small. */
 JXLFT_API void JXLFT_CALL JxlB200LastStageTimes(float* ms8);
 JXLFT_API int64_t JXLFT_CALL JxlB200KernelLaunchCount(void);
 JXLFT_API int64_t JXLFT_CALL JxlB200DebugDecodeStage(const uint8_t* data, size_t dataSize, int32_t which, float* out, int64_t capacity, int32_t* dims2, ErrorInfo* errorInfo);

@@ -28,7 +28,7 @@ def all_deps():
     deps = []
     for root, _, files in os.walk(CSRC):
         for f in files:
-            if f.endswith((".cu", ".cuh", ".h", ".cc")):
+            if f.endswith((".cu", ".cuh", ".h", ".cc", ".inc")):   # .inc: generated tables (dev/idct_tables.inc)
                 deps.append(os.path.join(root, f))
     deps.append(os.path.join(os.path.dirname(HERE), "include", "JxlFileTypeIO.h"))
     return deps

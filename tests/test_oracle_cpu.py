@@ -31,13 +31,16 @@ def test_golden_files_are_what_the_encoder_still_produces(oracle):
         assert oracle.encode(img, **m["encode"]) == open(os.path.join(GOLDEN, name + ".jxl"), "rb").read()
 
 
-@pytest.mark.parametrize("strategy", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 18, 19, 20, 21])
+# covered 8x8 cells (rows, columns) per AC strategy; 14-17 (AFV) are not supported
+COVERED_Y = [1, 1, 1, 1, 2, 4, 2, 1, 4, 1, 4, 2, 1, 1, 1, 1, 1, 1, 8, 8, 4, 16, 16, 8, 32, 32, 16]
+COVERED_X = [1, 1, 1, 1, 2, 4, 1, 2, 1, 4, 2, 4, 1, 1, 1, 1, 1, 1, 8, 4, 8, 16, 8, 16, 32, 16, 32]
+PLAIN_DCTS = [0, 4, 5, 6, 7, 8, 9, 10, 11, 18, 19, 20, 21, 22, 23, 24, 25, 26]
+
+
+@pytest.mark.parametrize("strategy", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 18, 19, 20, 21, 22, 23, 24, 25, 26])
 def test_transforms_invert_and_match_fp64_dct(oracle, strategy):
-    import ctypes as C
     L = oracle.lib()
-    cy = [1, 1, 1, 1, 2, 4, 2, 1, 4, 1, 4, 2, 1, 1, 1, 1, 1, 1, 8, 8, 4, 16][strategy]
-    cx = [1, 1, 1, 1, 2, 4, 1, 2, 1, 4, 2, 4, 1, 1, 1, 1, 1, 1, 8, 4, 8, 16][strategy]
-    H, W = cy * 8, cx * 8
+    H, W = COVERED_Y[strategy] * 8, COVERED_X[strategy] * 8
     rng = np.random.default_rng(strategy)
     px = rng.standard_normal((H, W)).astype(np.float32)
     coef = np.zeros(H * W, np.float32)
@@ -45,15 +48,46 @@ def test_transforms_invert_and_match_fp64_dct(oracle, strategy):
     L.jxlo_transform_from_pixels(strategy, px.ctypes.data, W, coef.ctypes.data)
     L.jxlo_transform_to_pixels(strategy, coef.ctypes.data, back.ctypes.data, W)
     assert np.max(np.abs(back - px)) < 2e-5
-    if strategy in (0, 4, 5, 18, 21):   # square plain DCTs: compare with the textbook fp64 DCT-II scaled by 1/N per dimension
+    if strategy in PLAIN_DCTS:   # separable textbook fp64 DCT-II scaled by 1/N per dimension
         def dct_mat(n):
             k, i = np.meshgrid(np.arange(n), np.arange(n), indexing="ij")
             m = np.cos((2 * i + 1) * k * np.pi / (2 * n)) * np.where(k == 0, 1.0, np.sqrt(2.0))
             return m / n
         F = dct_mat(H) @ px.astype(np.float64) @ dct_mat(W).T      # F[vf][hf]
-        S = coef.reshape(W, H)                                      # square blocks are stored transposed: S[hf][vf]
-        assert np.max(np.abs(S.T - F)) < 1e-5
+        # SURVEY A.9 storage: min(H, W) rows of max(H, W) coefficients, the longer side horizontal. A block at least as tall as wide
+        # (square ones included) is stored transposed, S[hf][vf]; a wide one as it is, S[vf][hf].
+        if H >= W:
+            S = coef.reshape(W, H).T
+        else:
+            S = coef.reshape(H, W)
+        assert np.max(np.abs(S - F)) < 2e-6 * max(1.0, np.abs(F).max())
         assert abs(S[0, 0] - px.mean()) < 1e-6                      # DC = block mean (A.9 scaling)
+        # the inverse is the fp64 DCT-III of the same coefficients
+        Fi = rng.standard_normal((H, W)) * np.exp(-np.add.outer(np.arange(H) / H, np.arange(W) / W) * 4)
+        stored = (Fi.T if H >= W else Fi).astype(np.float32).reshape(-1)
+        L.jxlo_transform_to_pixels(strategy, stored.ctypes.data, back.ctypes.data, W)
+        want = np.linalg.solve(dct_mat(H), np.linalg.solve(dct_mat(W), Fi.astype(np.float32).astype(np.float64).T).T)
+        assert np.max(np.abs(back - want)) < 1e-5 * max(1.0, np.abs(want).max())
+
+
+def test_gaborish_stage_matches_fp64_convolution(oracle):
+    """SURVEY A.10 gaborish in float64 (default weights w1 = 0.115169525, w2 = 0.061248592 for every channel, 3x3 kernel
+    [w2 w1 w2; w1 1 w1; w2 w1 w2] / (1 + 4 w1 + 4 w2), edges mirrored at the image size, not at the padded size) on the oracle's
+    reconstruction reproduces the oracle's gaborish stage inside the image."""
+    w, h = 203, 141                                                  # neither a multiple of 8: the planes carry padding
+    data = oracle.encode(oracle.synthetic_image(w, h, seed=4), effort=7, gab=1, epf=0)
+    d = oracle.decode(data, keep_stages=True)
+    idct = d.stages["idct"].reshape(3, d.ypad, d.xpad).astype(np.float64)[:, :h, :w]
+    gab = d.stages["gab"].reshape(3, d.ypad, d.xpad)[:, :h, :w]
+    w1, w2 = 0.115169525, 0.061248592
+    norm = 1 + 4 * w1 + 4 * w2
+    p = np.pad(idct, ((0, 0), (1, 1), (1, 1)), mode="symmetric")    # x[-1] = x[0], x[n] = x[n - 1]
+    def at(dy, dx):
+        return p[:, 1 + dy:1 + dy + h, 1 + dx:1 + dx + w]
+    want = (at(0, 0) + w1 * (at(-1, 0) + at(1, 0) + at(0, -1) + at(0, 1)) + w2 * (at(-1, -1) + at(-1, 1) + at(1, -1) + at(1, 1))) / norm
+    err = np.abs(gab - want).max(axis=(1, 2)) / np.abs(want).max(axis=(1, 2))
+    assert np.all(err < 1e-6), err                                   # fp32 rounding of the weights and the sums
+    assert np.abs(gab - idct).max() > 1e-3                           # the filter did something
 
 
 def test_resample_scale_closed_form(oracle):
