@@ -177,10 +177,8 @@ JXLFT_API EncoderStatus JXLFT_CALL JxlB200AssembleBands(uint32_t width, uint32_t
  *   which = 3: the LF planes the reconstruction reads, [3][yblocks][xblocks], after dequantisation, chroma-from-luma and adaptive
  *              LF smoothing (unsmoothed when the frame skips it or has at most 2 block rows or columns).
  *   which = 0: the XYB buffer, [3][ypad][xpad] (padded to whole 8x8 blocks). It holds the reconstruction (dequantisation, CfL, LLF
- *              and inverse transforms, before gaborish and EPF) whenever the fused render ran or the frame has no restoration filter;
- *              with JXLB200_UNFUSED set and a filter on, the unfused filter kernels leave filtered planes in it.
- *   which = 1: the second plane buffer (filter ping-pong and large-transform scratch): contents depend on the path taken.
- * dims2 receives (xpad, ypad) for which = 0 and 1. Returns the element count written (<= capacity), or 0 when the file is not
+ *              and inverse transforms, before gaborish and EPF).
+ * dims2 receives (xpad, ypad) for which = 0. Returns the element count written (<= capacity), or 0 when the file is not
  * VarDCT, the decode failed or the buffer is too small. */
 JXLFT_API void JXLFT_CALL JxlB200LastStageTimes(float* ms8);
 JXLFT_API int64_t JXLFT_CALL JxlB200KernelLaunchCount(void);

@@ -222,6 +222,9 @@ static std::vector<cudaStream_t>& ShardStreams(int device, int slot, int want) {
 // lock-step, so every copy waits for the tiles phase at the end (r02: 267 ms per step = ~100 ms until the first image is rendered + 167 ms of
 // copies). Starting the images at the rate the link can take them away turns the batch into a rolling pipeline: copies run from the first
 // finished image on, beside the entropy phases of the images started later. One pacer per device, shared by every batch in flight on it.
+// The rate images are started at: somewhat above the 55.6 GB/s the link was measured to deliver (the sweep in profiles/r02_e2e_pipeline.md);
+// the in-flight cap gives the back-pressure.
+static const double kPaceGBps = 80.0;
 static std::atomic<int64_t> g_pace_next_ns[64];
 static int64_t SteadyNs() { return std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 static int64_t PaceReserve(int dev, int64_t step_ns) {   // -> earliest start time of the caller's next bundle
@@ -320,13 +323,9 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
       return progressed;
     };
     bool reserved = reserve_sets == 0;
-    // pacing (host outputs only): ns per image = its output bytes over a rate somewhat above the link's (JXLB200_D2H_GBPS, default 80 against the
-    // 55.6 GB/s measured: the sweep in profiles/r02_e2e_pipeline.md; the in-flight cap gives the back-pressure); JXLB200_PACE=0 switches it off
+    // pacing (host outputs only): ns per image = its output bytes over kPaceGBps
     int64_t pace_ns = 0, launch_at = 0;
-    if (a.hostOutputs && a.count >= 64) {
-      const char* off = getenv("JXLB200_PACE"); const double gbps = getenv("JXLB200_D2H_GBPS") ? atof(getenv("JXLB200_D2H_GBPS")) : 80.0;
-      if (!(off && *off == '0') && gbps > 0) pace_ns = int64_t(double(a.outputBytes[begin]) / gbps);
-    }
+    if (a.hostOutputs && a.count >= 64) pace_ns = int64_t(double(a.outputBytes[begin]) / kPaceGBps);
     while (done < count) {
       double t0 = now(); bool progressed = advance(); t_ret += now() - t0;
       if (pace_ns && next < count && !free_streams.empty() && launch_at == 0) launch_at = PaceReserve(cur_dev, pace_ns * std::min(bundle_size, count - next));
@@ -392,14 +391,11 @@ JxlB200Batch* JxlB200DecodeBatchSubmit(int32_t device, int32_t count, const uint
     // AC sections per warp: more lanes = fewer resident warps and instructions per section, but a longer walk (16 / 24 / 31 / 41 ms for
     // 1 / 4 / 8 / 16 lanes on a 12 MP image). Large batches are bound by issue slots and take 16; small ones (a rank's share of a
     // sharded batch) are bound by the walk itself and take just enough lanes to keep every section resident at once.
-    const int env_lanes = getenv("JXLB200_BATCH_LANES") ? atoi(getenv("JXLB200_BATCH_LANES")) : 0;
-    const int batch_lanes = env_lanes > 0 ? env_lanes : nstreams < 8 ? 1 : count >= 192 ? 16 : count >= 96 ? 8 : count >= 48 ? 4 : count >= 24 ? 2 : 1;
-    const int env_bundle = getenv("JXLB200_BUNDLE") ? atoi(getenv("JXLB200_BUNDLE")) : 0;
-    const int bundle_size = std::max(1, std::min(env_bundle > 0 ? env_bundle : ((count > nstreams && nstreams >= 32) ? 2 : 1), kMaxBundle));   // images per stream / per entropy launch: only when the batch has more images than streams
+    const int batch_lanes = nstreams < 8 ? 1 : count >= 192 ? 16 : count >= 96 ? 8 : count >= 48 ? 4 : count >= 24 ? 2 : 1;
+    const int bundle_size = std::max(1, std::min((count > nstreams && nstreams >= 32) ? 2 : 1, kMaxBundle));   // images per stream / per entropy launch: only when the batch has more images than streams
     // Host threads: the per-image enqueue work is split over `shards` threads, each with its own share of the streams.
-    const int env_threads = getenv("JXLB200_HOST_THREADS") ? atoi(getenv("JXLB200_HOST_THREADS")) : 0;   // read per call (cheap): lets a caller tune it between batches
     int hw = int(std::thread::hardware_concurrency()); if (hw <= 0) hw = 4;
-    int shards = env_threads > 0 ? env_threads : std::min(4, std::max(1, hw / 2));
+    int shards = std::min(4, std::max(1, hw / 2));
     shards = std::max(1, std::min(std::min(shards, nstreams / 8), count / 16));   // small batches keep a single enqueue thread
     b->args = BatchArgs{device, count, b->datas.data(), b->sizes.data(), b->outputs.data(), b->out_bytes.data(), bgra, hostInputs, hostOutputs, b->statuses.data()};
     b->results.resize(size_t(shards));

@@ -428,7 +428,7 @@ void DecodeJob::Setup(const DecodeRequest& req) {
   toc = ReadToc(br, fh); frame_off = pos + br.pos / 8; JXLG_CHECK(frame_off + toc.total <= cs.size(), "JxlDecoderProcessInput needs more input, but it already received the entire image.");
   info.frame_name = fh.name; info.bpp = double(cs.size()) * 8.0 / (double(m.xsize) * m.ysize);
   memset(&h, 0, sizeof(h)); bgra = req.bgra; device_output = req.device_output;
-  { int l = req.ac_lanes; const int env_lanes = getenv("JXLB200_AC_LANES") ? atoi(getenv("JXLB200_AC_LANES")) : 0; if (env_lanes > 0) l = env_lanes; ac_lanes = 1; while (ac_lanes * 2 <= l && ac_lanes < 32) ac_lanes *= 2; }
+  ac_lanes = 1; while (ac_lanes * 2 <= req.ac_lanes && ac_lanes < 32) ac_lanes *= 2;
   h.xsize = fh.xsize; h.ysize = fh.ysize; h.xb = fh.xblocks; h.yb = fh.yblocks; h.xpad = h.xb * 8; h.ypad = h.yb * 8; h.xt = (h.xb + 7) / 8; h.yt = (h.yb + 7) / 8; h.xgroups = fh.xgroups; h.ygroups = fh.ygroups; h.num_groups = fh.num_groups;
   h.xlfgroups = fh.xlfgroups; h.ylfgroups = fh.ylfgroups; h.num_lf_groups = fh.num_lf_groups; h.group_dim = fh.group_dim; h.num_passes = fh.passes.num_passes; h.encoding = fh.encoding; h.flags = uint32_t(fh.flags);
   info.group_dim = h.group_dim; info.num_group_rows = h.ygroups;
@@ -544,8 +544,7 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
     { static std::atomic<uint32_t> lf_cursor{0}, ac_cursor{0};   // concurrent images start their few long-running CTAs on different SMs
       h.lf_cta_offset = lf_cursor.fetch_add(h.num_lf_groups) % 148u; h.ac_cta_offset = vardct ? ac_cursor.fetch_add(uint32_t(AcCtas(h, ac_lanes))) % 148u : 0; }
     // + the transposed alias table of the speculative LF loop (32 slots x 8 bytes per alias entry), when it stays small
-    { static const bool no_spec = getenv("JXLB200_NO_SPEC") != nullptr;   // A/B switch: without room for the transposed alias table the kernels take the one-lane loop
-      const uint32_t spec = has_tree && !h.mod_code.use_prefix && !no_spec ? (256u << h.mod_code.log_alpha) : 0u; const uint32_t copies = h.num_mod_channels > h.first_group_channel ? 4u : 1u;   // k_mod_group: one table per warp, 4 warps per CTA
+    { const uint32_t spec = has_tree && !h.mod_code.use_prefix ? (256u << h.mod_code.log_alpha) : 0u; const uint32_t copies = h.num_mod_channels > h.first_group_channel ? 4u : 1u;   // k_mod_group: one table per warp, 4 warps per CTA
       h.lf_smem = std::min<uint32_t>(modb + 64 + (spec * copies <= 64 * 1024 ? spec * copies + 64 : (spec <= 64 * 1024 ? spec + 16 : 0)), 96 * 1024); } ac_budget = [this, code_bytes]() { uint32_t acb = 0; bool prefix = false; for (uint32_t p = 0; p < h.num_passes; p++) { acb = std::max(acb, code_bytes(h.ac_code[p])); prefix |= h.ac_code[p].use_prefix != 0; }
       for (uint32_t p = 0; p < h.num_passes; p++) prefix |= h.ac_code[p].lz77 != 0;   // LZ77 streams take the generic reader too
       h.ac_smem = acb + 64; h.ac_fast = (!prefix && h.ac_smem <= 96 * 1024) ? 1 : 0; if (!h.ac_fast) h.ac_smem = 0; };
@@ -615,24 +614,14 @@ void DecodeJob::RunAc() {
 // Phase 3: dequant + IDCT, restoration filters, colour transform, pack, and the copy back to the host.
 void DecodeJob::RunRender() {
   const bool vardct = h.encoding == 0; const DFrame* d = d_frame.as<DFrame>(); double tt = NowMs();
-  static const bool unfused_env = getenv("JXLB200_UNFUSED") != nullptr; const bool unfused = unfused_env && !h.band_on;   // the unfused filter kernels walk the whole frame: not for band buffers
   if (vardct && !d_xyb_tmp.p) {   // phased job: the LF phase has drained, its flag word is already in host memory
     const bool big_blocks = h_err.as<volatile uint32_t>()[12] != 0;   // written by k_lf_group straight into this page-locked word
-    const bool filters = h.lpf.gab || h.lpf.epf_iters;
-    if (big_blocks || (filters && unfused)) { d_xyb_tmp.Alloc(size_t(h.xpad) * h.ypad * 3 * 4); h.xyb_tmp = d_xyb_tmp.as<float>() - xyb_row_shift; UploadFrame(); }
+    if (big_blocks) { d_xyb_tmp.Alloc(size_t(h.xpad) * h.ypad * 3 * 4); h.xyb_tmp = d_xyb_tmp.as<float>() - xyb_row_shift; UploadFrame(); }
   }
-#ifdef JXLB200_DEBUG   // timing experiments only (never in release builds: skipped stages leave invalid pixels): 1 = no reconstruction, 2 = no render, 3 = neither
-  static const int dbg_skip = getenv("JXLB200_DEBUG_SKIP") ? atoi(getenv("JXLB200_DEBUG_SKIP")) : 0;
-#else
-  const int dbg_skip = 0;
-#endif
-  if (vardct && !(dbg_skip & 1)) LaunchReconstruct(d, h, stream);
+  if (vardct) LaunchReconstruct(d, h, stream);
   if (timed) cudaEventRecord(ev[3], stream);
-  bool fused = false;
   if (h.num_ops) LaunchInverseRct(d, h, ops_host.data(), stream);
-  if (dbg_skip & 2) fused = true; else
-  if (vardct && !unfused) fused = LaunchFusedRender(d, h, stream);   // gaborish + EPF + colour + pack in one kernel
-  if (vardct && !fused) LaunchFilters(d, h, stream);
+  const bool fused = vardct && LaunchFusedRender(d, h, stream);   // gaborish + EPF + colour + pack in one kernel
   if (timed) cudaEventRecord(ev[4], stream);
   if (!fused) LaunchOutput(d, h, stream);
   if (timed) cudaEventRecord(ev[5], stream);
@@ -806,7 +795,7 @@ DecodeResult DecodeOnGpu(const DecodeRequest& req) {
 bool DecodeDebugPlanes(const std::shared_ptr<DecodeJob>& job, int which, std::vector<float>* out, int* xpad, int* ypad) {
   if (!job || job->h.encoding != 0) return false; size_t px = size_t(job->h.xpad) * job->h.ypad; *xpad = int(job->h.xpad); *ypad = int(job->h.ypad);
   const float* src = nullptr; size_t n = px * 3;
-  if (which == 0) src = job->h.xyb; else if (which == 1) src = job->h.xyb_tmp; else if (which == 3) { src = job->h.lf_src; n = size_t(job->h.xb) * job->h.yb * 3; } else return false;
+  if (which == 0) src = job->h.xyb; else if (which == 3) { src = job->h.lf_src; n = size_t(job->h.xb) * job->h.yb * 3; } else return false;
   out->resize(n); return cudaMemcpy(out->data(), src, n * 4, cudaMemcpyDeviceToHost) == cudaSuccess;
 }
 bool DecodeDebugCoeffs(const std::shared_ptr<DecodeJob>& job, std::vector<int16_t>* out) {

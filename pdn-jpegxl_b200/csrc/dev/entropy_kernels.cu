@@ -509,7 +509,7 @@ void LaunchAcGroupsMulti(const DFrameSet& set, int lanes, cudaStream_t st) {   /
   EnsureSmemAttr(); uint32_t smem = 0; for (uint32_t i = 0; i < set.n; i++) smem = std::max(smem, set.f[i].ac_smem);
   // Occupancy cap: a padded shared-memory request bounds the AC CTAs resident per SM, which leaves registers and shared memory for the
   // tile kernels (reconstruction, render) of images that are further along (they otherwise queue behind ~70 ms entropy CTAs).
-  { const char* e = getenv("JXLB200_AC_SMEM_KB"); const uint32_t pad = e ? uint32_t(atoi(e)) * 1024u : kAcBatchSmem; if (lanes >= 8) smem = std::max(smem, std::min(pad, 200u * 1024u)); }
+  if (lanes >= 8) smem = std::max(smem, kAcBatchSmem);
   k_ac_vardct_multi<true><<<set.first[set.n] + set.cta_offset, 32 * AcWarpsFor(lanes), smem, st>>>(set, lanes);
 }
 void LaunchLfDequant(const DFrame* d, const DFrame& h, bool smooth, cudaStream_t st) {

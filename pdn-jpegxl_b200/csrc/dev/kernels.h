@@ -14,7 +14,6 @@ int LaunchAcGroups(const DFrame* d, const DFrame& h, int pass, int lanes, cudaSt
 void LaunchModLfGroups(const DFrame& h, cudaStream_t st);   // Modular frames: channels of shift >= 3 in the LF-group sections
 void LaunchModularGlobal(const DFrame* d, const DFrame& h, uint64_t start_bitpos, uint32_t num_channels, cudaStream_t st);
 void LaunchReconstruct(const DFrame* d, const DFrame& h, cudaStream_t st);       // dequant + CfL + LLF + inverse transforms
-void LaunchFilters(const DFrame* d, const DFrame& h, cudaStream_t st);           // gaborish + EPF (result in h.xyb)
 bool LaunchFusedRender(const DFrame* d, const DFrame& h, cudaStream_t st);       // gaborish + EPF + colour fused (returns false when not applicable)
 void LaunchInverseRct(const DFrame* d, const DFrame& h, const DModOp* ops, cudaStream_t st);   // ops: host copy of the op table (h.ops or the blob table)
 void LaunchOutput(const DFrame* d, const DFrame& h, cudaStream_t st);            // colour transform + sample conversion + interleave (+BGRA)

@@ -2,8 +2,9 @@
 //   k_reconstruct : HF dequant + chroma-from-luma + LLF-from-LF + inverse transform for every varblock of a
 //                   256x256 group (SURVEY.md A.8 "Dequant", A.9). int16 coefficients in, fp32 XYB planes out:
 //                   6 B + 12 B = 18 algorithmic bytes per pixel.
-//   k_inv_sigma, k_gaborish, k_epf : restoration filters (A.10), 24 B/px per pass.
-//   k_output / k_output_modular : XYB -> linear -> transfer function -> sample type, interleave, optional
+//   k_inv_sigma : the EPF's 1/sigma per 8x8 block. k_gaborish : one gaborish pass over whole planes (the encoder's inverse gaborish).
+//   k_render_wide_tma, k_render : restoration filters (A.10) + colour + pack fused, one tile and its halo at a time in shared memory.
+//   k_output / k_output_int : XYB -> linear -> transfer function -> sample type, interleave, optional
 //                   fused BGRA32 surface pack (15-16 B/px for 8-bit RGB/BGRA), bit-exact integer path for lossless.
 // Replaces libjxl's dequant / IDCT / render-pipeline stages reached from N/Decoder/JxlDecoder.cpp:252 and the
 // managed repack loops I/DecoderLayerData.cs:667-992 + S/JpegXLLoad.cs:219-249 (bgra mode).
@@ -15,7 +16,7 @@
 #include <cuda_fp16.h>
 #include <cuda.h>
 #include <cmath>
-#include <cstdlib>
+#include <stdexcept>
 
 namespace jxlgpu {
 
@@ -387,30 +388,6 @@ __global__ void k_gaborish(const DFrame* fp, const float* __restrict__ src, floa
     dst[c * plane + size_t(y) * f.xpad + x] = m[x] * mul + (t[x] + b[x] + m[xl] + m[xr]) * (w1 * mul) + (t[xl] + t[xr] + b[xl] + b[xr]) * (w2 * mul); }
 }
 
-template <int PASS>
-__global__ void k_epf(const DFrame* fp, const float* __restrict__ src, float* __restrict__ dst) {
-  const DFrame& f = *fp; const int xs = int(f.xsize), ys = int(f.ysize); const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y; if (x >= xs || y >= ys) return;
-  const size_t plane = size_t(f.xpad) * f.ypad; const size_t at = size_t(y) * f.xpad + x;
-  const float is = f.inv_sigma[size_t(y >> 3) * f.xb + (x >> 3)];
-  if (is < -3.90524291751269967465540850526868f) { for (int c = 0; c < 3; c++) dst[c * plane + at] = src[c * plane + at]; return; }
-  const float sigma_scale = PASS == 0 ? f.lpf.pass0_sigma_scale : PASS == 2 ? f.lpf.pass2_sigma_scale : 1.0f; const float sm = sigma_scale * 1.65f;
-  const bool border = ((y & 7) == 0 || (y & 7) == 7 || (x & 7) == 0 || (x & 7) == 7); const float inv = is * (border ? sm * f.lpf.border_sad_mul : sm);
-  const int n12[12][2] = {{-2, 0}, {-1, -1}, {-1, 0}, {-1, 1}, {0, -2}, {0, -1}, {0, 1}, {0, 2}, {1, -1}, {1, 0}, {1, 1}, {2, 0}}; const int n4[4][2] = {{-1, 0}, {0, -1}, {0, 1}, {1, 0}};
-  const int plus[5][2] = {{0, 0}, {-1, 0}, {1, 0}, {0, -1}, {0, 1}};
-  const int nn = PASS == 0 ? 12 : 4;
-  float wsum = 1.0f, acc[3]; for (int c = 0; c < 3; c++) acc[c] = src[c * plane + at];
-  for (int i = 0; i < nn; i++) {
-    const int dy = PASS == 0 ? n12[i][0] : n4[i][0], dx = PASS == 0 ? n12[i][1] : n4[i][1]; float sad = 0;
-    for (int c = 0; c < 3; c++) { const float* p = src + c * plane; float s = 0;
-      if (PASS == 2) s = fabsf(p[size_t(MirrorDev(y + dy, ys)) * f.xpad + MirrorDev(x + dx, xs)] - p[at]);
-      else for (int k = 0; k < 5; k++) { int yy = y + plus[k][0], xx = x + plus[k][1]; s += fabsf(p[size_t(MirrorDev(yy + dy, ys)) * f.xpad + MirrorDev(xx + dx, xs)] - p[size_t(MirrorDev(yy, ys)) * f.xpad + MirrorDev(xx, xs)]); }
-      sad += s * f.lpf.epf_channel_scale[c]; }
-    float wgt = fmaxf(0.f, 1.0f + sad * inv); wsum += wgt; const size_t nat = size_t(MirrorDev(y + dy, ys)) * f.xpad + MirrorDev(x + dx, xs);
-    for (int c = 0; c < 3; c++) acc[c] += wgt * src[c * plane + nat];
-  }
-  const float iw = 1.0f / wsum; for (int c = 0; c < 3; c++) dst[c * plane + at] = acc[c] * iw;
-}
-
 // ------------------------------------------------------------------ inverse RCT on the global Modular image
 __global__ void k_inverse_rct(const DFrame* fp, uint32_t op_index) {
   const DFrame& f = *fp; const DModOp& op = ModOp(f, op_index); const uint32_t type = op.rct_type; const size_t n = size_t(op.w) * op.h; size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; if (i >= n) return;
@@ -681,7 +658,7 @@ __global__ void __launch_bounds__(256) k_render(const __grid_constant__ DFrame f
 // gaborish + EPF pass 1 (+ pass 2) + XYB -> RGB8 for the common output (RGB8, identity orientation) with 64x32 output tiles and
 // vector shared-memory accesses. Same arithmetic as k_render; what changes is the work per instruction:
 //   * 64x32 tiles: halo overhead (70x38)/(64x32) = 1.30 instead of 1.41 for 32x32, and rows of 72 floats so that every row starts
-//     16-byte aligned (x = -4 sits in column 0): interior tiles are loaded with aligned float4 loads, filters read LDS.128;
+//     16-byte aligned (x = -4 sits in column 0): filters read LDS.128;
 //   * gaborish: a thread owns (channel, 4 columns, 9 rows) with a rolling three-row window: 3 shared loads per 4 outputs;
 //   * EPF: the 5-tap-cross SADs are sums of channel-weighted |horizontal| / |vertical| difference maps Dh, Dv built once; a thread
 //     filters a 4x2 patch and builds the cross sums of its patch from LDS.128 rows, ~6 shared loads per pixel instead of 16;
@@ -689,8 +666,8 @@ __global__ void __launch_bounds__(256) k_render(const __grid_constant__ DFrame f
 // Buffers: A[3][38][72] (raw XYB; later Dh = A[0], Dv = A[1]), B[3][38][72] (after gaborish). Row r <-> y = ty0 - 3 + r, column c <-> x = tx0 - 4 + c.
 static const int kRfS = 72, kRfRows = 38, kRfPlane = kRfS * kRfRows;
 static const int kRfBuf = (3 * kRfPlane * 4 + 127) / 128 * 128 / 4;   // floats per three-plane buffer, padded so that every buffer starts 128-byte aligned (TMA destination)
-__device__ __forceinline__ bool WideTileInterior(const DFrame& f, int tx0, int ty0) { return tx0 >= 4 && tx0 + 68 <= int(f.xsize) && ty0 >= 3 && ty0 + 35 <= int(f.ysize); }
-// tile + halo -> A with mirrored image borders (the slow path of border tiles; interior tiles use float4 loads or TMA)
+__host__ __device__ __forceinline__ bool WideTileInterior(const DFrame& f, int tx0, int ty0) { return tx0 >= 4 && tx0 + 68 <= int(f.xsize) && ty0 >= 3 && ty0 + 35 <= int(f.ysize); }
+// tile + halo -> A with mirrored image borders (the slow path of border tiles; interior tiles arrive by TMA)
 __device__ __forceinline__ void WideTileFillMirrored(const DFrame& f, float* A, int tx0, int ty0, int tid) {
   const int xs = int(f.xsize), ys = int(f.ysize); const size_t plane = size_t(f.xpad) * f.ypad;
   for (int i = tid; i < 3 * kRfRows * kRfS; i += 256) { const int c = i / kRfPlane, rem = i - c * kRfPlane, r = rem / kRfS, col = rem - r * kRfS;
@@ -833,30 +810,17 @@ __device__ __forceinline__ void WideTileStages(const DFrame& f, float* A, float*
   }
 }
 
-// Front-end 1: one CTA per tile, the tile is loaded by the threads themselves (aligned float4 loads for interior tiles).
-template <int EPF, bool BGRA>
-__global__ void __launch_bounds__(256, 2) k_render_wide(const __grid_constant__ DFrame f) {
-  extern __shared__ __align__(128) float rw[];
-  float* A = rw; float* B = rw + kRfBuf; __shared__ float s_is[32];
-  const int tid = threadIdx.x, tx0 = blockIdx.x * 64, ty0 = blockIdx.y * 32;
-  if (f.band_on && (ty0 + 32 <= int(f.out_y0) || ty0 >= int(f.out_y1))) return;
-  const size_t plane = size_t(f.xpad) * f.ypad;
-  if (tid < 32) { const int by = (ty0 >> 3) + (tid >> 3), bx = (tx0 >> 3) + (tid & 7); s_is[tid] = (by < int(f.yb) && bx < int(f.xb)) ? f.inv_sigma[size_t(by) * f.xb + bx] : 0.f; }
-  if (WideTileInterior(f, tx0, ty0)) {
-    for (int i = tid; i < 3 * kRfRows * 18; i += 256) { const int c = i / (kRfRows * 18), rem = i - c * kRfRows * 18, r = rem / 18, q = rem - r * 18;
-      reinterpret_cast<float4*>(A)[i] = __ldg(reinterpret_cast<const float4*>(f.xyb + c * plane + size_t(ty0 - 3 + r) * f.xpad + tx0 - 4) + q); }
-  } else WideTileFillMirrored(f, A, tx0, ty0, tid);
-  __syncthreads();
-  WideTileStages<EPF, BGRA>(f, A, B, s_is, tx0, ty0, tid);
-}
-
-// Front-end 2 (the default): persistent CTAs, two per SM, that walk the tiles with a grid stride; the raw 72x38x3 box of the NEXT tile is
-// fetched by one TMA operation (cp.async.bulk.tensor.3d, completion on an mbarrier) into the second raw buffer while the current tile is
-// filtered, so no warp ever waits on HBM latency inside the stages. Border tiles (mirrored samples: TMA can only zero-fill) are loaded
-// by the threads. The A/B against front-end 1 is in profiles/ (JXLB200_RENDER_TMA=0 selects front-end 1).
+// Frame row of the first row the XYB planes hold: a band decode allocates them from its first reconstructed group row (the halo row above
+// the band) and addresses them through a base shifted back by that many rows; a whole-frame decode starts at row 0.
+__host__ __device__ __forceinline__ int XybFirstRow(const DFrame& f) { return f.band_on ? int(f.comp_g0 * f.group_dim) : 0; }
+// Persistent CTAs, two per SM, walk the tiles [t0, t1) with a grid stride (a band decode passes its own tile rows). The raw 72x38x3 box of
+// the NEXT tile is fetched by one TMA operation (cp.async.bulk.tensor.3d, completion on an mbarrier) into the second raw buffer while the
+// current tile is filtered, so no warp waits on HBM latency inside the stages (profiles/r02_render_tma_ab.md). Border tiles (mirrored
+// samples: TMA can only zero-fill) are loaded by the threads. Interior tiles of a band stay inside its allocated rows: the band carries one
+// group row of halo on each side, more than the 3 rows above and 35 below that WideTileInterior asks for.
 __device__ __forceinline__ uint32_t SmemU32(const void* p) { return uint32_t(__cvta_generic_to_shared(p)); }
 template <int EPF, bool BGRA>
-__global__ void __launch_bounds__(256, 2) k_render_wide_tma(const __grid_constant__ DFrame f, const __grid_constant__ CUtensorMap tmap, const int ntx, const int ntiles) {
+__global__ void __launch_bounds__(256, 2) k_render_wide_tma(const __grid_constant__ DFrame f, const __grid_constant__ CUtensorMap tmap, const int ntx, const int t0, const int t1) {
   extern __shared__ __align__(128) float rw[];
   float* B = rw + 2 * kRfBuf;   // raw buffers: rw + b * kRfBuf, b = 0, 1
   __shared__ __align__(8) unsigned long long bar[2]; __shared__ float s_is[32];
@@ -868,22 +832,20 @@ __global__ void __launch_bounds__(256, 2) k_render_wide_tma(const __grid_constan
   }
   __syncthreads();
   auto tile_xy = [&](int t, int& tx0, int& ty0) { tx0 = (t % ntx) * 64; ty0 = (t / ntx) * 32; };
-  auto in_band = [&](int ty0) { return !f.band_on || !(ty0 + 32 <= int(f.out_y0) || ty0 >= int(f.out_y1)); };
   auto issue = [&](int t, int b) {   // one thread: arm the barrier with the box size and start the bulk copy
     int tx0, ty0; tile_xy(t, tx0, ty0);
-    if (tid != 0 || !in_band(ty0) || !WideTileInterior(f, tx0, ty0)) return;
+    if (tid != 0 || !WideTileInterior(f, tx0, ty0)) return;
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the buffer was last written through the generic proxy (difference maps)
     const uint32_t bytes = 3u * kRfPlane * 4u, mb = SmemU32(&bar[b]);
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mb), "r"(bytes) : "memory");
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 ::"r"(SmemU32(rw + b * kRfBuf)), "l"(reinterpret_cast<uint64_t>(&tmap)), "r"(mb), "r"(tx0 - 4), "r"(ty0 - 3), "r"(0) : "memory");
+                 ::"r"(SmemU32(rw + b * kRfBuf)), "l"(reinterpret_cast<uint64_t>(&tmap)), "r"(mb), "r"(tx0 - 4), "r"(ty0 - 3 - XybFirstRow(f)), "r"(0) : "memory");
   };
   uint32_t phase_bits = 0u;   // bit b: parity of buffer b's barrier
-  int t = blockIdx.x; if (t < ntiles) issue(t, 0);
-  for (int b = 0; t < ntiles; t += int(gridDim.x), b ^= 1) {
-    if (t + int(gridDim.x) < ntiles) issue(t + int(gridDim.x), b ^ 1);
+  int t = t0 + int(blockIdx.x); if (t < t1) issue(t, 0);
+  for (int b = 0; t < t1; t += int(gridDim.x), b ^= 1) {
+    if (t + int(gridDim.x) < t1) issue(t + int(gridDim.x), b ^ 1);
     int tx0, ty0; tile_xy(t, tx0, ty0);
-    if (!in_band(ty0)) continue;   // uniform over the CTA; no copy was issued for this tile
     float* A = rw + b * kRfBuf;
     if (tid < 32) { const int by = (ty0 >> 3) + (tid >> 3), bx = (tx0 >> 3) + (tid & 7); s_is[tid] = (by < int(f.yb) && bx < int(f.xb)) ? f.inv_sigma[size_t(by) * f.xb + bx] : 0.f; }
     if (WideTileInterior(f, tx0, ty0)) {
@@ -919,54 +881,51 @@ void LaunchReconstruct(const DFrame* d, const DFrame& h, cudaStream_t st) {
     k_reconstruct_dct8<<<grid, 256, d8smem, st>>>(h, items); }
   k_reconstruct<16><<<h.num_groups * 4, kReconWarps * 32, smem16, st>>>(d); k_reconstruct<32><<<h.num_groups * 4, kReconWarps * 32, smem32, st>>>(d); CountLaunch(3);
 }
-// Runs gaborish + EPF; ping-pongs between xyb and xyb_tmp. Returns the buffer holding the result.
-void LaunchFilters(const DFrame* d, const DFrame& h, cudaStream_t st) {
-  dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8); float* a = h.xyb; float* b = h.xyb_tmp;
-  if (h.lpf.gab) { k_gaborish<<<grid, blk, 0, st>>>(d, a, b); CountLaunch(); std::swap(a, b); }
-  if (h.lpf.epf_iters) {
-    size_t n = size_t(h.xb) * h.yb; k_inv_sigma<<<unsigned((n + 255) / 256), 256, 0, st>>>(d); CountLaunch();
-    if (h.lpf.epf_iters == 3) { k_epf<0><<<grid, blk, 0, st>>>(d, a, b); CountLaunch(); std::swap(a, b); }
-    k_epf<1><<<grid, blk, 0, st>>>(d, a, b); CountLaunch(); std::swap(a, b);
-    if (h.lpf.epf_iters >= 2) { k_epf<2><<<grid, blk, 0, st>>>(d, a, b); CountLaunch(); std::swap(a, b); }
-  }
-}
 void LaunchGaborishPlanes(const DFrame* d, const DFrame& h, const float* src, float* dst, cudaStream_t st) { dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8); k_gaborish<<<grid, blk, 0, st>>>(d, src, dst); CountLaunch(); }
-const float* FilteredPlanes(const DFrame& h) { int n = (h.lpf.gab ? 1 : 0) + (h.lpf.epf_iters == 3 ? 3 : int(h.lpf.epf_iters)); return (n & 1) ? h.xyb_tmp : h.xyb; }
 // TMA descriptor of the three XYB planes as one rank-3 fp32 tensor {xpad, ypad, 3}, box {72, 38, 3}: one bulk copy fetches a whole
-// tile-plus-halo into the dense [plane][row][72] layout the filters read. The driver entry point is looked up at run time (no libcuda link).
+// tile-plus-halo into the dense [plane][row][72] layout the filters read. The tensor starts at the planes' first allocated row (XybFirstRow),
+// so a band's map covers exactly its ypad rows. The driver entry point is looked up at run time (no libcuda link).
 static bool EncodeXybTensorMap(const DFrame& h, CUtensorMap* out) {
   typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
                                CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
   static EncodeFn fn = []() -> EncodeFn { void* p = nullptr; cudaDriverEntryPointQueryResult q;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) { cudaGetLastError(); return nullptr; } return reinterpret_cast<EncodeFn>(p); }();
-  if (!fn || h.xpad < 72 || h.ypad < 38) return false;
+  if (!fn) return false;
   const cuuint64_t gdim[3] = {h.xpad, h.ypad, 3}, gstride[2] = {cuuint64_t(h.xpad) * 4, cuuint64_t(h.xpad) * h.ypad * 4}; const cuuint32_t box[3] = {kRfS, kRfRows, 3}, es[3] = {1, 1, 1};
-  return fn(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, h.xyb, gdim, gstride, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  return fn(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, h.xyb + size_t(XybFirstRow(h)) * h.xpad, gdim, gstride, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+// k_render_wide_tma for the RGB8 or opaque BGRA32 output of a frame with gaborish + one EPF iteration
+static void LaunchRenderWide(const DFrame& h, bool bgra, cudaStream_t st) {
+  const size_t smem = size_t(3) * kRfBuf * sizeof(float);
+  { static bool attr[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (!attr[dev & 63]) {
+      cudaFuncSetAttribute(k_render_wide_tma<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); cudaFuncSetAttribute(k_render_wide_tma<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); attr[dev & 63] = true; } }
+  const int ntx = int(h.xsize + 63) / 64;
+  // tile rows of the output rows: a band's out_y0 is a multiple of the group size, hence of the 32-row tile height
+  const int t0 = h.band_on ? int(h.out_y0 / 32) * ntx : 0, t1 = int(((h.band_on ? h.out_y1 : h.ysize) + 31) / 32) * ntx;
+  CUtensorMap tmap{};
+  // Tile (64, 32) is the first that can be interior: a frame smaller than 132 x 67 has no interior tile, issues no copy and gets the zero map.
+  if (WideTileInterior(h, 64, 32) && !EncodeXybTensorMap(h, &tmap)) throw std::runtime_error("cuTensorMapEncodeTiled failed for the render kernel's XYB planes");
+  const int grid = std::min(t1 - t0, 148 * 2);
+  if (bgra) k_render_wide_tma<1, true><<<grid, 256, smem, st>>>(h, tmap, ntx, t0, t1); else k_render_wide_tma<1, false><<<grid, 256, smem, st>>>(h, tmap, ntx, t0, t1);
 }
 // gaborish + EPF + colour in one pass over the frame (VarDCT frames with at least one restoration filter)
 template <int GAB, int EPF> static void LaunchRenderT(const DFrame& h, cudaStream_t st) {
   constexpr int H = GAB + (EPF == 3 ? 3 : 0) + (EPF >= 1 ? 2 : 0) + (EPF >= 2 ? 1 : 0), D = 32 + 2 * H; size_t smem = (size_t(EPF ? 8 : 6) * D * D + 64) * sizeof(float);
-  { static bool attr[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (!attr[dev & 63]) { cudaFuncSetAttribute(k_render<GAB, EPF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); cudaFuncSetAttribute(k_render<GAB, EPF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); attr[dev & 63] = true; } }
+  constexpr bool kWide = GAB == 1 && EPF == 1;   // RGB8 output of these filters takes k_render_wide_tma, so k_render<1, 1, true> is never built
+  { static bool attr[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (!attr[dev & 63]) { cudaFuncSetAttribute(k_render<GAB, EPF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+      if constexpr (!kWide) cudaFuncSetAttribute(k_render<GAB, EPF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); attr[dev & 63] = true; } }
   const DOutput& o = h.out;
   const bool rgb8 = !o.bgra && o.sample_type == 0 && o.num_channels == 3 && o.color_channels == 3 && o.alpha_plane < 0 && o.black_plane < 0 && !o.premultiplied && o.orientation == 1;
-  const bool fast = rgb8 && (size_t(h.xsize) * 3) % 4 == 0 && (reinterpret_cast<uintptr_t>(h.out_px) & 3) == 0;
   dim3 grid((h.xsize + 31) / 32, (h.ysize + 31) / 32);
-  static const bool no_wide = getenv("JXLB200_NO_WIDE_RENDER") != nullptr;
-  // opaque BGRA32 surface of an 8-bit RGB image (JxlB200LoadImageBgra, BASELINE config 2): the same kernel with a 16-byte store per 4 pixels
-  const bool fast_bgra = o.bgra && o.color_channels == 3 && o.alpha_plane < 0 && o.black_plane < 0 && !o.premultiplied && o.orientation == 1 && (reinterpret_cast<uintptr_t>(h.out_px) & 15) == 0;
-  if ((rgb8 || fast_bgra) && GAB == 1 && EPF == 1 && !no_wide) {   // rows that are not 4-byte aligned fall back to byte stores inside the kernel
-    const size_t wsmem = size_t(2) * kRfBuf * sizeof(float), tsmem = size_t(3) * kRfBuf * sizeof(float);
-    { static bool wattr[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (!wattr[dev & 63]) {
-        cudaFuncSetAttribute(k_render_wide<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(wsmem)); cudaFuncSetAttribute(k_render_wide<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(wsmem));
-        cudaFuncSetAttribute(k_render_wide_tma<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(tsmem)); cudaFuncSetAttribute(k_render_wide_tma<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(tsmem)); wattr[dev & 63] = true; } }
-    const dim3 wgrid((h.xsize + 63) / 64, (h.ysize + 31) / 32);
-    static const bool use_tma = !(getenv("JXLB200_RENDER_TMA") && atoi(getenv("JXLB200_RENDER_TMA")) == 0);
-    CUtensorMap tmap;
-    if (use_tma && !h.band_on && EncodeXybTensorMap(h, &tmap)) {   // band decodes address the planes through a shifted base: thread loads
-      const int ntiles = int(wgrid.x * wgrid.y), grid1 = std::min(ntiles, 148 * 2);
-      if (fast_bgra) k_render_wide_tma<1, true><<<grid1, 256, tsmem, st>>>(h, tmap, int(wgrid.x), ntiles); else k_render_wide_tma<1, false><<<grid1, 256, tsmem, st>>>(h, tmap, int(wgrid.x), ntiles);
-    } else if (fast_bgra) k_render_wide<1, true><<<wgrid, 256, wsmem, st>>>(h); else k_render_wide<1, false><<<wgrid, 256, wsmem, st>>>(h);
-  } else if (fast) k_render<GAB, EPF, true><<<grid, 256, smem, st>>>(h); else k_render<GAB, EPF, false><<<grid, 256, smem, st>>>(h);
+  if constexpr (kWide) {
+    // opaque BGRA32 surface of an 8-bit RGB image (JxlB200LoadImageBgra, BASELINE config 2): the same kernel with a 16-byte store per 4 pixels
+    const bool fast_bgra = o.bgra && o.color_channels == 3 && o.alpha_plane < 0 && o.black_plane < 0 && !o.premultiplied && o.orientation == 1 && (reinterpret_cast<uintptr_t>(h.out_px) & 15) == 0;
+    if (rgb8 || fast_bgra) LaunchRenderWide(h, fast_bgra, st);   // rows that are not 4-byte aligned fall back to byte stores inside the kernel
+    else k_render<1, 1, false><<<grid, 256, smem, st>>>(h);
+  } else {
+    const bool fast = rgb8 && (size_t(h.xsize) * 3) % 4 == 0 && (reinterpret_cast<uintptr_t>(h.out_px) & 3) == 0;
+    if (fast) k_render<GAB, EPF, true><<<grid, 256, smem, st>>>(h); else k_render<GAB, EPF, false><<<grid, 256, smem, st>>>(h);
+  }
   CountLaunch();
 }
 bool LaunchFusedRender(const DFrame* d, const DFrame& h, cudaStream_t st) {
@@ -1021,7 +980,7 @@ void LaunchOutput(const DFrame* d, const DFrame& h, cudaStream_t st) {
   dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8);
   bool int_path = h.encoding == 1 && !h.color.xyb_encoded && h.out.exp_bits == 0 && h.out.black_plane < 0 && !h.out.premultiplied && (h.out.sample_type == 0 ? h.out.bits == 8 : (h.out.sample_type == 1 && h.out.bits == 16)) &&
                   (h.out.alpha_plane < 0 || (h.out.alpha_bits == h.out.bits && h.out.alpha_exp_bits == 0 && h.out_ch[h.out.alpha_plane].hshift == 0));
-  if (int_path) k_output_int<<<grid, blk, 0, st>>>(d); else k_output<<<grid, blk, 0, st>>>(h, FilteredPlanes(h));
+  if (int_path) k_output_int<<<grid, blk, 0, st>>>(d); else k_output<<<grid, blk, 0, st>>>(h, h.xyb);
   CountLaunch();
 }
 

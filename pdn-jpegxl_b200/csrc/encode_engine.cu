@@ -159,7 +159,6 @@ EncPlan MakePlan(uint32_t xs, uint32_t ys, uint32_t flags, const EncodeRequest& 
   p.single = NumTocEntries(fh) == 1;
   // effort >= 5: adaptive quantisation and chroma from luma (block-local decisions made on the device; what libjxl's higher efforts add first)
   p.aq = p.cfl = !p.lossless && req.effort >= 5;
-  { const char* v = getenv("JXLB200_ENC_AQ"); if (v && *v == '0') p.aq = false; v = getenv("JXLB200_ENC_CFL"); if (v && *v == '0') p.cfl = false; }   // measurement switches (scripts/compare_efforts.py)
   p.tree = p.lossless ? MakeLosslessTree(p.ncolor + p.num_ec) : MakeVarDctTree(nlf, p.num_ec, p.aq, p.cfl); TokenizeTree(p.tree, &p.tree_tokens);
   EncOptions topt; topt.cfg = HybridCfg{4, 1, 0}; p.mopt.cfg = HybridCfg{4, 1, 0}; p.mopt.max_clusters = 48; p.aopt.cfg = HybridCfg{4, 2, 0}; p.aopt.max_clusters = 64;
   if (req.effort <= 2) { p.mopt.use_prefix = true; p.aopt.use_prefix = true; }   // the fastest efforts write prefix codes: no serial state chain in the stream writer

@@ -1,4 +1,4 @@
-"""BASELINE config 4a: 4096x4096 RGBA8 lossless Modular, decode stage times through LoadImage (CUDA events). JXLB200_NO_SPEC=1 = one-lane loops."""
+"""BASELINE config 4a: 4096x4096 RGBA8 lossless Modular, decode stage times through LoadImage (CUDA events)."""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))

@@ -201,20 +201,26 @@ def test_batch_pipeline_mixed_content(gpu, oracle):
                 assert np.array_equal(o, s)
 
 
-@pytest.mark.parametrize("kw", [dict(effort=7), dict(effort=7, distance=8.0), dict(effort=3, force_strategy=24), dict(lossless=True, channels=4), dict(effort=5, channels=4)])
+@pytest.mark.parametrize("kw", [dict(effort=7), dict(effort=7, distance=8.0), dict(effort=3, force_strategy=24), dict(lossless=True, channels=4), dict(effort=5, channels=4),
+                                dict(effort=7, bgra=True)])
 def test_band_decode_stitches_to_the_full_frame(gpu, oracle, kw):
     """Config-5 style sharding on one GPU: the frame decoded as three bands of group rows equals the full decode bit for bit (each band
-    reconstructs one extra group row per side, so gaborish + 3 EPF iterations see the same neighbours as in the full frame)."""
+    reconstructs one extra group row per side, so gaborish + 3 EPF iterations see the same neighbours as in the full frame). The BGRA32
+    bands are compared with the BGRA32 surface of the whole file."""
     kw = dict(kw)
     ch = kw.pop("channels", 3)
+    bgra = kw.pop("bgra", False)
     img = oracle.synthetic_image(700, 1500, seed=31, channels=ch)
     data = oracle.encode(img, **kw)
-    ld = _decode_gpu(gpu, data).layer_data
-    full = ld.color if ld.transparency is None else np.concatenate([ld.color, ld.transparency[..., None]], axis=2)
+    if bgra:
+        full = gpu.load_image_bgra(data)
+    else:
+        ld = _decode_gpu(gpu, data).layer_data
+        full = ld.color if ld.transparency is None else np.concatenate([ld.color, ld.transparency[..., None]], axis=2)
     w, h, gdim, rows = gpu.band_layout(data)
     assert (w, h) == (700, 1500) and rows == -(-1500 // gdim)
     cuts = [0, 1, rows - 2, rows] if rows >= 4 else [0, 1, rows]
-    parts = [gpu.decode_band(data, a, b) for a, b in zip(cuts[:-1], cuts[1:]) if b > a]
+    parts = [gpu.decode_band(data, a, b, bgra=bgra) for a, b in zip(cuts[:-1], cuts[1:]) if b > a]
     assert np.array_equal(np.concatenate(parts, axis=0), full)
     with pytest.raises(gpu.FormatException):
         gpu.decode_band(data, 0, rows + 1)

@@ -8,8 +8,6 @@ scale. Here every stage is compared at the precision it is computed in:
   * reconstruction after dequantisation, CfL, LLF and the inverse transforms (which=0): fp32 level, relative to each channel's range;
   * output samples: within half a code unit (+ a measured delta) of a float64 colour conversion of the oracle's filtered planes.
 Each float bound sits at about 4x the worst value measured on a B200 and is checked against what one 8-bit LSB means in that stage."""
-import os
-
 import numpy as np
 import pytest
 from spec_cases import OPSIN_BIAS, OPSIN_INV
@@ -28,12 +26,6 @@ RECON_REL_BOUND = 7e-6   # measured 1.7e-6 (B channel, DCT256); 1.4e-6 for DCT16
 # side is at most 16 px go to k_reconstruct<16>, 32-px ones to k_reconstruct<32>, and a side of 64 px or more to the large-block pass.
 RECON_KERNEL = {0: "k_reconstruct_dct8", **{s: "k_reconstruct<16>" for s in (1, 2, 3, 4, 6, 7, 12, 13)},
                 **{s: "k_reconstruct<32>" for s in (5, 8, 9, 10, 11)}, **{s: ">=64 pass" for s in range(18, 27)}}
-
-
-def _skip_unless_fused():
-    # JXLB200_UNFUSED runs the unfiltered filter kernels, which overwrite the reconstruction in the XYB buffer with filtered planes
-    if os.environ.get("JXLB200_UNFUSED") is not None:
-        pytest.skip("JXLB200_UNFUSED: the XYB buffer holds filtered planes, not the reconstruction")
 
 
 def _geometry(w, h):
@@ -217,7 +209,6 @@ RECON_CASES = [("strategy%d" % s, 531, 277, dict(effort=3, force_strategy=s)) fo
 
 @pytest.mark.parametrize("name,w,h,kw", RECON_CASES, ids=[c[0] for c in RECON_CASES])
 def test_reconstruction_matches_the_oracle(gpu, oracle, name, w, h, kw):
-    _skip_unless_fused()
     data, cells = _encode(oracle, w, h, **kw)
     s = kw.get("force_strategy")
     if s is not None:
@@ -241,11 +232,10 @@ def render_branch(gab, epf, w, h, sample="u8", alpha=False, orientation=1, bgra=
     (device buffers are always aligned, so the alignment conditions hold)."""
     if not gab and not epf:
         return "k_output"
-    xpad, ypad = 8 * -(-w // 8), 8 * -(-h // 8)
     rgb8 = not bgra and sample == "u8" and not alpha and orientation == 1
     fast_bgra = bgra and not alpha and orientation == 1
     if (rgb8 or fast_bgra) and gab == 1 and epf == 1:
-        return "k_render_wide%s<1,%s>" % ("_tma" if xpad >= 72 and ypad >= 38 else "", "true" if bgra else "false")
+        return "k_render_wide_tma<1,%s>" % ("true" if bgra else "false")
     return "k_render<%d,%d,%s>" % (gab, epf, "true" if rgb8 and (w * 3) % 4 == 0 else "false")
 
 
@@ -274,8 +264,8 @@ RENDER_CASES = [
     ("wide_tma_191x161", 191, 161, GW, {}, "k_render_wide_tma<1,false>"),
     ("wide_tma_256x160", 256, 160, GW, {}, "k_render_wide_tma<1,false>"),   # 4-byte aligned rows
     ("wide_tma_bgra", 193, 65, GW, dict(bgra=True), "k_render_wide_tma<1,true>"),
-    ("wide_narrow", 64, 150, GW, {}, "k_render_wide<1,false>"),             # xpad < 72
-    ("wide_short", 200, 30, GW, {}, "k_render_wide<1,false>"),              # ypad < 38
+    ("wide_narrow", 64, 150, GW, {}, "k_render_wide_tma<1,false>"),         # narrower than 132: no interior tile, no TMA copy
+    ("wide_short", 200, 30, GW, {}, "k_render_wide_tma<1,false>"),          # shorter than 67: no interior tile, no TMA copy
     ("render_0_1", 200, 136, dict(gab=0, epf=1), {}, "k_render<0,1,true>"),
     ("render_0_2", 200, 136, dict(gab=0, epf=2), {}, "k_render<0,2,true>"),
     ("render_0_3", 200, 136, dict(gab=0, epf=3), {}, "k_render<0,3,true>"),
