@@ -164,6 +164,26 @@ JXLFT_API EncoderStatus JXLFT_CALL JxlB200BandEncoderTokenize(JxlB200BandEncoder
 JXLFT_API EncoderStatus JXLFT_CALL JxlB200BandEncoderFinish(JxlB200BandEncoder* enc, const uint64_t* frameHist, size_t histWords, uint8_t** sections,
                                                              size_t* sectionBytes, float* deviceMs, ErrorInfo* errorInfo);
 JXLFT_API void JXLFT_CALL JxlB200BandEncoderDestroy(JxlB200BandEncoder* enc);
+/* Stage dumps of a band session for parity tests: copies one device buffer to `out` (host memory, capacityBytes) and returns the bytes
+ * written. Valid only between Tokenize and Finish (Finish's ANS writer overwrites the token words in place). Outside that window, for a
+ * stage the session does not have (2-4 below effort 5; 0-8 for lossless) or when `out` is too small (NULL included), it returns 0 with a
+ * message; dims4 still receives the shape in that last case, so a first call can size the buffer. A whole frame is a session with
+ * frameHeight = height, firstRow = 0 and no halo; rows are those of the session (ext_rows includes the halo rows when gaborish is on).
+ *   which = 0: the XYB planes as the colour conversion wrote them (before the inverse gaborish), f32 [3][ext_rows][xpad], dims (3, ext_rows, xpad).
+ *              Columns past the width repeat the last column, rows past the height the last row.
+ *   which = 1: the XYB planes the DCT reads (after the inverse gaborish; the same as 0 when gaborish is off), same layout.
+ *   which = 2: per-block statistics {sum |AC of Y|, sum X*Y, sum B*Y, sum Y*Y} over the AC coefficients, f32 [yblocks][xblocks][4].
+ *   which = 3: the quantiser multiplier (hf_mul) of every block, u8 [yblocks][xblocks].
+ *   which = 4: the chroma-from-luma factors ytox, ytob of every 64x64 tile, i8 [2][ytiles][xtiles].
+ *   which = 5: LF (coefficient 0 of each block's DCT), f32 [3 (X, Y, B)][yblocks][xblocks].
+ *   which = 6: quantised LF as coded, stream order Y, X, B: i32 [3][yblocks][xblocks].
+ *   which = 7: quantised AC coefficients, i16 [group][3 (X, Y, B)][1024 cells][64] (the cell layout of JxlB200DebugDecodeStage which = 4).
+ *   which = 8: non-zero AC coefficients per block, u8 [3 (X, Y, B)][yblocks][xblocks].
+ *   which = 9: the device's tokens: u32 counts[streams], then for each stream its tokens as u32 pairs {ctx | symbol << 16 | nbits << 24, extra
+ *              bits}; the Modular streams (LF coefficients per LF group, then extra channels) first, then one AC stream per group.
+ *              dims = (streams, tokens, Modular streams).
+ * Blocks, tiles and groups are those of the session's own rows (a band counts its blocks from its first row). */
+JXLFT_API int64_t JXLFT_CALL JxlB200BandEncoderDebugStage(JxlB200BandEncoder* enc, int32_t which, void* out, int64_t capacityBytes, int64_t* dims4, ErrorInfo* errorInfo);
 JXLFT_API EncoderStatus JXLFT_CALL JxlB200AssembleBands(uint32_t width, uint32_t height, const EncoderOptions* options, const EncoderImageMetadata* metadata,
                                                          uint32_t frameFlags, const uint64_t* frameHist, size_t histWords, const uint8_t* const* bandSections,
                                                          const size_t* bandSectionBytes, int32_t bandCount, uint8_t** out, size_t* outSize, ErrorInfo* errorInfo);

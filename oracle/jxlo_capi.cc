@@ -89,6 +89,12 @@ const uint8_t* jxlo_image_exif(const jxlo_image* i, size_t* n) { *n = i->img.exi
 const uint8_t* jxlo_image_xmp(const jxlo_image* i, int k, size_t* n) { *n = i->img.xmp[k].size(); return i->img.xmp[k].data(); }
 // which: 0 idct, 1 gab, 2 epf (3 planes xpad*ypad floats), 3 lf (3 planes xb*yb); returns element count
 size_t jxlo_image_stage_f32(const jxlo_image* i, int which, const float** p) { const std::vector<float>& v = which == 0 ? i->img.stage_idct : which == 1 ? i->img.stage_gab : which == 2 ? i->img.stage_epf : i->img.stage_lf; *p = v.data(); return v.size(); }
+// which: 0 quantised LF (3 planes xb*yb, channel order X, Y, B), 1 hf_mul (xb*yb), 2 ytox, 3 ytob (xt*yt), 4 quantiser {global_scale, quant_lf,
+// x_qm_scale, b_qm_scale}; returns element count
+size_t jxlo_image_stage_i32(const jxlo_image* i, int which, const int32_t** p) {
+  const DecodedImage& d = i->img; const std::vector<int32_t>& v = which == 0 ? d.stage_lfq : which == 1 ? d.stage_hf_mul : which == 2 ? d.stage_ytox : which == 3 ? d.stage_ytob : d.stage_quant;
+  *p = v.data(); return v.size();
+}
 size_t jxlo_image_stage_coeffs(const jxlo_image* i, const int32_t** p) { *p = i->img.stage_coeffs.data(); return i->img.stage_coeffs.size(); }
 
 int jxlo_signature_check(const uint8_t* d, size_t n) { return SignatureCheck(d, n); }

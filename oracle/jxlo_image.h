@@ -33,7 +33,10 @@ inline void DecodeFrame(FrameState& fs, const uint8_t* data, size_t size, size_t
   if (fh.encoding == 0) { for (size_t i = 0; i < fs.strategy.size(); i++) JXLO_CHECK(fs.strategy[i] != 255, "HF metadata does not cover every block"); }
   { BitReader b = sr.Get(1 + nlf); if (fh.encoding == 0) DecodeHfGlobal(fs, b); sr.Done(b); }
   if (fh.encoding == 0 && !(fh.flags & kFlagSkipAdaptiveLfSmoothing)) AdaptiveLfSmoothing(fs);
-  if (dbg && opt.keep_stages && fh.encoding == 0) { dbg->stage_lf.clear(); for (int c = 0; c < 3; c++) dbg->stage_lf.insert(dbg->stage_lf.end(), fs.lf[c].d.begin(), fs.lf[c].d.end()); dbg->stage_coeffs.assign(size_t(3) * fs.xpad * fs.ypad, 0); }
+  if (dbg && opt.keep_stages && fh.encoding == 0) { dbg->stage_lf.clear(); for (int c = 0; c < 3; c++) dbg->stage_lf.insert(dbg->stage_lf.end(), fs.lf[c].d.begin(), fs.lf[c].d.end()); dbg->stage_coeffs.assign(size_t(3) * fs.xpad * fs.ypad, 0);
+    dbg->stage_lfq.clear(); for (int c = 0; c < 3; c++) dbg->stage_lfq.insert(dbg->stage_lfq.end(), fs.lfq[c].begin(), fs.lfq[c].end());
+    dbg->stage_hf_mul = fs.hf_mul; dbg->stage_ytox.assign(fs.ytox.begin(), fs.ytox.end()); dbg->stage_ytob.assign(fs.ytob.begin(), fs.ytob.end());
+    dbg->stage_quant = {int32_t(fs.q.global_scale), int32_t(fs.q.quant_lf), int32_t(fh.x_qm_scale), int32_t(fh.b_qm_scale)}; }
   auto group_job = [&](size_t g) {
     std::vector<int32_t> coeffs[3]; std::vector<uint16_t> nz[3];
     if (fh.encoding == 0) for (auto& c : coeffs) c.assign(256 * 256, 0);

@@ -176,6 +176,9 @@ struct DecodedImage {
   ImageMetadata meta; std::string frame_name; bool is_container = false; std::vector<uint8_t> exif; std::vector<std::vector<uint8_t>> xmp; bool has_exif = false;
   // stage dumps (keep_stages)
   int xpad = 0, ypad = 0; std::vector<float> stage_idct, stage_gab, stage_epf, stage_lf; std::vector<int32_t> stage_coeffs;
+  // the HF metadata and LF integers the file carries: quantised LF [3 (X, Y, B)][yb][xb], hf_mul [yb][xb], ytox / ytob [yt][xt], and the
+  // quantiser {global_scale, quant_lf, x_qm_scale, b_qm_scale}
+  std::vector<int32_t> stage_lfq, stage_hf_mul, stage_ytox, stage_ytob, stage_quant;
 };
 
 inline size_t BytesPerSample(int t) { return t == kU8 ? 1 : t == kF32 ? 4 : 2; }

@@ -78,7 +78,8 @@ class IOCallbacks(C.Structure):
 EXPORTS = ["GetLibJxlVersion", "LoadImage", "SaveImage", "JxlB200LoadImageBgra", "JxlB200PeekInfo", "JxlB200DecodeBatch", "JxlB200EncodeToMemory",
            "JxlB200Free", "JxlB200LastStageTimes", "JxlB200KernelLaunchCount", "JxlB200DebugDecodeStage", "JxlB200CudaAvailable", "JxlB200BandLayout",
            "JxlB200DecodeBand", "JxlB200ReleaseMemory", "JxlB200DebugParseIcc", "JxlB200DecodeBatchSubmit", "JxlB200DecodeBatchWait", "JxlB200LoadImageLayers",
-           "JxlB200BandEncoderCreate", "JxlB200BandEncoderTokenize", "JxlB200BandEncoderFinish", "JxlB200BandEncoderDestroy", "JxlB200AssembleBands", "JxlB200DebugSectionSizes"]
+           "JxlB200BandEncoderCreate", "JxlB200BandEncoderTokenize", "JxlB200BandEncoderFinish", "JxlB200BandEncoderDestroy", "JxlB200AssembleBands", "JxlB200DebugSectionSizes",
+           "JxlB200BandEncoderDebugStage"]
 
 _lib.GetLibJxlVersion.restype = C.c_uint32
 _lib.LoadImage.argtypes = [C.POINTER(DecoderCallbacks), C.c_void_p, C.c_size_t, C.POINTER(ErrorInfo)]
@@ -597,6 +598,8 @@ _lib.JxlB200BandEncoderFinish.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.
 _lib.JxlB200BandEncoderFinish.restype = C.c_int32
 _lib.JxlB200BandEncoderDestroy.argtypes = [C.c_void_p]
 _lib.JxlB200BandEncoderDestroy.restype = None
+_lib.JxlB200BandEncoderDebugStage.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.POINTER(ErrorInfo)]
+_lib.JxlB200BandEncoderDebugStage.restype = C.c_int64
 _lib.JxlB200AssembleBands.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(EncoderOptionsNative), C.POINTER(EncoderImageMetadataNative), C.c_uint32, C.c_void_p, C.c_size_t,
                                       C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(ErrorInfo)]
 _lib.JxlB200AssembleBands.restype = C.c_int32
@@ -610,13 +613,16 @@ def _enc_check(st, ei):
 class BandEncoder:
     """One band of a frame on one GPU (JxlB200BandEncoder*). `rows_bgra`: the rows handed over, halo rows included (H x W x 4 uint8)."""
 
-    def __init__(self, rows_bgra, frame_height, first_row, halo_top, halo_bottom, options, device=-1):
+    def __init__(self, rows_bgra, frame_height, first_row, halo_top, halo_bottom, options, device=-1, metadata=None):
         self._rows = np.ascontiguousarray(rows_bgra, dtype=np.uint8)
         h, w, _ = self._rows.shape
         bitmap = BitmapData(self._rows.ctypes.data, w, h - halo_top - halo_bottom, self._rows.strides[0])
         self._opts = EncoderOptionsNative(options.distance, options.effort, options.lossless)
         flags, ei = C.c_uint32(), ErrorInfo()
-        self._h = _lib.JxlB200BandEncoderCreate(device, C.byref(bitmap), frame_height, first_row, halo_top, halo_bottom, C.byref(self._opts), None, 0, C.byref(flags), C.byref(ei))
+        meta, hold = _native_metadata(metadata) if metadata is not None else (None, None)   # the session keeps its own copy of the ICC profile
+        self._h = _lib.JxlB200BandEncoderCreate(device, C.byref(bitmap), frame_height, first_row, halo_top, halo_bottom, C.byref(self._opts),
+                                                C.byref(meta) if meta is not None else None, 0, C.byref(flags), C.byref(ei))
+        del hold
         if not self._h:
             raise FormatException("EncodeError", _message(ei) or "band encoder")
         self.flags = int(flags.value)
@@ -637,6 +643,30 @@ class BandEncoder:
         _lib.JxlB200Free(p)
         self.device_ms = float(ms.value)
         return blob
+
+    # element type of each stage of JxlB200BandEncoderDebugStage (9, the tokens, is returned as (counts, tokens, Modular stream count))
+    _STAGE_DTYPES = {0: np.float32, 1: np.float32, 2: np.float32, 3: np.uint8, 4: np.int8, 5: np.float32, 6: np.int32, 7: np.int16, 8: np.uint8}
+
+    def debug_stage(self, which):
+        """One device buffer of the session between tokenize() and finish(), shaped as the header documents."""
+        dims, ei = (C.c_int64 * 4)(), ErrorInfo()
+        _lib.JxlB200BandEncoderDebugStage(self._h, which, None, 0, dims, C.byref(ei))   # sizes the buffer (or fails with the reason)
+        d = [int(v) for v in dims]
+        if which == 9:
+            nbytes = d[0] * 4 + d[1] * 8
+        else:
+            shape = tuple(v for v in d if v)
+            if not shape:
+                raise FormatException("EncodeError", _message(ei) or "debug stage unavailable")
+            nbytes = int(np.prod(shape)) * np.dtype(self._STAGE_DTYPES[which]).itemsize
+        buf = np.empty(max(nbytes, 1), np.uint8)
+        n = _lib.JxlB200BandEncoderDebugStage(self._h, which, buf.ctypes.data, buf.size, dims, C.byref(ei))
+        if n == 0 or n != nbytes:
+            raise FormatException("EncodeError", _message(ei) or "debug stage unavailable")
+        if which == 9:
+            counts = buf[:d[0] * 4].view(np.uint32).copy()
+            return counts, buf[d[0] * 4:nbytes].view(np.uint32).reshape(-1, 2).copy(), d[2]
+        return buf[:nbytes].view(self._STAGE_DTYPES[which]).reshape(shape).copy()
 
     def close(self):
         if self._h:

@@ -493,6 +493,13 @@ EncoderStatus JxlB200BandEncoderFinish(JxlB200BandEncoder* enc, const uint64_t* 
     *sections = static_cast<uint8_t*>(CopyOut(blob.data(), blob.size())); *sectionBytes = blob.size(); return EncoderStatus_Ok;
   } catch (const std::bad_alloc&) { return EncoderStatus_OutOfMemory; } catch (...) { return EncoderStatus_EncodeError; }
 }
+int64_t JxlB200BandEncoderDebugStage(JxlB200BandEncoder* enc, int32_t which, void* out, int64_t capacityBytes, int64_t* dims4, ErrorInfo* errorInfo) {
+  if (!enc) { SetErrorMessage(errorInfo, "null parameter"); return 0; }
+  try {
+    if (enc->device >= 0) cudaSetDevice(enc->device);
+    std::string msg; const int64_t n = BandEncoderDebugStage(enc->s, which, out, capacityBytes, dims4, &msg); if (!n) SetErrorMessage(errorInfo, msg); return n;
+  } catch (...) { SetErrorMessage(errorInfo, "stage dump failed"); return 0; }
+}
 void JxlB200BandEncoderDestroy(JxlB200BandEncoder* enc) { if (!enc) return; try { if (enc->device >= 0) cudaSetDevice(enc->device); BandEncoderDestroy(enc->s); } catch (...) {} delete enc; }
 EncoderStatus JxlB200AssembleBands(uint32_t width, uint32_t height, const EncoderOptions* options, const EncoderImageMetadata* metadata, uint32_t frameFlags, const uint64_t* frameHist, size_t histWords,
                                    const uint8_t* const* bandSections, const size_t* bandSectionBytes, int32_t bandCount, uint8_t** out, size_t* outSize, ErrorInfo* errorInfo) {

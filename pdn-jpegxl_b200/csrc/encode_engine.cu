@@ -200,6 +200,7 @@ class BandEncoder {
   uint32_t Begin();                                         // -> flags of this band (bit 0: a non-gray pixel, bit 1: a non-opaque pixel)
   std::vector<uint64_t> Tokenize(uint32_t frame_flags);     // -> this band's histograms, [context][kEncAlphabet] (Modular contexts, then AC contexts)
   std::vector<BandSection> Finish(const std::vector<uint64_t>& frame_hist);
+  int64_t DebugStage(int32_t which, void* out, int64_t capacity, int64_t* dims4);   // JxlB200BandEncoderDebugStage
   const EncPlan& Plan() const { return plan; }
   float device_ms = 0;
 
@@ -213,6 +214,7 @@ class BandEncoder {
   std::vector<DEncModStream> mod_streams; std::vector<DEncStream> m_streams, a_streams; std::vector<uint32_t> ac_counts;
   uint32_t first_lf_stream = 0, first_group_stream = 0, max_mod_tokens = 0; uint64_t byte_cursor = 0;
   std::vector<std::vector<Token>> hfmeta_tokens; std::vector<uint32_t> hfmeta_nb;
+  bool stages_valid = false;                             // between Tokenize and Finish: k_enc_ans overwrites the token words in place
 };
 
 uint32_t BandEncoder::Begin() {
@@ -236,7 +238,7 @@ uint32_t BandEncoder::Begin() {
 }
 
 std::vector<uint64_t> BandEncoder::Tokenize(uint32_t frame_flags) {
-  Timer t(st, &device_ms);
+  Timer t(st, &device_ms); stages_valid = false;
   const uint32_t xs = req.width, ys = req.height;
   plan = MakePlan(xs, frame_h, frame_flags, req);
   const bool lossless = plan.lossless; const int nplanes = plan.nplanes;
@@ -354,7 +356,44 @@ std::vector<uint64_t> BandEncoder::Tokenize(uint32_t frame_flags) {
     TokenizeSmallChannel(info, nb, 2, 2, sid, plan.tree, &hfmeta_tokens[g]); TokenizeSmallChannel(sharp, w, h, 3, sid, plan.tree, &hfmeta_tokens[g]);
     for (const Token& t : hfmeta_tokens[g]) { uint32_t tok, nbits, bits; HybridEncode(plan.mopt.cfg, t.value, &tok, &nbits, &bits); JXLG_CHECK(tok < kEncAlphabet, "HF metadata token"); hist[size_t(t.ctx) * kEncAlphabet + tok]++; }
   }
+  stages_valid = true;
   return hist;
+}
+
+// Copies one device buffer of the session to `out` (see JxlB200BandEncoderDebugStage for the layouts). dims4 receives the shape even when
+// `out` is too small, so that a caller can size its buffer with a first call.
+int64_t BandEncoder::DebugStage(int32_t which, void* out, int64_t capacity, int64_t* dims4) {
+  JXLG_CHECK(stages_valid, "stage dumps exist only between Tokenize and Finish");
+  JXLG_CHECK(which >= 0 && which <= 9, "unknown stage");
+  JXLG_CHECK(which == 9 || !plan.lossless, "a lossless session has no VarDCT stages");
+  JXLG_CHECK(!(which >= 2 && which <= 4) || e.hf_mul_map, "block statistics and the HF maps exist from effort 5 on");
+  const size_t cells = size_t(e.xb) * e.yb, epx = size_t(e.xpad) * e.ext_rows, tiles = size_t(e.xt) * e.yt;
+  struct Piece { const void* p; size_t n; }; std::vector<Piece> pieces; int64_t d[4] = {0, 0, 0, 0};
+  std::vector<uint32_t> counts;   // stage 9: token count of every stream, written ahead of the tokens
+  switch (which) {
+    case 0: pieces.push_back({plan.fh.lf.gab ? d_tmp1.p : d_xyb.p, epx * 12}); d[0] = 3; d[1] = e.ext_rows; d[2] = e.xpad; break;
+    case 1: pieces.push_back({d_xyb.p, epx * 12}); d[0] = 3; d[1] = e.ext_rows; d[2] = e.xpad; break;
+    case 2: pieces.push_back({d_stats.p, cells * 16}); d[0] = e.yb; d[1] = e.xb; d[2] = 4; break;
+    case 3: pieces.push_back({d_hfm.p, cells}); d[0] = e.yb; d[1] = e.xb; break;
+    case 4: pieces.push_back({d_ytox.p, tiles}); pieces.push_back({d_ytob.p, tiles}); d[0] = 2; d[1] = e.yt; d[2] = e.xt; break;
+    case 5: pieces.push_back({d_lf.p, cells * 12}); d[0] = 3; d[1] = e.yb; d[2] = e.xb; break;
+    case 6: pieces.push_back({d_lfq.p, cells * 12}); d[0] = 3; d[1] = e.yb; d[2] = e.xb; break;
+    case 7: pieces.push_back({d_coeffs.p, size_t(e.num_groups) * 3 * 65536 * 2}); d[0] = e.num_groups; d[1] = 3; d[2] = 1024; d[3] = 64; break;
+    case 8: pieces.push_back({d_nz.p, cells * 3}); d[0] = 3; d[1] = e.yb; d[2] = e.xb; break;
+    default: {
+      uint64_t total = 0;
+      for (const std::vector<DEncStream>* v : {&m_streams, &a_streams}) for (const DEncStream& s : *v) {
+        counts.push_back(s.count); total += s.count; if (s.count) pieces.push_back({d_tokens.as<uint2>() + s.token_off, size_t(s.count) * 8}); }
+      d[0] = int64_t(counts.size()); d[1] = int64_t(total); d[2] = int64_t(m_streams.size());
+    }
+  }
+  if (dims4) memcpy(dims4, d, sizeof(d));
+  size_t bytes = counts.size() * 4; for (const Piece& p : pieces) bytes += p.n;
+  JXLG_CHECK(out && int64_t(bytes) <= capacity, "stage buffer too small: " + std::to_string(bytes) + " bytes needed");
+  uint8_t* o = static_cast<uint8_t*>(out); if (!counts.empty()) { memcpy(o, counts.data(), counts.size() * 4); o += counts.size() * 4; }
+  for (const Piece& p : pieces) { CUDA_OK(cudaMemcpyAsync(o, p.p, p.n, cudaMemcpyDeviceToHost, st)); o += p.n; }
+  CUDA_OK(cudaStreamSynchronize(st));
+  return int64_t(bytes);
 }
 
 namespace {
@@ -369,6 +408,7 @@ FrameCodes CodesFromHist(const EncPlan& plan, const std::vector<uint64_t>& hist)
 
 std::vector<BandSection> BandEncoder::Finish(const std::vector<uint64_t>& frame_hist) {
   const bool lossless = plan.lossless; const uint32_t nlf = fb.num_lf_groups, ng = fb.num_groups;
+  stages_valid = false;
   FrameCodes codes = CodesFromHist(plan, frame_hist);
   std::vector<uint64_t> bits_m(m_streams.size(), 0), bits_a(ng, 0), dense_off; std::vector<uint8_t> bytes;
   {
@@ -523,6 +563,9 @@ EncStatus BandEncoderFinish(BandSession* s, const uint64_t* hist, size_t words, 
   catch (const std::bad_alloc&) { return EncStatus::OutOfMemory; } catch (const std::exception& ex) { *message = ex.what(); return EncStatus::EncodeError; }
 }
 void BandEncoderDestroy(BandSession* s) { delete s; }
+int64_t BandEncoderDebugStage(BandSession* s, int32_t which, void* out, int64_t capacity, int64_t* dims4, std::string* message) {
+  try { return s->enc->DebugStage(which, out, capacity, dims4); } catch (const std::exception& ex) { *message = ex.what(); return 0; }
+}
 EncStatus AssembleBands(const EncodeRequest& frame, uint32_t frame_flags, const uint64_t* hist, size_t words, const uint8_t* const* blobs, const size_t* sizes, size_t count, std::vector<uint8_t>* file, std::string* message) {
   try {
     EncPlan plan = MakePlan(frame.width, frame.height, frame_flags, frame); std::vector<uint64_t> h(hist, hist + words);

@@ -94,6 +94,8 @@ BandSession* BandEncoderCreate(const EncodeRequest& band, uint32_t* band_flags, 
 EncStatus BandEncoderTokenize(BandSession* s, uint32_t frame_flags, std::vector<uint64_t>* band_hist, std::string* message);
 EncStatus BandEncoderFinish(BandSession* s, const uint64_t* frame_hist, size_t words, std::vector<uint8_t>* sections, float* device_ms, std::string* message);
 void BandEncoderDestroy(BandSession* s);
+// Stage dump of a session between Tokenize and Finish (JxlB200BandEncoderDebugStage): bytes written, or 0 with a message.
+int64_t BandEncoderDebugStage(BandSession* s, int32_t which, void* out, int64_t capacity, int64_t* dims4, std::string* message);
 EncStatus AssembleBands(const EncodeRequest& frame, uint32_t frame_flags, const uint64_t* frame_hist, size_t words, const uint8_t* const* blobs, const size_t* sizes, size_t count,
                         std::vector<uint8_t>* file, std::string* message);
 

@@ -56,6 +56,8 @@ def lib():
         L.jxlo_image_stage_f32.restype = C.c_size_t
         L.jxlo_image_stage_coeffs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
         L.jxlo_image_stage_coeffs.restype = C.c_size_t
+        L.jxlo_image_stage_i32.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]
+        L.jxlo_image_stage_i32.restype = C.c_size_t
         L.jxlo_set_next_icc.argtypes = [C.c_char_p, C.c_size_t]
         for n in ("jxlo_icc_stream_write", "jxlo_icc_stream_read", "jxlo_icc_unpredict"):
             getattr(L, n).argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_char_p, C.c_size_t]
@@ -208,6 +210,15 @@ def decode(data, threads=1, keep_stages=False):
             cnt = lib().jxlo_image_stage_coeffs(img, C.byref(ptr))
             if cnt:
                 d.stages["coeffs"] = np.frombuffer(C.string_at(ptr, cnt * 4), dtype=np.int32).copy().reshape(3, -1)
+            # the integers the file carries: quantised LF [3 (X, Y, B)][yb][xb], hf_mul [yb][xb], ytox / ytob [yt][xt], and the quantiser
+            xb, yb = d.xpad // 8, d.ypad // 8
+            shapes = {"lfq": (3, yb, xb), "hf_mul": (yb, xb), "ytox": (-(-yb // 8), -(-xb // 8)), "ytob": (-(-yb // 8), -(-xb // 8)), "quant": (4,)}
+            for which, name in enumerate(("lfq", "hf_mul", "ytox", "ytob", "quant")):
+                cnt = lib().jxlo_image_stage_i32(img, which, C.byref(ptr))
+                if cnt:
+                    d.stages[name] = np.frombuffer(C.string_at(ptr, cnt * 4), dtype=np.int32).copy().reshape(shapes[name])
+            if "quant" in d.stages:
+                d.global_scale, d.quant_lf, d.x_qm_scale, d.b_qm_scale = (int(v) for v in d.stages.pop("quant"))
         return d
     finally:
         lib().jxlo_image_free(img)
