@@ -94,6 +94,12 @@ class Bits:
             self.u(n, v - (1 << n))
 
 
+def f16_exact(x):
+    """x itself, asserted to survive the trip through binary16 (a field the syntax stores as F16 must carry exactly the value meant)."""
+    assert struct.unpack("<e", struct.pack("<e", x))[0] == x, "%r is not representable as F16" % x
+    return x
+
+
 def pack_signed(v):
     return 2 * v if v >= 0 else -2 * v - 1
 
@@ -180,7 +186,9 @@ def color_encoding(b, color_space=CS_RGB, white_point=WP_D65, primaries=PR_SRGB,
     b.enum(intent)
 
 
-def image_metadata(b, bits=8, exp_bits=0, extra_channels=(), xyb_encoded=False, orientation=1, color=None, intensity_target=None):
+def image_metadata(b, bits=8, exp_bits=0, extra_channels=(), xyb_encoded=False, orientation=1, color=None, intensity_target=None, opsin=None):
+    """opsin = (inverse matrix: 9 values, row-major; bias: 3 values; quant_bias: 4 values), all F16-exact: written as CustomTransformData with
+    default_m = 0 (an XYB-encoded image only)."""
     color = color or {}
     all_default = bits == 8 and exp_bits == 0 and not extra_channels and xyb_encoded and orientation == 1 and not color and intensity_target is None
     b.bool(all_default)
@@ -208,7 +216,13 @@ def image_metadata(b, bits=8, exp_bits=0, extra_channels=(), xyb_encoded=False, 
                 b.bool(False)     # relative_to_max_display
                 b.f16(0.0)        # linear_below
         b.u64(0)                  # extensions
-    b.bool(True)                  # default_m: default opsin inverse matrix and upsampling weights
+    b.bool(opsin is None)         # default_m: default opsin inverse matrix and upsampling weights
+    if opsin is not None:
+        assert xyb_encoded
+        b.bool(False)             # OpsinInverseMatrix.all_default
+        for v in list(opsin[0]) + list(opsin[1]) + list(opsin[2]):
+            b.f16(f16_exact(v))
+        b.u(3, 0)                 # custom_weights_mask: default upsampling weights
 
 
 def passes(b, num_passes=1, shifts=(), downsample=(), last_pass=()):
@@ -228,7 +242,7 @@ FLAG_NOISE, FLAG_PATCHES, FLAG_SPLINES, FLAG_USE_LF_FRAME, FLAG_SKIP_LF_SMOOTHIN
 
 
 def frame_header(b, modular, num_extra=0, xyb_encoded=False, flags=0, group_size_shift=1, num_passes=1, pass_shifts=(), name=b"",
-                 x_qm_scale=3, b_qm_scale=2, crop=None, canvas=None, blend=None, ec_blend=None, is_last=True, save_as_reference=0):
+                 x_qm_scale=3, b_qm_scale=2, crop=None, canvas=None, blend=None, ec_blend=None, is_last=True, save_as_reference=0, gab=False, epf_iters=0):
     """A regular frame without restoration filters. Defaults: full size, last, blend mode Replace. crop = (x0, y0, width, height) with
     canvas = (image width, image height); blend / ec_blend[i] = dict(mode, alpha_channel, clamp, source) (F.2: BlendingInfo)."""
     b.bool(False)                 # all_default
@@ -282,10 +296,19 @@ def frame_header(b, modular, num_extra=0, xyb_encoded=False, flags=0, group_size
     b.u32((("val", 0), ("bits", 4), ("bo", 5, 16), ("bo", 10, 48)), len(name))
     for ch in name:
         b.u(8, ch)
-    # RestorationFilter: not all_default (the default switches gaborish and two EPF iterations on)
+    # RestorationFilter: not all_default (the default switches gaborish and two EPF iterations on); default weights and parameters
     b.bool(False)
-    b.bool(False)                 # gab
-    b.u(2, 0)                     # epf_iters
+    b.bool(gab)
+    if gab:
+        b.bool(False)             # gab_custom
+    b.u(2, epf_iters)
+    if epf_iters:
+        if not modular:
+            b.bool(False)         # epf_sharp_custom
+        b.bool(False)             # epf_weight_custom
+        b.bool(False)             # epf_sigma_custom
+        if modular:
+            b.f16(1.0)            # epf_sigma_for_modular
     b.u64(0)                      # restoration filter extensions
     b.u64(0)                      # frame header extensions
 
@@ -368,9 +391,14 @@ def flat_distribution(n):
     return [4096 // n + (1 if i < 4096 % n else 0) for i in range(n)]
 
 
+class TreeSelect(tuple):
+    """Four symbols of a simple prefix code written with tree-select = 1: code lengths 1, 2, 3, 3 in the order listed."""
+
+
 class EntropyCode:
     """One clustered entropy code. Each cluster is ("flat", n) | ("single", sym) | ("two", s0, s1, p0) for ANS, or a tuple of
-    1..4 symbols for a simple prefix code. ctx_map maps context -> cluster."""
+    1..4 symbols for a simple prefix code (four symbols as a TreeSelect: code lengths 1, 2, 3, 3 in listed order instead of 2, 2, 2, 2).
+    ctx_map maps context -> cluster."""
 
     def __init__(self, ctx_map, clusters, hybrids=None, use_prefix=False, log_alpha=None, lz77=None):
         """lz77: None or dict(min_symbol, min_length, len_hybrid=Hybrid(..)): ctx_map then carries one extra entry, the cluster of the
@@ -411,6 +439,8 @@ class EntropyCode:
             lens = {syms[0]: 1, syms[1]: 1}
         elif n == 3:
             lens = {syms[0]: 1, syms[1]: 2, syms[2]: 2}
+        elif isinstance(syms, TreeSelect):
+            lens = {syms[0]: 1, syms[1]: 2, syms[2]: 3, syms[3]: 3}
         else:
             lens = {s: 2 for s in syms}
         code, codes, prev = 0, {}, 0
@@ -458,7 +488,7 @@ class EntropyCode:
                 for s in syms:
                     b.u(width, s)
                 if len(syms) == 4:
-                    b.bool(False)                       # tree-select: lengths 2,2,2,2
+                    b.bool(isinstance(syms, TreeSelect))   # tree-select: lengths 1,2,3,3 or 2,2,2,2
         else:
             for c in self.clusters:
                 if c[0] == "flat":
@@ -517,25 +547,32 @@ class EntropyCode:
             b.u(nb, ex)
 
 
-def write_permutation_stream(b, perm):
-    """TOC permutation (C.3.2 Lehmer code) with its own 8-context entropy code (flat ANS over 64 symbols)."""
+def permutation_items(perm, skip=0):
+    """(context, value) items of a Lehmer-coded permutation (C.3.2; A.5): `end`, then the Lehmer codes of positions skip .. skip + end - 1
+    (the first `skip` positions must be the identity; trailing zero codes are not written)."""
     n = len(perm)
+    assert list(perm[:skip]) == list(range(skip))
     lehmer, rest = [], list(range(n))
     for p in perm:
         k = rest.index(p)
         lehmer.append(k)
         rest.pop(k)
     end = n
-    while end and lehmer[end - 1] == 0:
+    while end > skip and lehmer[end - 1] == 0:
         end -= 1
     ctx_of = lambda x: min(7, ceil_log2(x + 1))
-    items, prev = [(ctx_of(n), end)], 0
-    for v in lehmer[:end]:
+    items, prev = [(ctx_of(n), end - skip)], 0
+    for v in lehmer[skip:end]:
         items.append((ctx_of(prev), v))
         prev = v
+    return items
+
+
+def write_permutation_stream(b, perm):
+    """TOC permutation (C.3.2 Lehmer code) with its own 8-context entropy code (flat ANS over 64 symbols)."""
     code = EntropyCode([0] * 8, [("flat", 64)], log_alpha=6)
     code.write_header(b)
-    code.write_stream(b, items)
+    code.write_stream(b, permutation_items(perm))
 
 
 # ----------------------------------------------------------------------------- Modular (18181-1 Annex H)
@@ -662,6 +699,36 @@ def rle_copies(items, min_length, dist_sym):
         else:
             out += items[i + 1:j + 1]
         i = j + 1
+    return out
+
+
+def lz77_copies(items, min_length, max_distance, dist_sym):
+    """Greedy LZ77 over the values of (context, value) items: wherever the next >= min_length values repeat values 1 .. max_distance back,
+    one ("copy", context, length, dist_sym(distance)) replaces them (the longest match, the nearest on a tie)."""
+    vals = [it[1] for it in items]
+    out, i, recent = [], 0, {}
+    while i < len(items):
+        best_len, best_d = 0, 0
+        key = tuple(vals[i:i + min_length])
+        if len(key) == min_length:
+            for j in reversed(recent.get(key, [])):
+                d = i - j
+                if d > max_distance:
+                    break
+                n = 0
+                while i + n < len(vals) and n < 1000 and vals[j + n] == vals[i + n]:   # may overlap the copy itself (j + n >= i), as a decoder allows
+                    n += 1
+                if n > best_len:
+                    best_len, best_d = n, d
+        take = best_len if best_len >= min_length else 1
+        if best_len >= min_length:
+            out.append(("copy", items[i][0], best_len, dist_sym(best_d)))
+        else:
+            out.append(items[i])
+        for k in range(i, i + take):
+            if k + min_length <= len(vals):
+                recent.setdefault(tuple(vals[k:k + min_length]), []).append(k)
+        i += take
     return out
 
 
@@ -1133,3 +1200,367 @@ def _write_ac_code_header(b, num_ctx):
     b.bool(True)                   # simple distribution
     b.bool(False)                  # one symbol
     b.u8(0)                        # symbol 0 with probability 4096
+
+
+# ----------------------------------------------------------------------------- VarDCT frame with AC coefficients (A.8, A.9)
+# Varblocks the writer places: strategy -> (cells down, cells across). A.8 names them; A.9: coefficients are stored with the longer side
+# horizontal, so DCT16X8 (two cells down) is stored as one row of two cells, like DCT8X16.
+VARBLOCK = {0: (1, 1), 4: (2, 2), 5: (4, 4), 6: (2, 1), 7: (1, 2)}
+ORDER_ID = {0: 0, 4: 2, 5: 3, 6: 4, 7: 4}       # A.8 coefficient-order ids
+# Dequantisation table of each strategy. The digest lists 17 tables but not their numbering; this is the standard's (DCT8, IDENTITY, DCT2X2,
+# DCT4X4, DCT16, DCT32, DCT8X16, ...), unpinned by the digest.
+QUANT_TABLE = {0: 0, 4: 4, 5: 5, 6: 6, 7: 6}
+QUANT_TABLE_SHAPE = {0: (8, 8), 4: (16, 16), 5: (32, 32), 6: (8, 16)}    # (rows, columns) of coefficients in storage layout
+NUM_ORDERS = 13
+NUM_NZ_BUCKETS, NUM_ZDC = 37, 458
+FREQ_CTX = [0] + list(range(15)) + [15 + i // 2 for i in range(16)] + [23 + i // 4 for i in range(32)]                # A.8 FreqCtx[64]
+# A.8 NumNZCtx[64]; the digest writes "206 x 32", one more than the 64 entries leave room for: 206 fills the remaining 31
+NUM_NZ_CTX = [0, 0, 31, 62, 62] + [93] * 4 + [123] * 4 + [152] * 8 + [180] * 12 + [206] * 31
+assert len(FREQ_CTX) == 64 and len(NUM_NZ_CTX) == 64
+
+# Deliberately wrong rules (vardct_frame(wrong=...)): each encodes the file as a reader with that one misreading would expect it.
+WRONG_RULES = ("preset_offset", "qf_ge", "lf_idx_xyb", "block_ctx_c", "perm_inverted", "perm_no_skip", "nz_bucket_63", "prev_lt", "lz77_multiplier",
+               "nz_floor")
+
+
+def storage_shape(strategy):
+    """(rows, columns) of a varblock's coefficients in storage layout: the shorter side vertical (A.9)."""
+    cy, cx = VARBLOCK[strategy]
+    return 8 * min(cy, cx), 8 * max(cy, cx)
+
+
+def llf_positions(strategy):
+    """Storage positions of the LLF entries (the cy x cx lowest frequencies, taken from the LF image, never coded)."""
+    cy, cx = VARBLOCK[strategy]
+    rows, cols = min(cy, cx), max(cy, cx)
+    return [r * 8 * cols + c for r in range(rows) for c in range(cols)]
+
+
+def coef_index(by, bx, strategy, p, xb):
+    """(cell, k) of storage position p of the varblock whose first cell is (by, bx): position p lives in the (p // 64)-th covered cell in raster
+    order of the block (the decoder's debug layout of quantised coefficients: [channel][cell][64])."""
+    bw = VARBLOCK[strategy][1]
+    j = p >> 6
+    return (by + j // bw) * xb + bx + j % bw, p & 63
+
+
+def nonzero_ctx(pred, wrong=None):
+    """A.8 NonZeroCtx: n < 8 ? n : n < 64 ? 4 + n / 2 : 36."""
+    limit = 63 if wrong == "nz_bucket_63" else 64
+    return pred if pred < 8 else (4 + pred // 2 if pred < limit else 36)
+
+
+def zero_density_ctx(nz, k, cells, log_cells):
+    return (NUM_NZ_CTX[min(63, (nz + cells - 1) >> log_cells)] + FREQ_CTX[min(63, k >> log_cells)]) * 2
+
+
+class BlockCtxMap:
+    """LfGlobal's BlockCtxMap (A.8): thresholds on the quantised LF of X, Y and B, thresholds on hf_mul, and a map of
+    3 x 13 x (#qf + 1) x n_lf entries to block contexts. lf_thr = (X, Y, B) lists; qf_thr values >= 1."""
+
+    def __init__(self, lf_thr, qf_thr, ctx_map):
+        self.lf_thr, self.qf_thr, self.ctx_map = [list(t) for t in lf_thr], list(qf_thr), [int(v) for v in ctx_map]
+        self.n_lf = (len(self.lf_thr[0]) + 1) * (len(self.lf_thr[1]) + 1) * (len(self.lf_thr[2]) + 1)
+        assert len(self.ctx_map) == 3 * NUM_ORDERS * (len(self.qf_thr) + 1) * self.n_lf
+        self.num_ctx = max(self.ctx_map) + 1
+
+    def lf_idx(self, qx, qy, qb, wrong=None):
+        ix, iy, ib = (sum(1 for t in thr if q > t) for thr, q in zip(self.lf_thr, (qx, qy, qb)))
+        ny, nb = len(self.lf_thr[1]) + 1, len(self.lf_thr[2]) + 1
+        if wrong == "lf_idx_xyb":
+            return (ix * ny + iy) * nb + ib
+        return (ix * nb + ib) * ny + iy                 # nested X, B, Y
+
+    def context(self, lf_idx, hf_mul, order, c, wrong=None):
+        qf_idx = sum(1 for t in self.qf_thr if (hf_mul >= t if wrong == "qf_ge" else hf_mul > t))
+        cc = c if wrong == "block_ctx_c" else (c ^ 1 if c < 2 else 2)     # the map lists Y, X, B
+        return self.ctx_map[((cc * NUM_ORDERS + order) * (len(self.qf_thr) + 1) + qf_idx) * self.n_lf + lf_idx]
+
+    def write(self, b):
+        b.bool(False)                                   # not the default map
+        for thr in self.lf_thr:
+            b.u(4, len(thr))
+            for t in thr:
+                b.u32((("bits", 4), ("bo", 8, 16), ("bo", 16, 272), ("bo", 32, 65808)), pack_signed(t))
+        b.u(4, len(self.qf_thr))
+        for t in self.qf_thr:
+            b.u32((("bits", 2), ("bo", 3, 4), ("bo", 5, 12), ("bo", 8, 44)), t - 1)
+        nbits = ceil_log2(self.num_ctx)
+        assert nbits <= 3, "the simple context map holds at most 8 block contexts"
+        b.bool(True)                                    # simple context map
+        b.u(2, nbits)
+        for v in self.ctx_map:
+            b.u(nbits, v)
+
+
+def vardct_frame(xsize, ysize, lfq, blocks, ytox, ytob, coeffs, sharp=None, lf_dequant=None, global_scale=32768, quant_lf=64, extra_precision=0,
+                 bctx=None, cfl=None, tables=None, presets=None, orders=None, pass_shift=None, code="ans", opsin=None, skip_smoothing=True,
+                 gab=False, epf_iters=0, x_qm_scale=3, b_qm_scale=2, wrong=None):
+    """A complete XYB VarDCT image (codestream) whose every integer is the caller's:
+      lfq: quantised LF, three (X, Y, B) integer arrays of yb x xb cells (row-major nested lists or numpy);
+      blocks: [(by, bx, strategy, hf_mul)] covering every cell once, strategies from VARBLOCK, never across a 256-px group border;
+      ytox, ytob: CfL factors per 64 x 64 tile (-128 .. 127); sharp: EPF sharpness per cell (default 0);
+      coeffs: quantised coefficients [3 (X, Y, B)][yb * xb][64] in the layout of coef_index(); LLF positions must be 0. With two passes
+        (pass_shift = s) the first pass carries coeffs >> s and the second the rest, so the decoded sum is `coeffs`.
+    LfGlobal: lf_dequant = three F16 values (the stored F16, i.e. 128 x the multiplier) or None; global_scale, quant_lf; bctx = BlockCtxMap or None
+      (default map); cfl = (colour_factor, base_x, base_b, x_factor_lf, b_factor_lf) or None.
+    HfGlobal: tables = {table id: [3 lists of band parameters (X, Y, B), first band in the file's units x 64] | "raw"}: every listed table is
+      written in mode 6 (DCT bands) or mode 7 (RAW, constant weights), the others as Library; None writes all_default. presets = per-group preset index list (num_hf_presets = max + 1);
+      orders = {order id: [pass][3 channels] permutation of range(size) whose first size/64 entries are the identity}: coefficient order =
+      natural[perm[k]].
+    code: "ans" (clustered ANS, 8 clusters), "prefix" (simple prefix codes; every value must be <= 3) or "lz77" (ANS + LZ77 copies at
+      distances 1 .. 160).
+    opsin = (inverse matrix, bias, quant_bias) as image_metadata(). wrong: one of WRONG_RULES."""
+    import oracle_py                                    # natural coefficient orders only (jxlo_natural_order); everything else is this writer's
+    import numpy as np
+    assert wrong is None or wrong in WRONG_RULES
+    xb, yb = -(-xsize // 8), -(-ysize // 8)
+    xg, yg = -(-xb // 32), -(-yb // 32)
+    xl, yl = -(-xb // 256), -(-yb // 256)
+    ngroups, nlf = xg * yg, xl * yl
+    npasses = 1 if pass_shift is None else 2
+    lfq = [np.asarray(p, dtype=np.int64) for p in lfq]
+    ytox, ytob = np.asarray(ytox, dtype=np.int64), np.asarray(ytob, dtype=np.int64)
+    sharp = np.zeros((yb, xb), np.int64) if sharp is None else np.asarray(sharp, dtype=np.int64)
+    coeffs = np.asarray(coeffs, dtype=np.int64).reshape(3, yb * xb, 64)
+    presets = list(presets) if presets is not None else [0] * ngroups
+    num_presets = max(presets) + 1
+    assert len(presets) == ngroups and (num_presets == 1 or num_presets <= (1 << ceil_log2(ngroups)))
+    # ---- cell map
+    first = {}
+    owner = np.full((yb, xb), -1, np.int64)
+    for i, (by, bx, s, hm) in enumerate(blocks):
+        cy, cx = VARBLOCK[s]
+        assert 1 <= hm <= 256 and by + cy <= yb and bx + cx <= xb and by // 32 == (by + cy - 1) // 32 and bx // 32 == (bx + cx - 1) // 32, (by, bx, s)
+        assert (owner[by:by + cy, bx:bx + cx] == -1).all(), "overlapping blocks"
+        owner[by:by + cy, bx:bx + cx] = i
+        first[(by, bx)] = i
+    assert (owner >= 0).all(), "cells without a block"
+
+    def natural(order_id):
+        n = {0: 64, 2: 256, 3: 1024, 4: 128}[order_id]
+        out = np.zeros(n, np.uint32)
+        assert oracle_py.lib().jxlo_natural_order(order_id, out.ctypes.data) == n
+        return [int(v) for v in out]
+
+    orders = orders or {}
+    used = [sorted(orders) if orders else [] for _ in range(npasses)]
+    coding_order = {}                                   # (pass, order id, channel) -> storage positions in coding order
+    for o in (0, 2, 3, 4):
+        nat = natural(o)
+        for p in range(npasses):
+            for c in range(3):
+                perm = orders[o][p][c] if o in orders else list(range(len(nat)))
+                coding_order[(p, o, c)] = [nat[perm[k]] for k in range(len(nat))]
+
+    # ---- entropy code of the AC coefficients: 8 clusters, each with its own hybrid-uint configuration and alphabet size
+    nbctx = bctx.num_ctx if bctx is not None else 15
+    num_ctx = 495 * num_presets * nbctx
+    ctx_cluster = [((c * 5) ^ (c >> 3) ^ (c >> 6)) % 8 for c in range(num_ctx)]    # adjacent contexts fall into different clusters
+    if code == "prefix":
+        # values 0..3: the first two configurations give tokens 0, 1, 2 (+ 1 extra bit for 2, 3), the others code 0..3 as tokens 0..3
+        hybrids = [Hybrid(0, 0, 0), Hybrid(1, 0, 0), Hybrid(2, 0, 0), Hybrid(1, 1, 0), Hybrid(1, 0, 1), Hybrid(2, 1, 0), Hybrid(2, 0, 1), Hybrid(3, 1, 1)]
+    else:
+        hybrids = [Hybrid(4, 2, 0), Hybrid(3, 1, 1), Hybrid(2, 0, 0), Hybrid(4, 1, 2), Hybrid(1, 0, 0), Hybrid(3, 2, 1), Hybrid(0, 0, 0), Hybrid(4, 0, 0)]
+    lz = code == "lz77"
+
+    def default_block_ctx(c, order_id):                 # A.8 default map: 15 block contexts
+        d = [0, 1, 2, 2, 3, 3, 4, 5, 6, 6, 6, 6, 6, 7, 8, 9, 9, 10, 11, 12, 13, 14, 14, 14, 14, 14, 7, 8, 9, 9, 10, 11, 12, 13, 14, 14, 14, 14, 14]
+        cc = c if wrong == "block_ctx_c" else (c ^ 1 if c < 2 else 2)
+        return d[cc * NUM_ORDERS + order_id]
+
+    def group_items(p, g):
+        """(context, value) items of pass p of group g (A.8 PassGroup AC decode)."""
+        gy, gx = divmod(g, xg)
+        items = []
+        nzc = np.zeros((3, 32, 32), np.int64)
+        offset = 0 if wrong == "preset_offset" else 495 * nbctx * presets[g]
+        for cy0 in range(32):
+            for cx0 in range(32):
+                by, bx = gy * 32 + cy0, gx * 32 + cx0
+                if (by, bx) not in first:
+                    continue
+                _, _, s, hm = blocks[first[(by, bx)]]
+                cy, cx = VARBLOCK[s]
+                cells, size = cy * cx, cy * cx * 64
+                log_cells = cells.bit_length() - 1
+                o = ORDER_ID[s]
+                for c in (1, 0, 2):
+                    if bctx is not None:
+                        li = bctx.lf_idx(lfq[0][by, bx], lfq[1][by, bx], lfq[2][by, bx], wrong)
+                        bc = bctx.context(li, hm, o, c, wrong)
+                    else:
+                        bc = default_block_ctx(c, o)
+                    if cx0 == 0:
+                        pred = 32 if cy0 == 0 else nzc[c, cy0 - 1, cx0]
+                    elif cy0 == 0:
+                        pred = nzc[c, cy0, cx0 - 1]
+                    else:
+                        pred = (nzc[c, cy0 - 1, cx0] + nzc[c, cy0, cx0 - 1] + 1) // 2
+                    order = coding_order[(p, o, c)]
+                    vals = []
+                    for k in range(size):
+                        cell, kk = coef_index(by, bx, s, order[k], xb)
+                        q = int(coeffs[c, cell, kk])
+                        if k < cells:
+                            assert q == 0, "LLF positions carry no coefficient"
+                            continue
+                        if npasses == 2:
+                            q = q >> pass_shift if p == 0 else q - ((q >> pass_shift) << pass_shift)
+                        vals.append(q)
+                    nz = sum(1 for v in vals if v)
+                    items.append((offset + nonzero_ctx(int(pred), wrong) * nbctx + bc, nz))
+                    per_cell = nz // cells if wrong == "nz_floor" else -(-nz // cells)
+                    nzc[c, cy0:cy0 + cy, cx0:cx0 + cx] = per_cell
+                    prev = int(nz < size // 16) if wrong == "prev_lt" else int(nz <= size // 16)
+                    left = nz
+                    histo = offset + nbctx * NUM_NZ_BUCKETS + NUM_ZDC * bc
+                    for i, v in enumerate(vals):
+                        if left == 0:
+                            break
+                        items.append((histo + zero_density_ctx(left, cells + i, cells, log_cells) + prev, pack_signed(v)))
+                        prev = int(v != 0)
+                        left -= prev
+        return items
+
+    streams = {(p, g): group_items(p, g) for p in range(npasses) for g in range(ngroups)}
+    if lz:
+        # AC rule: distance = symbol + 1 (no multiplier, no special-distance table). Distances up to 160 give symbols on both sides of 120,
+        # where a reader that sent AC distances through Modular's table (symbols < 120) or its offset (symbol - 119) would go astray.
+        dist_sym = (lambda d: d + 119) if wrong == "lz77_multiplier" else (lambda d: d - 1)
+        streams = {k: lz77_copies(v, 3, 160, dist_sym) for k, v in streams.items()}
+    # alphabets: every cluster gets its own size, larger than any token it has to code
+    tok_max = 0
+    for items in streams.values():
+        for it in items:
+            if it[0] != "copy":
+                tok_max = max(tok_max, hybrids[ctx_cluster[it[0]]].encode(it[1])[0])
+    if code == "prefix":
+        assert tok_max <= 3, "prefix-code case: values must stay <= 3"
+        # clusters 0 and 1 (tokens 0..2): an unused fourth symbol sets the alphabet size; the rest code tokens 0..3. Lengths 1, 2, 3, 3 in listed
+        # order, a different order per cluster, except cluster 2 (2, 2, 2, 2): no two clusters share a code
+        clusters = [TreeSelect((0, 1, 2, 5)), TreeSelect((2, 0, 1, 7)), (0, 1, 2, 3), TreeSelect((3, 2, 1, 0)), TreeSelect((1, 3, 0, 2)),
+                    TreeSelect((2, 0, 3, 1)), TreeSelect((0, 2, 1, 3)), TreeSelect((3, 0, 2, 1))]
+        ac_code = EntropyCode(ctx_cluster, clusters, hybrids=hybrids, use_prefix=True)
+    elif lz:
+        assert tok_max < 224
+        lzp = dict(min_symbol=224, min_length=3, len_hybrid=Hybrid(0, 0, 0))
+        ac_code = EntropyCode(ctx_cluster + [5], [("flat", 240 + 2 * k) for k in range(8)], hybrids=hybrids, log_alpha=8, lz77=lzp)
+    else:
+        ac_code = EntropyCode(ctx_cluster, [("flat", tok_max + 1 + 3 * k) for k in range(8)], hybrids=hybrids, log_alpha=8)
+
+    # ---- headers
+    b = Bits()
+    b.u(16, 0x0AFF)
+    size_header(b, xsize, ysize)
+    image_metadata(b, xyb_encoded=True, opsin=opsin)
+    b.pad_to_byte()
+    frame_header(b, modular=False, xyb_encoded=True, flags=FLAG_SKIP_LF_SMOOTHING if skip_smoothing else 0, num_passes=npasses,
+                 pass_shifts=(pass_shift,) if npasses == 2 else (), x_qm_scale=x_qm_scale, b_qm_scale=b_qm_scale, gab=gab, epf_iters=epf_iters)
+    single = ngroups == 1 and npasses == 1
+    sections = []
+    s = Bits()
+    # ---- LfGlobal
+    s.bool(lf_dequant is None)                          # LfChannelDequantization.all_default
+    if lf_dequant is not None:
+        for v in lf_dequant:
+            s.f16(f16_exact(v))
+    s.u32((("bo", 11, 1), ("bo", 11, 2049), ("bo", 12, 4097), ("bo", 16, 8193)), global_scale)
+    s.u32((("val", 16), ("bo", 5, 1), ("bo", 8, 1), ("bo", 16, 1)), quant_lf)
+    if bctx is None:
+        s.bool(True)
+    else:
+        bctx.write(s)
+    s.bool(cfl is None)                                 # ColorCorrelation.all_default
+    if cfl is not None:
+        s.u32((("val", 84), ("val", 256), ("bo", 8, 2), ("bo", 16, 258)), cfl[0])
+        s.f16(f16_exact(cfl[1]))
+        s.f16(f16_exact(cfl[2]))
+        s.u(8, cfl[3])
+        s.u(8, cfl[4])
+    s.bool(True)                                        # global MA tree
+    tree = Leaf(0, 5)
+    write_tree(s, tree)
+    mcode = EntropyCode([0], [("flat", 256)], hybrids=[Hybrid(4, 2, 0)], log_alpha=8)
+    mcode.write_header(s)
+
+    def next_section():
+        nonlocal s
+        if not single:
+            sections.append(s.bytes())
+            s = Bits()
+
+    next_section()
+    # ---- LfGroups: LF coefficients (Y, X, B), HF metadata
+    for li in range(nlf):
+        ly, lx = divmod(li, xl)
+        c0, r0 = lx * 256, ly * 256
+        w, h = min(256, xb - c0), min(256, yb - r0)
+        s.u(2, extra_precision)
+        group_header(s)
+        sub = lambda a: [[int(v) for v in row[c0:c0 + w]] for row in a[r0:r0 + h]]
+        mcode.write_stream(s, modular_items(tree, [sub(lfq[1]), sub(lfq[0]), sub(lfq[2])], 1 + li))
+        listed = []
+        for y in range(r0, r0 + h):
+            for x in range(c0, c0 + w):
+                if (y, x) in first:
+                    listed.append(blocks[first[(y, x)]])
+        s.u(ceil_log2(w * h), len(listed) - 1)
+        group_header(s)
+        t0, tw, th = c0 // 8, -(-w // 8), -(-h // 8)
+        tiles = lambda a: [[int(v) for v in row[t0:t0 + tw]] for row in a[r0 // 8:r0 // 8 + th]]
+        info = [[bl[2] for bl in listed], [bl[3] - 1 for bl in listed]]
+        mcode.write_stream(s, modular_items(tree, [tiles(ytox), tiles(ytob), info, sub(sharp)], 1 + 2 * nlf + li))
+        next_section()
+    # ---- HfGlobal
+    s.bool(tables is None)                              # dequantisation matrices all_default
+    if tables is not None:
+        for t in range(17):
+            if t not in tables:
+                s.u(3, 0)                               # Library
+                continue
+            if tables[t] == "raw":                      # RAW: F16 denominator, then the weights as a 3-channel Modular image (A.8)
+                rows, cols = QUANT_TABLE_SHAPE[t]
+                s.u(3, 7)
+                s.f16(1.0 / 64)
+                group_header(s)
+                mcode.write_stream(s, modular_items(tree, [[[100] * cols for _ in range(rows)]] * 3, 1 + 3 * nlf + t))
+                continue
+            s.u(3, 6)                                   # DCT bands
+            nb = len(tables[t][0])
+            s.u(4, nb - 1)
+            for c in range(3):
+                assert len(tables[t][c]) == nb
+                for i, v in enumerate(tables[t][c]):
+                    s.f16(f16_exact(v / 64.0 if i == 0 else v))
+    s.u(ceil_log2(ngroups), num_presets - 1)
+    for p in range(npasses):
+        mask = sum(1 << o for o in used[p])
+        s.u32((("val", 0x5F), ("val", 0x13), ("val", 0), ("bits", 13)), mask)
+        if mask:
+            items = []
+            for o in used[p]:
+                for c in range(3):
+                    perm = list(orders[o][p][c])
+                    n = len(perm)
+                    if wrong == "perm_inverted":
+                        inv = [0] * n
+                        for k, v in enumerate(perm):
+                            inv[v] = k
+                        perm = inv
+                    items += permutation_items(perm, 0 if wrong == "perm_no_skip" else n // 64)
+            pcode = EntropyCode([0] * 8, [("flat", 64)], log_alpha=6)
+            pcode.write_header(s)
+            pcode.write_stream(s, items)
+        ac_code.write_header(s)
+    next_section()
+    # ---- PassGroups, pass-major
+    for p in range(npasses):
+        for g in range(ngroups):
+            s.u(ceil_log2(num_presets), presets[g])
+            ac_code.write_stream(s, streams[(p, g)])
+            next_section()
+    if single:
+        sections = [s.bytes()]
+    toc(b, [len(x) for x in sections])
+    return b.bytes() + b"".join(sections)

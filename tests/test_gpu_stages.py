@@ -119,12 +119,14 @@ def pq_to_linear(e):
     return np.sign(e) * (np.maximum(p - PQ_C1, 0) / (PQ_C2 - PQ_C3 * p)) ** (1 / PQ_M1)
 
 
-def xyb_to_output(xyb, primaries=1, tf=TF_SRGB, intensity_target=255.0):
-    """xyb: [3][h][w] float64 -> [h][w][3] colour samples in the output encoding (before the sample type)."""
+def xyb_to_output(xyb, primaries=1, tf=TF_SRGB, intensity_target=255.0, opsin_inv=OPSIN_INV, opsin_bias=(OPSIN_BIAS,) * 3):
+    """xyb: [3][h][w] float64 -> [h][w][3] colour samples in the output encoding (before the sample type). opsin_inv: the 3 x 3 inverse
+    opsin matrix; opsin_bias: the three (positive) biases b of m = (g + cbrt(b))^3 - b."""
     X, Y, B = xyb
-    cb = np.cbrt(OPSIN_BIAS)
-    mix = np.stack([(Y + X + cb) ** 3 - OPSIN_BIAS, (Y - X + cb) ** 3 - OPSIN_BIAS, (B + cb) ** 3 - OPSIN_BIAS], axis=-1)
-    lin = mix @ (linear_srgb_to(primaries) @ OPSIN_INV).T * (255.0 / intensity_target)
+    bias = np.asarray(opsin_bias, np.float64)
+    cb = np.cbrt(bias)
+    mix = np.stack([(Y + X + cb[0]) ** 3 - bias[0], (Y - X + cb[1]) ** 3 - bias[1], (B + cb[2]) ** 3 - bias[2]], axis=-1)
+    lin = mix @ (linear_srgb_to(primaries) @ np.asarray(opsin_inv, np.float64).reshape(3, 3)).T * (255.0 / intensity_target)
     return transfer(lin, tf, intensity_target)
 
 
