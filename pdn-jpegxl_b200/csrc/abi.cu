@@ -3,7 +3,7 @@
 //   LoadImage  restates DecoderReadImage           N/Decoder/JxlDecoder.cpp:796-852 (callback order :461-784, :389-400)
 //   SaveImage  restates EncoderWriteImage          N/Encoder/JxlEncoder.cpp:147-392 and OutputProcessor (N/Encoder/OutputProcessor.cpp:18-151)
 //   error text restates SetErrorMessage            N/Common.cpp:18-53
-// No exception crosses the boundary; every failure becomes a status code (+ optional message).
+// No exception crosses the boundary: Guard turns every failure into a status code (+ optional message).
 #include "../../include/JxlFileTypeIO.h"
 #include "engine.h"
 #include "dev/kernels.h"
@@ -36,6 +36,21 @@ void SetErrorMessage(ErrorInfo* ei, const std::string& s) { if (s.size() > 255) 
 
 thread_local StageTimes g_last_times;
 
+// Runs one engine call and keeps its stage times for JxlB200LastStageTimes (zero when the call fails).
+template <class Result, class Request> Result WithTimes(Result (*call)(const Request&), const Request& req) { g_last_times = StageTimes(); Result r = call(req); g_last_times = r.times; return r; }
+
+// The one place where the engine's exceptions become what a C caller sees. `body` returns the status of a call that did not throw;
+// a failure becomes StatusError's status, OutOfMemory, or DecodeError / EncodeError, with the exception's text in ErrorInfo.
+struct Decoding { static const int32_t kOutOfMemory = DecoderStatus_OutOfMemory, kError = DecoderStatus_DecodeError; };
+struct Encoding { static const int32_t kOutOfMemory = EncoderStatus_OutOfMemory, kError = EncoderStatus_EncodeError; };
+template <class Codec, class F> int32_t Guard(ErrorInfo* ei, F&& body) {
+  try { return body(); }
+  catch (const StatusError& e) { SetErrorMessage(ei, std::string(e.what())); return e.status; }
+  catch (const std::bad_alloc&) { return Codec::kOutOfMemory; }
+  catch (const std::exception& e) { SetErrorMessage(ei, std::string(e.what())); return Codec::kError; }
+  catch (...) { return Codec::kError; }
+}
+
 const int32_t kSOk = 0, kEPointer = int32_t(0x80004003), kEAbort = int32_t(0x80004004), kEOutOfMemory = int32_t(0x8007000E);
 
 // N/Encoder/OutputProcessor.cpp: <= 64 KiB chunks, sticky first failure, progress tick per buffer request.
@@ -61,6 +76,8 @@ class OutputProcessor {
 };
 
 bool ReportProgress(ProgressProc p, int32_t pct) { return p ? p(pct) : true; }
+// malloc'ed copies for the caller (freed with JxlB200Free)
+void* CopyOut(const void* p, size_t n) { void* m = malloc(n ? n : 1); if (!m) throw std::bad_alloc(); if (n) memcpy(m, p, n); return m; }
 
 }  // namespace
 
@@ -70,11 +87,9 @@ uint32_t GetLibJxlVersion(void) { return (0u << 24) | (11u << 16) | (1u << 8); }
 
 DecoderStatus LoadImage(DecoderCallbacks* callbacks, const uint8_t* data, size_t dataSize, ErrorInfo* errorInfo) {
   if (!callbacks || !data) return DecoderStatus_NullParameter;
-  try {
+  return Guard<Decoding>(errorInfo, [&] {
     // pass 1: basic info, colour profile, metadata boxes (N/Decoder/JxlDecoder.cpp:412-793)
-    DecodeResult info = ParseInfo(data, dataSize);
-    if (info.status != Status::Ok) { SetErrorMessage(errorInfo, info.message); return DecoderStatus(info.status); }
-    const ParsedInfo& pi = info.info;
+    const ParsedInfo pi = ParseInfo(data, dataSize);
     callbacks->setBasicInfo(int32_t(pi.width), int32_t(pi.height), pi.format, pi.sample_type, pi.has_alpha);
     if (pi.known_profile >= 0) { if (!callbacks->setKnownColorProfile(pi.known_profile)) return DecoderStatus_CreateMetadataError; }
     else if (!pi.icc.empty()) { std::vector<uint8_t> icc = pi.icc; if (!callbacks->setIccProfile(icc.data(), icc.size())) return DecoderStatus_CreateMetadataError; }
@@ -84,21 +99,18 @@ DecoderStatus LoadImage(DecoderCallbacks* callbacks, const uint8_t* data, size_t
     }
     // pass 2: the frame (N/Decoder/JxlDecoder.cpp:217-410)
     DecodeRequest req; req.data = data; req.size = dataSize;
-    DecodeResult res = DecodeOnGpu(req); g_last_times = res.times;
-    if (res.status != Status::Ok) { SetErrorMessage(errorInfo, res.message); return DecoderStatus(res.status); }
+    const DecodeResult res = WithTimes(DecodeOnGpu, req);
     // layer name: length passed includes the NUL terminator (N/Decoder/JxlDecoder.cpp:274,366-370 — Appendix C-3)
     std::vector<char> name; if (!res.info.frame_name.empty()) { name.assign(res.info.frame_name.begin(), res.info.frame_name.end()); name.push_back(0); }
     if (!callbacks->setLayerData(res.pixels, name.empty() ? nullptr : name.data(), name.size())) return DecoderStatus_CreateLayerError;
-  } catch (const std::bad_alloc&) { return DecoderStatus_OutOfMemory; }
-  catch (const std::exception& e) { SetErrorMessage(errorInfo, e.what()); return DecoderStatus_DecodeError; }
-  catch (...) { return DecoderStatus_DecodeError; }
-  return DecoderStatus_Ok;
+    return DecoderStatus_Ok;
+  });
 }
 
 EncoderStatus SaveImage(const BitmapData* bitmap, const EncoderOptions* options, const EncoderImageMetadata* metadata, IOCallbacks* callbacks, ErrorInfo* errorInfo, ProgressProc progressCallback) {
   if (!bitmap || !options || !callbacks || !metadata) return EncoderStatus_NullParameter;
   if (errorInfo) errorInfo->errorMessage[0] = 0;   // the managed caller passes it uninitialised (I/JpegXLNative.cs:102)
-  try {
+  return Guard<Encoding>(errorInfo, [&]() -> EncoderStatus {
     // progress sequence 0, 5, 15, 20, 25, then +5 per output buffer from 30 capped at 90, then 95 (N/Encoder/JxlEncoder.cpp:162-362)
     if (!ReportProgress(progressCallback, 0)) return EncoderStatus_UserCanceled;
     EncodeRequest req; req.bgra = bitmap->scan0; req.width = bitmap->width; req.height = bitmap->height; req.stride = bitmap->stride;
@@ -109,8 +121,7 @@ EncoderStatus SaveImage(const BitmapData* bitmap, const EncoderOptions* options,
     if (!ReportProgress(progressCallback, 20)) return EncoderStatus_UserCanceled;
     if (!ReportProgress(progressCallback, 25)) return EncoderStatus_UserCanceled;
     OutputProcessor out(callbacks); out.InitializeProgressReporting(progressCallback, 30, 90, 5);
-    EncodeResult res = EncodeOnGpu(req); g_last_times = res.times;
-    if (res.status != EncStatus::Ok) { SetErrorMessage(errorInfo, res.message); return EncoderStatus(res.status); }
+    const EncodeResult res = WithTimes(EncodeOnGpu, req);
     // libjxl streams output while encoding; the engine produces the file after the kernels finish and streams it the same way
     size_t half = res.file.size() / 2;
     bool ok = out.Write(res.file.data(), half);
@@ -118,27 +129,27 @@ EncoderStatus SaveImage(const BitmapData* bitmap, const EncoderOptions* options,
     if (!ReportProgress(progressCallback, 95)) return EncoderStatus_UserCanceled;
     ok = out.Write(res.file.data() + half, res.file.size() - half);
     if (!ok) { EncoderStatus st = out.GetWriteStatus(); if (st != EncoderStatus_Ok) return st; SetErrorMessage(errorInfo, "JxlEncoderFlushInput failed."); return EncoderStatus_EncodeError; }
-  } catch (const std::bad_alloc&) { return EncoderStatus_OutOfMemory; }
-  catch (...) { return EncoderStatus_EncodeError; }
-  return EncoderStatus_Ok;
+    return EncoderStatus_Ok;
+  });
 }
 
 DecoderStatus JxlB200PeekInfo(const uint8_t* data, size_t dataSize, int32_t* info, ErrorInfo* errorInfo) {
   if (!data || !info) return DecoderStatus_NullParameter;
-  DecodeResult r = ParseInfo(data, dataSize); if (r.status != Status::Ok) { SetErrorMessage(errorInfo, r.message); return DecoderStatus(r.status); }
-  info[0] = int32_t(r.info.width); info[1] = int32_t(r.info.height); info[2] = r.info.format; info[3] = r.info.sample_type; info[4] = r.info.has_alpha; info[5] = r.info.num_channels; info[6] = r.info.known_profile; info[7] = r.info.is_container;
-  return DecoderStatus_Ok;
+  return Guard<Decoding>(errorInfo, [&] {
+    const ParsedInfo r = ParseInfo(data, dataSize);
+    info[0] = int32_t(r.width); info[1] = int32_t(r.height); info[2] = r.format; info[3] = r.sample_type; info[4] = r.has_alpha; info[5] = r.num_channels; info[6] = r.known_profile; info[7] = r.is_container;
+    return DecoderStatus_Ok;
+  });
 }
 
 DecoderStatus JxlB200LoadImageBgra(const uint8_t* data, size_t dataSize, uint8_t* surface, size_t surfaceBytes, int32_t* width, int32_t* height, ErrorInfo* errorInfo) {
   if (!data || !surface) return DecoderStatus_NullParameter;
-  try {
-    DecodeRequest req; req.data = data; req.size = dataSize; req.bgra = true; DecodeResult res = DecodeOnGpu(req); g_last_times = res.times;
-    if (res.status != Status::Ok) { SetErrorMessage(errorInfo, res.message); return DecoderStatus(res.status); }
+  return Guard<Decoding>(errorInfo, [&] {
+    DecodeRequest req; req.data = data; req.size = dataSize; req.bgra = true; const DecodeResult res = WithTimes(DecodeOnGpu, req);
     if (surfaceBytes < res.pixel_bytes) { SetErrorMessage(errorInfo, "surface buffer too small"); return DecoderStatus_InvalidParameter; }
     memcpy(surface, res.pixels, res.pixel_bytes); if (width) *width = int32_t(res.out_width); if (height) *height = int32_t(res.out_height);
-  } catch (const std::bad_alloc&) { return DecoderStatus_OutOfMemory; } catch (const std::exception& e) { SetErrorMessage(errorInfo, e.what()); return DecoderStatus_DecodeError; } catch (...) { return DecoderStatus_DecodeError; }
-  return DecoderStatus_Ok;
+    return DecoderStatus_Ok;
+  });
 }
 
 // The managed layer repack as a GPU epilogue (I/DecoderLayerData.cs:26-125 and its eighteen Set*ImageData variants): the decoder's
@@ -147,10 +158,9 @@ DecoderStatus JxlB200LoadImageBgra(const uint8_t* data, size_t dataSize, uint8_t
 DecoderStatus JxlB200LoadImageLayers(const uint8_t* data, size_t dataSize, uint8_t* color, size_t colorBytes, uint8_t* transparency, size_t transparencyBytes,
                                      int32_t* info6, ErrorInfo* errorInfo) {
   if (!data || !color) return DecoderStatus_NullParameter;
-  void* d_color = nullptr; void* d_alpha = nullptr; void* pool_c = nullptr; void* pool_a = nullptr; size_t bytes_c = 0, bytes_a = 0; DecoderStatus rc = DecoderStatus_Ok;   // cached device buffers (engine pool)
-  try {
-    DecodeRequest req; req.data = data; req.size = dataSize; req.device_output = true; DecodeResult res = DecodeOnGpu(req); g_last_times = res.times;
-    if (res.status != Status::Ok) { SetErrorMessage(errorInfo, res.message); return DecoderStatus(res.status); }
+  void* d_color = nullptr; void* d_alpha = nullptr; void* pool_c = nullptr; void* pool_a = nullptr; size_t bytes_c = 0, bytes_a = 0;   // cached device buffers (engine pool)
+  const DecoderStatus rc = Guard<Decoding>(errorInfo, [&] {
+    DecodeRequest req; req.data = data; req.size = dataSize; req.device_output = true; const DecodeResult res = WithTimes(DecodeOnGpu, req);
     const ParsedInfo& pi = res.info; const size_t npix = size_t(res.out_width) * res.out_height; const size_t bps = pi.sample_type == 0 ? 1 : pi.sample_type == 3 ? 4 : 2;
     if (pi.format == 2 && pi.sample_type != 0) { SetErrorMessage(errorInfo, "unsupported CMYK channel representation"); return DecoderStatus_UnsupportedChannelFormat; }   // I/DecoderLayerData.cs:127-162
     const size_t dst_ch = pi.format == 2 ? 4 : 3, need_color = npix * dst_ch * bps, need_alpha = pi.has_alpha ? npix : 0;
@@ -161,9 +171,10 @@ DecoderStatus JxlB200LoadImageLayers(const uint8_t* data, size_t dataSize, uint8
       LaunchSplitLayers(res.pixels, d_color, static_cast<uint8_t*>(d_alpha), npix, pi.format, pi.sample_type, pi.has_alpha, 0);
       cudaError_t e = cudaMemcpy(color, d_color, need_color, cudaMemcpyDeviceToHost);
       if (e == cudaSuccess && need_alpha) e = cudaMemcpy(transparency, d_alpha, need_alpha, cudaMemcpyDeviceToHost);
-      if (e != cudaSuccess) { SetErrorMessage(errorInfo, std::string("CUDA: ") + cudaGetErrorString(e)); rc = DecoderStatus_DecodeError; }
+      JXLG_CHECK(e == cudaSuccess, std::string("CUDA: ") + cudaGetErrorString(e));
     }
-  } catch (const std::bad_alloc&) { rc = DecoderStatus_OutOfMemory; } catch (const std::exception& e) { SetErrorMessage(errorInfo, e.what()); rc = DecoderStatus_DecodeError; } catch (...) { rc = DecoderStatus_DecodeError; }
+    return DecoderStatus_Ok;
+  });
   if (d_color || d_alpha) cudaDeviceSynchronize();   // the split kernel ran on the default stream; the copies above were synchronous
   DevicePut(d_color, bytes_c, pool_c); DevicePut(d_alpha, bytes_a, pool_a);
   return rc;
@@ -175,21 +186,21 @@ DecoderStatus JxlB200LoadImageLayers(const uint8_t* data, size_t dataSize, uint8
 // and tightly packed exactly as LoadImage would hand them to setLayerData.
 DecoderStatus JxlB200BandLayout(const uint8_t* data, size_t dataSize, int32_t* layout4, ErrorInfo* errorInfo) {
   if (!data || !layout4) return DecoderStatus_NullParameter;
-  ParsedInfo pi; std::string msg; Status st = DecodeBandLayout(data, dataSize, &pi, &msg);
-  if (st != Status::Ok) { SetErrorMessage(errorInfo, msg); return DecoderStatus(st); }
-  layout4[0] = int32_t(pi.width); layout4[1] = int32_t(pi.height); layout4[2] = int32_t(pi.group_dim); layout4[3] = int32_t(pi.num_group_rows); return DecoderStatus_Ok;
+  return Guard<Decoding>(errorInfo, [&] {
+    const ParsedInfo pi = DecodeBandLayout(data, dataSize);
+    layout4[0] = int32_t(pi.width); layout4[1] = int32_t(pi.height); layout4[2] = int32_t(pi.group_dim); layout4[3] = int32_t(pi.num_group_rows); return DecoderStatus_Ok;
+  });
 }
 DecoderStatus JxlB200DecodeBand(int32_t device, const uint8_t* data, size_t dataSize, uint32_t groupRowBegin, uint32_t groupRowEnd, uint8_t* out, size_t outBytes, int32_t bgra, int32_t* rows, ErrorInfo* errorInfo) {
   if (!data || !out) return DecoderStatus_NullParameter;
-  try {
+  return Guard<Decoding>(errorInfo, [&] {
     if (device >= 0 && cudaSetDevice(device) != cudaSuccess) { SetErrorMessage(errorInfo, "cudaSetDevice failed"); return DecoderStatus_InvalidParameter; }
     if (groupRowBegin >= groupRowEnd) { SetErrorMessage(errorInfo, "band decode: empty group-row range"); return DecoderStatus_InvalidParameter; }
-    DecodeRequest req; req.data = data; req.size = dataSize; req.bgra = bgra != 0; req.band_begin = groupRowBegin; req.band_end = groupRowEnd; DecodeResult res = DecodeOnGpu(req); g_last_times = res.times;
-    if (res.status != Status::Ok) { SetErrorMessage(errorInfo, res.message); return DecoderStatus(res.status); }
+    DecodeRequest req; req.data = data; req.size = dataSize; req.bgra = bgra != 0; req.band_begin = groupRowBegin; req.band_end = groupRowEnd; const DecodeResult res = WithTimes(DecodeOnGpu, req);
     if (outBytes < res.pixel_bytes) { SetErrorMessage(errorInfo, "band buffer too small"); return DecoderStatus_InvalidParameter; }
     memcpy(out, res.pixels, res.pixel_bytes); if (rows) *rows = int32_t(res.out_height);
-  } catch (const std::bad_alloc&) { return DecoderStatus_OutOfMemory; } catch (const std::exception& e) { SetErrorMessage(errorInfo, e.what()); return DecoderStatus_DecodeError; } catch (...) { return DecoderStatus_DecodeError; }
-  return DecoderStatus_Ok;
+    return DecoderStatus_Ok;
+  });
 }
 
 // One shard of a batch: images [begin, end) of the caller's arrays, decoded by the three-phase pipeline below on `nstreams` streams owned
@@ -250,7 +261,7 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     std::vector<cudaStream_t>& all_streams = ShardStreams(cur_dev, slot, nstreams + 1);
     cudaStream_t copy_stream = all_streams[0];
     std::vector<cudaStream_t> free_streams(all_streams.rbegin(), all_streams.rbegin() + nstreams);
-    struct InFlight { int idx; std::shared_ptr<DecodeJob> job; DecodeResult res; bool direct = false; };
+    struct InFlight { int idx; std::shared_ptr<DecodeJob> job; bool direct = false; };
     std::vector<size_t> in_off(size_t(count) + 1, 0); const uint8_t* host_in = nullptr;
     // Device-resident inputs: the headers are parsed on the host, so every file comes back once through one pinned buffer. The copies
     // are queued up front on their own stream, one event per file, and a file is only waited for when its turn to be parsed comes.
@@ -281,22 +292,27 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     std::deque<std::unique_ptr<Bundle>> q1, q2, q3; int next = 0, done = 0;
     const double t_start = now(); double ph_first[3] = {-1, -1, -1}, ph_last[3] = {0, 0, 0};   // trace: when the first / last bundle left phase 1, 2, 3
     auto stamp = [&](int ph) { const double t = now() - t_start; if (ph_first[ph] < 0) ph_first[ph] = t; ph_last[ph] = t; };
-    auto finish = [&](InFlight& f) {   // records the status of a finished or failed image
-      DecoderStatus st = DecoderStatus(f.res.status);
-      if (st == DecoderStatus_Ok) {
-        if (f.res.pixel_bytes > a.outputBytes[f.idx]) st = DecoderStatus_InvalidParameter;
-        else if (!f.direct) memcpy(a.outputs[f.idx], f.res.pixels, f.res.pixel_bytes);
-      }
-      record(f.idx, st, f.res.message);
-      if (trace) { const StageTimes& t = f.res.times; acc_t[0] += t.lf; acc_t[1] += t.ac; acc_t[2] += t.recon; acc_t[3] += t.filters + t.output; acc_t[4] += t.total; }
-      f.job.reset(); f.res.job.reset(); done++;
+    auto finish = [&](InFlight& f, const DecodeResult& res) {   // records a decoded image
+      DecoderStatus st = DecoderStatus_Ok;
+      if (res.pixel_bytes > a.outputBytes[f.idx]) st = DecoderStatus_InvalidParameter;
+      else if (!f.direct) memcpy(a.outputs[f.idx], res.pixels, res.pixel_bytes);
+      record(f.idx, st, std::string());
+      if (trace) { const StageTimes& t = res.times; acc_t[0] += t.lf; acc_t[1] += t.ac; acc_t[2] += t.recon; acc_t[3] += t.filters + t.output; acc_t[4] += t.total; }
+      f.job.reset(); done++;
+    };
+    // Runs one step of an image (enqueue, a later phase, finish). A failure is recorded for the image and drops it (false).
+    auto step = [&](InFlight& f, auto&& fn) {
+      ErrorInfo ei; ei.errorMessage[0] = 0;
+      const DecoderStatus st = Guard<Decoding>(&ei, [&] { fn(); return DecoderStatus_Ok; });
+      if (st != DecoderStatus_Ok) { record(f.idx, st, ei.errorMessage); f.job.reset(); done++; }
+      return st == DecoderStatus_Ok;
     };
     auto idle = [](const Bundle& b) { return cudaStreamQuery(b.stream) != cudaErrorNotReady; };
     auto jobs_of = [](Bundle& b) { std::vector<std::shared_ptr<DecodeJob>> v; for (auto& it : b.items) v.push_back(it->job); return v; };
     auto next_phase = [&](Bundle& b, int phase) {   // enqueue `phase` for every image of the bundle; images that fail are finished and dropped
       for (size_t k = 0; k < b.items.size();) {
         InFlight& f = *b.items[k];
-        if (DecodeEnqueuePhase(f.job, phase, &f.res)) k++; else { finish(f); b.items.erase(b.items.begin() + k); }
+        if (step(f, [&] { DecodeEnqueuePhase(f.job, phase); })) k++; else b.items.erase(b.items.begin() + k);
       }
       if (phase == 2) DecodeBundleLaunch(jobs_of(b), 2);
     };
@@ -305,7 +321,7 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
       for (size_t k = 0; k < std::min(kWindow, q3.size());) {
         if (!idle(*q3[k])) { k++; continue; }
         Bundle& b = *q3[k];
-        for (auto& f : b.items) { DecodeFinish(f->job, &f->res); finish(*f); }
+        for (auto& f : b.items) step(*f, [&] { finish(*f, DecodeFinish(f->job)); });
         free_streams.push_back(b.stream); q3.erase(q3.begin() + k); progressed = true; stamp(2);
       }
       for (size_t k = 0; k < std::min(kWindow, q2.size());) {
@@ -340,12 +356,13 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
           if (a.hostInputs) req.data = a.datas[i]; else { cudaEventSynchronize(in_ready[li]); req.data = host_in + in_off[li]; req.device_input = a.datas[i]; }
           if (!a.hostOutputs) { req.out_device = a.outputs[i]; f->direct = true; } else if (out_is_pinned[li]) { req.out_pinned = a.outputs[i]; f->direct = true; }
           if (reserve_sets == 0 && a.count >= 32) for (int spin = 0; spin < 40000 && !g_pools_warm[cur_dev & 63].load(); spin++) std::this_thread::sleep_for(std::chrono::microseconds(50));   // at most 2 s, first batch only
-          f->job = DecodeEnqueue(req, b->stream, &f->res, true, bundle_size > 1);
+          bool layered = false;
+          step(*f, [&] { try { f->job = DecodeEnqueue(req, b->stream, true, bundle_size > 1); } catch (const LayeredStill&) { layered = true; } });
           if (!reserved) { reserved = true; if (f->job) DecodeReservePools(f->job, reserve_sets); g_pools_warm[cur_dev & 63].store(1); }   // the first image tells the buffer sizes of the batch
-          if (!f->job && f->res.layered) {   // a layered still inside a batch: composited by the single-image path, on this shard's thread
-            DecodeRequest lr = req; lr.ac_lanes = 0; f->res = DecodeOnGpu(lr);
+          if (layered) {   // a layered still inside a batch: composited by the single-image path, on this shard's thread
+            DecodeRequest lr = req; lr.ac_lanes = 0; step(*f, [&] { finish(*f, DecodeOnGpu(lr)); });
           }
-          if (f->job) b->items.push_back(std::move(f)); else finish(*f);
+          if (f->job) b->items.push_back(std::move(f));
         }
         if (bundle_size > 1) DecodeBundleLaunch(jobs_of(*b), 1);
         t_enq += now() - t0;
@@ -356,7 +373,7 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     if (trace && acc_t[4] > 0) fprintf(stderr, "[jxlb200] shard %d GPU ms/image under load (JXLB200_TRACE=2 events): lf %.2f ac %.2f recon %.2f render %.2f total %.2f\n", slot, acc_t[0] / count, acc_t[1] / count, acc_t[2] / count, acc_t[3] / count, acc_t[4] / count);
     if (trace) fprintf(stderr, "[jxlb200] shard %d phase exits, ms after shard start (first .. last bundle): LF %.1f .. %.1f, AC %.1f .. %.1f, tiles %.1f .. %.1f\n", slot, ph_first[0], ph_last[0], ph_first[1], ph_last[1], ph_first[2], ph_last[2]);
     if (trace) fprintf(stderr, "[jxlb200] shard %d, %d images: host parse + LF phase %.2f ms (%.2f ms/image), polling + later phases + retire %.2f ms, idle (GPU-bound) %.2f ms\n", slot, count, t_enq, t_enq / std::max(count, 1), t_ret, t_idle);
-  } catch (const std::exception& e) {
+  } catch (const std::exception& e) {   // a failure of the shard itself (streams, input copies): every image not finished yet fails with it
     // Work may still be running on this shard's streams and writing into caller-owned buffers: wait for it before returning them.
     cudaDeviceSynchronize(); cudaGetLastError();
     const DecoderStatus st = dynamic_cast<const std::bad_alloc*>(&e) ? DecoderStatus_OutOfMemory : DecoderStatus_DecodeError;
@@ -381,9 +398,10 @@ static void ReleaseSlot(int slot) { std::lock_guard<std::mutex> lk(g_slot_mu); g
 JxlB200Batch* JxlB200DecodeBatchSubmit(int32_t device, int32_t count, const uint8_t* const* datas, const size_t* dataSizes, uint8_t* const* outputs, const size_t* outputBytes, int32_t bgra,
                                        int32_t hostInputs, int32_t hostOutputs, int32_t maxInFlight, ErrorInfo* errorInfo) {
   if (!datas || !dataSizes || !outputs || !outputBytes || count < 0) { SetErrorMessage(errorInfo, "null parameter"); return nullptr; }
-  try {
-    std::string why; if (!CudaAvailable(&why)) { SetErrorMessage(errorInfo, why); return nullptr; }
-    if (device >= 0 && cudaSetDevice(device) != cudaSuccess) { SetErrorMessage(errorInfo, "cudaSetDevice failed"); return nullptr; }
+  JxlB200Batch* raw = nullptr;
+  Guard<Decoding>(errorInfo, [&] {
+    std::string why; JXLG_CHECK(CudaAvailable(&why), why);
+    JXLG_CHECK(device < 0 || cudaSetDevice(device) == cudaSuccess, "cudaSetDevice failed");
     std::unique_ptr<JxlB200Batch> b(new JxlB200Batch);
     b->datas.assign(datas, datas + count); b->sizes.assign(dataSizes, dataSizes + count); b->outputs.assign(outputs, outputs + count); b->out_bytes.assign(outputBytes, outputBytes + count);
     b->statuses.assign(size_t(count), DecoderStatus_Ok);
@@ -400,17 +418,17 @@ JxlB200Batch* JxlB200DecodeBatchSubmit(int32_t device, int32_t count, const uint
     b->args = BatchArgs{device, count, b->datas.data(), b->sizes.data(), b->outputs.data(), b->out_bytes.data(), bgra, hostInputs, hostOutputs, b->statuses.data()};
     b->results.resize(size_t(shards));
     const size_t reserve_sets = size_t(std::min(count, nstreams * bundle_size)) - (count > 0 ? 1 : 0);
-    JxlB200Batch* raw = b.get();
+    JxlB200Batch* self = b.get();
     for (int k = 0; k < shards; k++) {
       const int i0 = int(int64_t(count) * k / shards), i1 = int(int64_t(count) * (k + 1) / shards), ns = nstreams * (k + 1) / shards - nstreams * k / shards;
       const int slot = AcquireSlot(); b->slots.push_back(slot);
-      b->threads.emplace_back([raw, k, slot, i0, i1, ns, batch_lanes, bundle_size, reserve_sets]() {
-        RunBatchShard(raw->args, slot, i0, i1, std::max(1, ns), batch_lanes, bundle_size, k == 0 ? reserve_sets : 0, &raw->results[size_t(k)]);
+      b->threads.emplace_back([self, k, slot, i0, i1, ns, batch_lanes, bundle_size, reserve_sets]() {
+        RunBatchShard(self->args, slot, i0, i1, std::max(1, ns), batch_lanes, bundle_size, k == 0 ? reserve_sets : 0, &self->results[size_t(k)]);
       });
     }
-    return b.release();
-  } catch (const std::exception& e) { SetErrorMessage(errorInfo, e.what()); } catch (...) {}
-  return nullptr;
+    raw = b.release(); return DecoderStatus_Ok;
+  });
+  return raw;
 }
 
 DecoderStatus JxlB200DecodeBatchWait(JxlB200Batch* batch, DecoderStatus* statuses, ErrorInfo* errorInfo) {
@@ -434,29 +452,29 @@ DecoderStatus JxlB200DecodeBatch(int32_t device, int32_t count, const uint8_t* c
 
 EncoderStatus JxlB200EncodeToMemory(const BitmapData* bitmap, const EncoderOptions* options, const EncoderImageMetadata* metadata, int32_t deviceInput, uint8_t** out, size_t* outSize, ErrorInfo* errorInfo) {
   if (!bitmap || !options || !out || !outSize) return EncoderStatus_NullParameter;
-  try {
+  return Guard<Encoding>(errorInfo, [&] {
     EncodeRequest req; req.bgra = bitmap->scan0; req.width = bitmap->width; req.height = bitmap->height; req.stride = bitmap->stride; req.distance = options->distance; req.effort = options->effort; req.lossless = options->lossless; req.device_input = deviceInput != 0;
     if (metadata) { req.exif = metadata->exif; req.exif_size = metadata->exifSize; req.icc = metadata->iccProfile; req.icc_size = metadata->iccProfileSize; req.xmp = metadata->xmp; req.xmp_size = metadata->xmpSize; }
-    EncodeResult res = EncodeOnGpu(req); g_last_times = res.times;
-    if (res.status != EncStatus::Ok) { SetErrorMessage(errorInfo, res.message); return EncoderStatus(res.status); }
-    *out = static_cast<uint8_t*>(malloc(res.file.size() ? res.file.size() : 1)); if (!*out) return EncoderStatus_OutOfMemory; memcpy(*out, res.file.data(), res.file.size()); *outSize = res.file.size();
-  } catch (const std::bad_alloc&) { return EncoderStatus_OutOfMemory; } catch (...) { return EncoderStatus_EncodeError; }
-  return EncoderStatus_Ok;
+    const EncodeResult res = WithTimes(EncodeOnGpu, req);
+    *out = static_cast<uint8_t*>(CopyOut(res.file.data(), res.file.size())); *outSize = res.file.size();
+    return EncoderStatus_Ok;
+  });
 }
 void JxlB200Free(void* p) { free(p); }
 // Host-only: what the encoder reads out of a matrix/TRC ICC profile (SaveImage with metadata->iccProfile, lossy): matrix9 = profile RGB
 // (linear) -> linear sRGB, lut768 = the three tone curves sampled at v/255. Returns 0 and a message when the profile cannot be used.
 int32_t JxlB200DebugParseIcc(const uint8_t* icc, size_t iccSize, float* matrix9, float* lut768, ErrorInfo* errorInfo) {
   if (!icc || !matrix9 || !lut768) return 0;
-  try { IccMatrixTrc m; std::string why; if (!ParseMatrixTrcIcc(icc, iccSize, &m, &why)) { SetErrorMessage(errorInfo, why); return 0; }
-    for (int i = 0; i < 9; i++) matrix9[i] = float(m.to_linear_srgb[i]); memcpy(lut768, m.lut, sizeof(m.lut)); return 1; }
-  catch (...) { return 0; }
+  return Guard<Encoding>(nullptr, [&] {
+    IccMatrixTrc m; std::string why; if (!ParseMatrixTrcIcc(icc, iccSize, &m, &why)) { SetErrorMessage(errorInfo, why); return EncoderStatus_EncodeError; }
+    for (int i = 0; i < 9; i++) matrix9[i] = float(m.to_linear_srgb[i]); memcpy(lut768, m.lut, sizeof(m.lut)); return EncoderStatus_Ok;
+  }) == EncoderStatus_Ok ? 1 : 0;
 }
 // Returns the cached device and page-locked buffers of the calling thread's current device to the driver (after a large batch the
 // pools hold one buffer set per image that was in flight).
 // ---- sharded encode (BASELINE config 5, SURVEY §8e "Encode sharding"): one band session per GPU, see encode_engine.cu
-struct JxlB200BandEncoder { BandSession* s = nullptr; int device = -1; };
-static void* CopyOut(const void* p, size_t n) { void* m = malloc(n ? n : 1); if (!m) throw std::bad_alloc(); if (n) memcpy(m, p, n); return m; }
+// The session holds the band encoder, its device and its own copy of the ICC profile (the caller's metadata need not outlive Create).
+struct JxlB200BandEncoder { std::unique_ptr<BandEncoder> enc; int device = -1; std::vector<uint8_t> icc; };
 static EncodeRequest BandRequest(const BitmapData* b, const EncoderOptions* o, const EncoderImageMetadata* md) {
   EncodeRequest req; req.bgra = b->scan0; req.width = b->width; req.height = b->height; req.stride = b->stride; req.distance = o->distance; req.effort = o->effort; req.lossless = o->lossless;
   if (md) { req.exif = md->exif; req.exif_size = md->exifSize; req.icc = md->iccProfile; req.icc_size = md->iccProfileSize; req.xmp = md->xmp; req.xmp_size = md->xmpSize; }
@@ -465,60 +483,69 @@ static EncodeRequest BandRequest(const BitmapData* b, const EncoderOptions* o, c
 JxlB200BandEncoder* JxlB200BandEncoderCreate(int32_t device, const BitmapData* band, uint32_t frameHeight, uint32_t firstRow, uint32_t haloTop, uint32_t haloBottom,
                                              const EncoderOptions* options, const EncoderImageMetadata* metadata, int32_t deviceInput, uint32_t* bandFlags, ErrorInfo* errorInfo) {
   if (!band || !band->scan0 || !options || !bandFlags) { SetErrorMessage(errorInfo, "null parameter"); return nullptr; }
-  try {
-    if (device >= 0 && cudaSetDevice(device) != cudaSuccess) { SetErrorMessage(errorInfo, "cudaSetDevice failed"); return nullptr; }
+  std::unique_ptr<JxlB200BandEncoder> h;
+  const EncoderStatus st = Guard<Encoding>(errorInfo, [&] {
+    JXLG_CHECK(device < 0 || cudaSetDevice(device) == cudaSuccess, "cudaSetDevice failed");
     EncodeRequest req = BandRequest(band, options, metadata); req.device_input = deviceInput != 0;
     req.frame_height = frameHeight; req.band_y0 = firstRow; req.halo_top = haloTop; req.halo_bottom = haloBottom;
-    EncStatus st = EncStatus::Ok; std::string msg; BandSession* s = BandEncoderCreate(req, bandFlags, &st, &msg);
-    if (!s) { SetErrorMessage(errorInfo, msg.empty() ? "band encoder: out of memory" : msg); return nullptr; }
-    JxlB200BandEncoder* h = new JxlB200BandEncoder; h->s = s; h->device = device; return h;
-  } catch (const std::exception& e) { SetErrorMessage(errorInfo, e.what()); } catch (...) {}
-  return nullptr;
+    h.reset(new JxlB200BandEncoder); h->device = device;
+    if (req.icc_size) { h->icc.assign(req.icc, req.icc + req.icc_size); req.icc = h->icc.data(); }
+    req.exif = nullptr; req.exif_size = 0; req.xmp = nullptr; req.xmp_size = 0;
+    h->enc.reset(new BandEncoder(req)); *bandFlags = h->enc->Begin();
+    return EncoderStatus_Ok;
+  });
+  if (st == EncoderStatus_OutOfMemory) SetErrorMessage(errorInfo, "band encoder: out of memory");
+  return st == EncoderStatus_Ok ? h.release() : nullptr;
 }
 EncoderStatus JxlB200BandEncoderTokenize(JxlB200BandEncoder* enc, uint32_t frameFlags, uint64_t** hist, size_t* histWords, ErrorInfo* errorInfo) {
   if (!enc || !hist || !histWords) return EncoderStatus_NullParameter;
-  try {
+  return Guard<Encoding>(errorInfo, [&] {
     if (enc->device >= 0) cudaSetDevice(enc->device);
-    std::vector<uint64_t> h; std::string msg; EncStatus st = BandEncoderTokenize(enc->s, frameFlags, &h, &msg);
-    if (st != EncStatus::Ok) { SetErrorMessage(errorInfo, msg); return EncoderStatus(st); }
+    const std::vector<uint64_t> h = enc->enc->Tokenize(frameFlags);
     *hist = static_cast<uint64_t*>(CopyOut(h.data(), h.size() * 8)); *histWords = h.size(); return EncoderStatus_Ok;
-  } catch (const std::bad_alloc&) { return EncoderStatus_OutOfMemory; } catch (...) { return EncoderStatus_EncodeError; }
+  });
 }
 EncoderStatus JxlB200BandEncoderFinish(JxlB200BandEncoder* enc, const uint64_t* frameHist, size_t histWords, uint8_t** sections, size_t* sectionBytes, float* deviceMs, ErrorInfo* errorInfo) {
   if (!enc || !frameHist || !sections || !sectionBytes) return EncoderStatus_NullParameter;
-  try {
+  return Guard<Encoding>(errorInfo, [&] {
     if (enc->device >= 0) cudaSetDevice(enc->device);
-    std::vector<uint8_t> blob; std::string msg; EncStatus st = BandEncoderFinish(enc->s, frameHist, histWords, &blob, deviceMs, &msg);
-    if (st != EncStatus::Ok) { SetErrorMessage(errorInfo, msg); return EncoderStatus(st); }
+    const std::vector<uint8_t> blob = enc->enc->FinishBlob(std::vector<uint64_t>(frameHist, frameHist + histWords)); if (deviceMs) *deviceMs = enc->enc->device_ms;
     *sections = static_cast<uint8_t*>(CopyOut(blob.data(), blob.size())); *sectionBytes = blob.size(); return EncoderStatus_Ok;
-  } catch (const std::bad_alloc&) { return EncoderStatus_OutOfMemory; } catch (...) { return EncoderStatus_EncodeError; }
+  });
 }
 int64_t JxlB200BandEncoderDebugStage(JxlB200BandEncoder* enc, int32_t which, void* out, int64_t capacityBytes, int64_t* dims4, ErrorInfo* errorInfo) {
   if (!enc) { SetErrorMessage(errorInfo, "null parameter"); return 0; }
-  try {
-    if (enc->device >= 0) cudaSetDevice(enc->device);
-    std::string msg; const int64_t n = BandEncoderDebugStage(enc->s, which, out, capacityBytes, dims4, &msg); if (!n) SetErrorMessage(errorInfo, msg); return n;
-  } catch (...) { SetErrorMessage(errorInfo, "stage dump failed"); return 0; }
+  int64_t n = 0;
+  Guard<Encoding>(errorInfo, [&] { if (enc->device >= 0) cudaSetDevice(enc->device); n = enc->enc->DebugStage(which, out, capacityBytes, dims4); return EncoderStatus_Ok; });
+  return n;
 }
-void JxlB200BandEncoderDestroy(JxlB200BandEncoder* enc) { if (!enc) return; try { if (enc->device >= 0) cudaSetDevice(enc->device); BandEncoderDestroy(enc->s); } catch (...) {} delete enc; }
+void JxlB200BandEncoderDestroy(JxlB200BandEncoder* enc) {
+  if (!enc) return;
+  Guard<Encoding>(nullptr, [&] { if (enc->device >= 0) cudaSetDevice(enc->device); enc->enc.reset(); return EncoderStatus_Ok; });   // the encoder waits for its stream
+  delete enc;
+}
 EncoderStatus JxlB200AssembleBands(uint32_t width, uint32_t height, const EncoderOptions* options, const EncoderImageMetadata* metadata, uint32_t frameFlags, const uint64_t* frameHist, size_t histWords,
                                    const uint8_t* const* bandSections, const size_t* bandSectionBytes, int32_t bandCount, uint8_t** out, size_t* outSize, ErrorInfo* errorInfo) {
   if (!options || !frameHist || !bandSections || !bandSectionBytes || !out || !outSize || bandCount <= 0) return EncoderStatus_NullParameter;
-  try {
+  return Guard<Encoding>(errorInfo, [&] {
     BitmapData whole{nullptr, width, height, width * 4}; EncodeRequest req = BandRequest(&whole, options, metadata);
-    std::vector<uint8_t> file; std::string msg; EncStatus st = AssembleBands(req, frameFlags, frameHist, histWords, bandSections, bandSectionBytes, size_t(bandCount), &file, &msg);
-    if (st != EncStatus::Ok) { SetErrorMessage(errorInfo, msg); return EncoderStatus(st); }
+    const std::vector<uint8_t> file = AssembleBands(req, frameFlags, frameHist, histWords, bandSections, bandSectionBytes, size_t(bandCount));
     *out = static_cast<uint8_t*>(CopyOut(file.data(), file.size())); *outSize = file.size(); return EncoderStatus_Ok;
-  } catch (const std::bad_alloc&) { return EncoderStatus_OutOfMemory; } catch (...) { return EncoderStatus_EncodeError; }
+  });
 }
 
 int64_t JxlB200DebugSectionSizes(const uint8_t* data, size_t dataSize, uint64_t* sizes, int64_t capacity, int32_t* counts2, ErrorInfo* errorInfo) {
   if (!data || !sizes) return 0;
-  std::vector<uint64_t> v; uint32_t nlf = 0, ng = 0; std::string msg; Status st = DecodeSectionSizes(data, dataSize, &v, &nlf, &ng, &msg);
-  if (st != Status::Ok) { SetErrorMessage(errorInfo, msg); return 0; }
-  if (int64_t(v.size()) > capacity) return 0; for (size_t i = 0; i < v.size(); i++) sizes[i] = v[i]; if (counts2) { counts2[0] = int32_t(nlf); counts2[1] = int32_t(ng); } return int64_t(v.size());
+  int64_t n = 0;
+  Guard<Decoding>(errorInfo, [&] {
+    const SectionSizes s = DecodeSectionSizes(data, dataSize);
+    if (int64_t(s.sizes.size()) > capacity) return DecoderStatus_Ok;
+    for (size_t i = 0; i < s.sizes.size(); i++) sizes[i] = s.sizes[i]; if (counts2) { counts2[0] = int32_t(s.num_lf_groups); counts2[1] = int32_t(s.num_groups); } n = int64_t(s.sizes.size());
+    return DecoderStatus_Ok;
+  });
+  return n;
 }
-void JxlB200ReleaseMemory(void) { try { cudaDeviceSynchronize(); TrimPools(); for (auto& w : g_pools_warm) w.store(0); } catch (...) {} }
+void JxlB200ReleaseMemory(void) { Guard<Decoding>(nullptr, [] { cudaDeviceSynchronize(); TrimPools(); for (auto& w : g_pools_warm) w.store(0); return DecoderStatus_Ok; }); }
 
 void JxlB200LastStageTimes(float* ms8) { if (!ms8) return; const StageTimes& t = g_last_times; ms8[0] = t.h2d; ms8[1] = t.lf; ms8[2] = t.ac; ms8[3] = t.recon; ms8[4] = t.filters; ms8[5] = t.output; ms8[6] = t.d2h; ms8[7] = t.total; }
 int64_t JxlB200KernelLaunchCount(void) { return LaunchCount(); }
@@ -526,13 +553,15 @@ int32_t JxlB200CudaAvailable(ErrorInfo* errorInfo) { std::string why; bool ok = 
 
 int64_t JxlB200DebugDecodeStage(const uint8_t* data, size_t dataSize, int32_t which, float* out, int64_t capacity, int32_t* dims2, ErrorInfo* errorInfo) {
   if (!data || !out) return 0;
-  try {
-    DecodeRequest req; req.data = data; req.size = dataSize; DecodeResult res = DecodeOnGpu(req);
-    if (res.status != Status::Ok) { SetErrorMessage(errorInfo, res.message); return 0; }
-    if (which == 4) { std::vector<int16_t> c; if (!DecodeDebugCoeffs(res.job, &c) || int64_t(c.size()) > capacity) return 0; for (size_t i = 0; i < c.size(); i++) out[i] = float(c[i]); return int64_t(c.size()); }
-    std::vector<float> v; int xp = 0, yp = 0; if (!DecodeDebugPlanes(res.job, which, &v, &xp, &yp) || int64_t(v.size()) > capacity) return 0;
-    memcpy(out, v.data(), v.size() * 4); if (dims2) { dims2[0] = xp; dims2[1] = yp; } return int64_t(v.size());
-  } catch (...) { return 0; }
+  int64_t n = 0;
+  Guard<Decoding>(errorInfo, [&] {
+    DecodeRequest req; req.data = data; req.size = dataSize; const DecodeResult res = DecodeOnGpu(req);
+    if (which == 4) { std::vector<int16_t> c; if (DecodeDebugCoeffs(res.job, &c) && int64_t(c.size()) <= capacity) { for (size_t i = 0; i < c.size(); i++) out[i] = float(c[i]); n = int64_t(c.size()); } return DecoderStatus_Ok; }
+    std::vector<float> v; int xp = 0, yp = 0; if (!DecodeDebugPlanes(res.job, which, &v, &xp, &yp) || int64_t(v.size()) > capacity) return DecoderStatus_Ok;
+    memcpy(out, v.data(), v.size() * 4); if (dims2) { dims2[0] = xp; dims2[1] = yp; } n = int64_t(v.size());
+    return DecoderStatus_Ok;
+  });
+  return n;
 }
 
 }  // extern "C"

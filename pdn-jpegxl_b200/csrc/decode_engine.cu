@@ -136,25 +136,25 @@ static ColorEncoding OutputEncoding(const ImageMetadata& m) {
   if (ok) return m.ce; t.color_space = m.ce.color_space == kCsGray ? kCsGray : kCsRGB; t.intent = 0; return t;
 }
 
-static Status ParseHeadersInto(const uint8_t* data, size_t size, Headers* h, ParsedInfo* info, std::string* msg) {
-  int sig = SignatureCheck(data, size); if (sig == 0) return Status::InvalidFileSignature;
+static void ParseHeadersInto(const uint8_t* data, size_t size, Headers* h, ParsedInfo* info) {
+  int sig = SignatureCheck(data, size); if (sig == 0) throw StatusError(DecoderStatus_InvalidFileSignature);
   h->ci = ParseContainer(data, size); info->is_container = h->ci.is_container; const ByteSpan& cs = h->ci.codestream;
   JXLG_CHECK(cs.size() >= 2 && cs[0] == 0xFF && cs[1] == 0x0A, "codestream signature");
   BitReader br(cs.data() + 2, cs.size() - 2); h->meta = ReadImageHeaders(br); const ImageMetadata& m = h->meta; h->frame_pos = 2 + br.pos / 8;
   // BASIC_INFO decisions, N/Decoder/JxlDecoder.cpp:461-561
-  if (m.xsize > 0x7fffffffu || m.ysize > 0x7fffffffu) return Status::ImageDimensionExceedsInt32;
+  if (m.xsize > 0x7fffffffu || m.ysize > 0x7fffffffu) throw StatusError(DecoderStatus_ImageDimensionExceedsInt32);
   int alpha = m.alpha_index(); uint32_t alpha_bits = alpha >= 0 ? m.ec[alpha].bd.bits : 0; info->has_alpha = alpha_bits != 0; int black = -1; bool first_alpha = false;
   for (size_t i = 0; i < m.ec.size(); i++) {
-    if (m.ec[i].type == kEcBlack) { if (black < 0) black = int(i); else return Status::UnsupportedChannelFormat; }
-    else if (m.ec[i].type == kEcAlpha) { if (info->has_alpha && !first_alpha) first_alpha = true; else return Status::UnsupportedChannelFormat; }
+    if (m.ec[i].type == kEcBlack) { if (black < 0) black = int(i); else throw StatusError(DecoderStatus_UnsupportedChannelFormat); }
+    else if (m.ec[i].type == kEcAlpha) { if (info->has_alpha && !first_alpha) first_alpha = true; else throw StatusError(DecoderStatus_UnsupportedChannelFormat); }
   }
   int cc = m.num_color_channels(); info->num_channels = cc + (info->has_alpha ? 1 : 0); info->format = cc == 1 ? 0 : (black >= 0 ? 2 : 1); info->sample_type = 0; info->width = m.xsize; info->height = m.ysize;
   if (m.bd.exp_bits > 0) {
-    if (info->format == 2) { *msg = "Floating point CMYK images are not supported."; return Status::DecodeError; }
-    if (m.bd.bits <= 16) info->sample_type = 2; else if (m.bd.bits <= 32) info->sample_type = 3; else { *msg = "Unsupported floating point bit depth: " + std::to_string(m.bd.bits) + "."; return Status::DecodeError; }
+    JXLG_CHECK(info->format != 2, "Floating point CMYK images are not supported.");
+    if (m.bd.bits <= 16) info->sample_type = 2; else if (m.bd.bits <= 32) info->sample_type = 3; else throw Error("Unsupported floating point bit depth: " + std::to_string(m.bd.bits) + ".");
   } else if (m.bd.bits > 8) {
-    if (m.bd.bits <= 16) { if (info->format == 2) { *msg = "CMYK64 images are not supported."; return Status::DecodeError; } info->sample_type = 1; }
-    else { *msg = "Unsupported integer bit depth: " + std::to_string(m.bd.bits) + "."; return Status::DecodeError; }
+    if (m.bd.bits <= 16) { JXLG_CHECK(info->format != 2, "CMYK64 images are not supported."); info->sample_type = 1; }
+    else throw Error("Unsupported integer bit depth: " + std::to_string(m.bd.bits) + ".");
   }
   if (m.orientation >= 5) std::swap(info->width, info->height);
   // COLOR_ENCODING, :562-686 — the profile reported is the one describing the delivered samples
@@ -167,15 +167,9 @@ static Status ParseHeadersInto(const uint8_t* data, size_t size, Headers* h, Par
     if (!strcmp(type, "brob") && n >= 4) { memcpy(type, p, 4); type[4] = 0; if (!strcmp(type, "Exif") || !strcmp(type, "xml ")) { tmp = BrotliDecompress(p + 4, n - 4); p = tmp.data(); n = tmp.size(); } }
     if (!strcmp(type, "Exif")) { if (!info->has_exif) { info->has_exif = true; info->exif.assign(p, p + n); } } else if (!strcmp(type, "xml ")) info->xmp.emplace_back(p, p + n);
   }
-  return Status::Ok;
 }
 
-DecodeResult ParseInfo(const uint8_t* data, size_t size) {
-  DecodeResult r; if (!data) { r.status = Status::NullParameter; return r; }
-  try { Headers h; r.status = ParseHeadersInto(data, size, &h, &r.info, &r.message); }
-  catch (const std::bad_alloc&) { r.status = Status::OutOfMemory; } catch (const std::exception& e) { r.status = Status::DecodeError; r.message = e.what(); }
-  return r;
-}
+ParsedInfo ParseInfo(const uint8_t* data, size_t size) { Headers h; ParsedInfo info; ParseHeadersInto(data, size, &h, &info); return info; }
 
 // ---------------------------------------------------------------- blob builder
 struct Blob {
@@ -224,6 +218,8 @@ static QuantEncoding ReadQuantEncodingHost(BitReader& br, int t) {
   }
   return e;
 }
+
+LayeredStill::LayeredStill() : Error("layered (multi-frame) files are decoded by LoadImage / JxlB200LoadImageBgra only, not by the batch and band calls") {}
 
 // ---------------------------------------------------------------- the job
 class DecodeJob {
@@ -421,7 +417,7 @@ void DecodeJob::Setup(const DecodeRequest& req) {
   JXLG_CHECK(fh.upsampling == 1, "upsampling is not supported"); JXLG_CHECK(!fh.do_ycbcr, "YCbCr (JPEG-recompressed) frames are not supported");
   if (!req.layer) {   // the plain single-frame file; layered files go through DecodeOnGpu's compositing loop, which sets req.layer for every frame
     const bool full = !fh.have_crop || (fh.x0 == 0 && fh.y0 == 0 && fh.width == m.xsize && fh.height == m.ysize);
-    JXLG_CHECK(FrameIsPlain(fh, m) && full, "layered (multi-frame) files are decoded by LoadImage / JxlB200LoadImageBgra only, not by the batch and band calls");
+    if (!FrameIsPlain(fh, m) || !full) throw LayeredStill();
   }
   JXLG_CHECK(fh.passes.num_passes <= uint32_t(kMaxPasses), "too many passes");
   JXLG_CHECK(fh.encoding != 0 || m.xyb_encoded, "VarDCT frames that are not XYB-encoded are not supported");
@@ -631,28 +627,42 @@ void DecodeJob::RunRender() {
   g_trace.t[6] += NowMs() - tt; g_trace.n++;
 }
 
-std::shared_ptr<DecodeJob> DecodeEnqueue(const DecodeRequest& req, cudaStream_t stream, DecodeResult* res, bool lf_phase_only, bool defer_entropy) {
-  std::shared_ptr<DecodeJob> job;
-  if (!req.data) { res->status = Status::NullParameter; return job; }
-  try {
-    std::string why; if (!CudaAvailable(&why)) { res->status = Status::DecodeError; res->message = why; return job; }
-    job = std::make_shared<DecodeJob>(); job->stream = stream; double t0 = NowMs();
-    { static const bool batch_times = getenv("JXLB200_TRACE") != nullptr && atoi(getenv("JXLB200_TRACE")) >= 2; if (batch_times) { job->timed = true; for (int i = 0; i < 7; i++) cudaEventCreate(&job->ev[i]); } }
-    res->status = ParseHeadersInto(req.data, req.size, &job->hd, &job->info, &res->message); if (res->status != Status::Ok) { job.reset(); return job; }
-    g_trace.t[0] += NowMs() - t0; t0 = NowMs(); job->phased = lf_phase_only; job->defer_entropy = defer_entropy && lf_phase_only; job->Setup(req); g_trace.t[1] += NowMs() - t0; if (lf_phase_only) job->RunLf(req); else job->Run(req); res->info = job->info;
-  } catch (const std::bad_alloc&) { res->status = Status::OutOfMemory; job.reset(); }
-  catch (const std::exception& e) { res->status = Status::DecodeError; res->message = e.what(); res->layered = res->message.rfind("layered (multi-frame)", 0) == 0; if (job) res->info = job->info; job.reset(); }
+// Position of the first frame after an optional preview frame, and whether that frame is a plain single-frame image.
+static bool FirstFrameIsPlain(const Headers& hd, size_t* first_pos) {
+  const ImageMetadata& m = hd.meta; const ByteSpan& cs = hd.ci.codestream; size_t pos = hd.frame_pos;
+  if (m.have_preview) { ImageMetadata pm = m; pm.xsize = m.preview_x; pm.ysize = m.preview_y; BitReader br(cs.data() + pos, cs.size() - pos); FrameHeader pf = ReadFrameHeader(br, pm); Toc t = ReadToc(br, pf); pos += br.pos / 8 + t.total; JXLG_CHECK(pos <= cs.size(), "preview frame truncated"); }
+  *first_pos = pos; BitReader br(cs.data() + pos, cs.size() - pos); FrameHeader fh = ReadFrameHeader(br, m);
+  const bool exact = !fh.have_crop || (fh.x0 == 0 && fh.y0 == 0 && fh.width == m.xsize && fh.height == m.ysize);
+  return FrameIsPlain(fh, m) && exact;
+}
+
+// The start of every decode: a job on `stream` (stage events when `timed`) with the headers parsed and the frame set up. With `layered_pos`,
+// a file whose first frame is not plain is left for compositing: the job holds only its headers, and *layered_pos receives that frame's position.
+static std::shared_ptr<DecodeJob> StartJob(const DecodeRequest& req, cudaStream_t stream, bool timed, size_t* layered_pos = nullptr) {
+  std::shared_ptr<DecodeJob> job = std::make_shared<DecodeJob>(); job->stream = stream;
+  if (timed) { job->timed = true; for (int i = 0; i < 7; i++) cudaEventCreate(&job->ev[i]); }
+  double t0 = NowMs(); ParseHeadersInto(req.data, req.size, &job->hd, &job->info); g_trace.t[0] += NowMs() - t0;
+  if (layered_pos && !FirstFrameIsPlain(job->hd, layered_pos)) return job;
+  if (layered_pos) *layered_pos = 0;
+  t0 = NowMs(); job->Setup(req); g_trace.t[1] += NowMs() - t0;
+  return job;
+}
+
+std::shared_ptr<DecodeJob> DecodeEnqueue(const DecodeRequest& req, cudaStream_t stream, bool lf_phase_only, bool defer_entropy) {
+  if (!req.data) throw StatusError(DecoderStatus_NullParameter);
+  std::string why; JXLG_CHECK(CudaAvailable(&why), why);
+  static const bool batch_times = getenv("JXLB200_TRACE") != nullptr && atoi(getenv("JXLB200_TRACE")) >= 2;
+  std::shared_ptr<DecodeJob> job = StartJob(req, stream, batch_times);
+  job->phased = lf_phase_only; job->defer_entropy = defer_entropy && lf_phase_only;
+  if (lf_phase_only) job->RunLf(req); else job->Run(req);
   return job;
 }
 
 // Phased enqueue (batches): phase 1 = DecodeEnqueue(..., lf_phase_only), then DecodeEnqueuePhase(job, 2) and (job, 3), each once
-// the stream has drained (DecodeStreamIdle), so that a queued dependent kernel never blocks a hardware queue shared with other streams.
-bool DecodeEnqueuePhase(std::shared_ptr<DecodeJob>& job, int phase, DecodeResult* res) {
-  if (!job) return false;
-  try { if (phase == 2) job->RunAc(); else job->RunRender(); return true; }
-  catch (const std::bad_alloc&) { res->status = Status::OutOfMemory; }
-  catch (const std::exception& e) { res->status = Status::DecodeError; res->message = e.what(); res->info = job->info; }
-  cudaStreamSynchronize(job->stream); job.reset(); return false;
+// the stream has drained, so that a queued dependent kernel never blocks a hardware queue shared with other streams.
+void DecodeEnqueuePhase(const std::shared_ptr<DecodeJob>& job, int phase) {
+  try { if (phase == 2) job->RunAc(); else job->RunRender(); }
+  catch (...) { cudaStreamSynchronize(job->stream); throw; }   // the caller drops the failed job: its buffers may go back to the pools only once its work has drained
 }
 // Bundle mode: the jobs share one stream and were enqueued with defer_entropy; their pending LF (phase 1) or AC (phase 2) entropy kernels
 // go out as multi-image launches of up to kMaxBundle frames each.
@@ -673,43 +683,25 @@ void DecodeBundleLaunch(const std::vector<std::shared_ptr<DecodeJob>>& jobs, int
   }
 }
 // Band layout of the first frame (host-only parse): group size in pixels and the number of group rows a caller can shard over.
-Status DecodeBandLayout(const uint8_t* data, size_t size, ParsedInfo* info, std::string* message) {
-  if (!data) return Status::NullParameter;
-  try { DecodeJob job; Status st = ParseHeadersInto(data, size, &job.hd, &job.info, message); if (st != Status::Ok) return st; DecodeRequest req; req.data = data; req.size = size; job.Setup(req); *info = job.info; return Status::Ok; }
-  catch (const std::bad_alloc&) { return Status::OutOfMemory; }
-  catch (const std::exception& e) { if (message) *message = e.what(); return Status::DecodeError; }
-}
+ParsedInfo DecodeBandLayout(const uint8_t* data, size_t size) { DecodeRequest req; req.data = data; req.size = size; return StartJob(req, nullptr, false)->info; }
 // Host-only: byte sizes of the first frame's TOC entries (sections in logical order). Instrumentation for the load-balance analysis of the AC kernel.
-Status DecodeSectionSizes(const uint8_t* data, size_t size, std::vector<uint64_t>* sizes, uint32_t* num_lf_groups, uint32_t* num_groups, std::string* message) {
-  if (!data) return Status::NullParameter;
-  try { DecodeJob job; Status st = ParseHeadersInto(data, size, &job.hd, &job.info, message); if (st != Status::Ok) return st; DecodeRequest req; req.data = data; req.size = size; job.Setup(req);
-    sizes->assign(job.toc.size.begin(), job.toc.size.end()); *num_lf_groups = job.fh.num_lf_groups; *num_groups = job.fh.num_groups; return Status::Ok; }
-  catch (const std::bad_alloc&) { return Status::OutOfMemory; }
-  catch (const std::exception& e) { if (message) *message = e.what(); return Status::DecodeError; }
+SectionSizes DecodeSectionSizes(const uint8_t* data, size_t size) {
+  DecodeRequest req; req.data = data; req.size = size; std::shared_ptr<DecodeJob> job = StartJob(req, nullptr, false);
+  SectionSizes r; r.sizes.assign(job->toc.size.begin(), job->toc.size.end()); r.num_lf_groups = job->fh.num_lf_groups; r.num_groups = job->fh.num_groups; return r;
 }
 void DecodeReservePools(const std::shared_ptr<DecodeJob>& job, size_t count) { if (job) job->ReservePools(count); }
-void DecodeStreamSync(const std::shared_ptr<DecodeJob>& job) { if (job) cudaStreamSynchronize(job->stream); }
-bool DecodeStreamIdle(const std::shared_ptr<DecodeJob>& job) { return !job || cudaStreamQuery(job->stream) != cudaErrorNotReady; }
 
-void DecodeFinish(const std::shared_ptr<DecodeJob>& job, DecodeResult* res) {
-  if (!job) return;
+DecodeResult DecodeFinish(const std::shared_ptr<DecodeJob>& job) {
   cudaError_t e = cudaStreamSynchronize(job->stream);
-  if (e != cudaSuccess) { res->status = Status::DecodeError; res->message = std::string("CUDA: ") + cudaGetErrorString(e); return; }
+  if (e != cudaSuccess) throw Error(std::string("CUDA: ") + cudaGetErrorString(e));
   uint32_t de = *job->h_err.as<uint32_t>();
   { static const bool dbg = getenv("JXLB200_TRACE") != nullptr; if (dbg && job->timed) fprintf(stderr, "[jxlb200] LF group 0: LF coefficients %u kcycles, HF metadata %u kcycles\n", job->h_err.as<uint32_t>()[13], job->h_err.as<uint32_t>()[14]); }
-  if (de) { res->status = Status::DecodeError; res->message = DevErrorText(de); return; }
-  res->info = job->info; res->pixels = job->device_output ? job->h.out_px : (job->ext_out_pinned ? job->ext_out_pinned : job->h_out.as<uint8_t>()); res->pixel_bytes = job->out_bytes; res->out_width = job->h.out.out_w; res->out_height = job->h.band_on ? job->h.out_y1 - job->h.out_y0 : job->h.out.out_h; res->job = job;
+  JXLG_CHECK(de == 0, DevErrorText(de));
+  DecodeResult r;
+  r.info = job->info; r.pixels = job->device_output ? job->h.out_px : (job->ext_out_pinned ? job->ext_out_pinned : job->h_out.as<uint8_t>()); r.pixel_bytes = job->out_bytes; r.out_width = job->h.out.out_w; r.out_height = job->h.band_on ? job->h.out_y1 - job->h.out_y0 : job->h.out.out_h; r.job = job;
   if (job->timed) { auto ms = [&](int a, int b) { float t = 0; cudaEventElapsedTime(&t, job->ev[a], job->ev[b]); return t; };
-    res->times.lf = ms(0, 1); res->times.ac = ms(1, 2); res->times.recon = ms(2, 3); res->times.filters = ms(3, 4); res->times.output = ms(4, 5); res->times.d2h = ms(5, 6); res->times.total = ms(0, 6); }
-}
-
-// Position of the first frame after an optional preview frame, and whether that frame is a plain single-frame image.
-static bool FirstFrameIsPlain(const Headers& hd, size_t* first_pos) {
-  const ImageMetadata& m = hd.meta; const ByteSpan& cs = hd.ci.codestream; size_t pos = hd.frame_pos;
-  if (m.have_preview) { ImageMetadata pm = m; pm.xsize = m.preview_x; pm.ysize = m.preview_y; BitReader br(cs.data() + pos, cs.size() - pos); FrameHeader pf = ReadFrameHeader(br, pm); Toc t = ReadToc(br, pf); pos += br.pos / 8 + t.total; JXLG_CHECK(pos <= cs.size(), "preview frame truncated"); }
-  *first_pos = pos; BitReader br(cs.data() + pos, cs.size() - pos); FrameHeader fh = ReadFrameHeader(br, m);
-  const bool exact = !fh.have_crop || (fh.x0 == 0 && fh.y0 == 0 && fh.width == m.xsize && fh.height == m.ysize);
-  return FrameIsPlain(fh, m) && exact;
+    r.times.lf = ms(0, 1); r.times.ac = ms(1, 2); r.times.recon = ms(2, 3); r.times.filters = ms(3, 4); r.times.output = ms(4, 5); r.times.d2h = ms(5, 6); r.times.total = ms(0, 6); }
+  return r;
 }
 
 // Layered stills (N/Decoder/JxlDecoder.cpp:252-400: the reference takes the first full image of a coalescing decoder). Every frame up to the
@@ -717,12 +709,11 @@ static bool FirstFrameIsPlain(const Headers& hd, size_t* first_pos) {
 // copy of the frame's source slot (dev/composite_kernels.cu); frames that may be referenced leave their result in a slot. The canvas that is
 // shown becomes the output: unpremultiply, sample type, orientation. Reference-only frames saved before the colour transform can only feed
 // patches (rejected) and are skipped.
-static void DecodeLayered(const DecodeRequest& req, size_t pos, cudaStream_t st, DecodeResult* res) {
-  struct SlotBuf { DevBuf buf; bool valid = false; }; SlotBuf slots[4]; ParsedInfo info;
+// `head` holds the file's headers.
+static DecodeResult DecodeLayered(const DecodeRequest& req, const DecodeJob& head, size_t pos, cudaStream_t st) {
+  struct SlotBuf { DevBuf buf; bool valid = false; }; SlotBuf slots[4]; ParsedInfo info = head.info;
+  const ImageMetadata& m = head.hd.meta; const ByteSpan& cs = head.hd.ci.codestream;
   for (int guard = 0; guard < 4096; guard++) {
-    std::shared_ptr<DecodeJob> job = std::make_shared<DecodeJob>(); job->stream = st;
-    Status hs = ParseHeadersInto(req.data, req.size, &job->hd, &job->info, &res->message); if (hs != Status::Ok) { res->status = hs; return; }
-    const ImageMetadata& m = job->hd.meta; const ByteSpan& cs = job->hd.ci.codestream; info = job->info;
     JXLG_CHECK(pos < cs.size(), "JxlDecoderProcessInput needs more input, but it already received the entire image.");
     BitReader br(cs.data() + pos, cs.size() - pos); const FrameHeader fh = ReadFrameHeader(br, m); const Toc toc = ReadToc(br, fh); const size_t next = pos + br.pos / 8 + toc.total;
     JXLG_CHECK(next <= cs.size(), "JxlDecoderProcessInput needs more input, but it already received the entire image.");
@@ -734,8 +725,7 @@ static void DecodeLayered(const DecodeRequest& req, size_t pos, cudaStream_t st,
     JXLG_CHECK(!(cb.mode == 2 || cb.mode == 3) || (alpha >= 0 && int(cb.alpha_channel) == alpha), "blending needs the image's alpha channel");
     JXLG_CHECK(alpha < 0 || ref_only || ab.source == cb.source, "colour and alpha blended from different reference slots are not supported");
     DecodeRequest r = req; r.layer = true; r.layer_pos = pos; r.device_output = true; r.out_device = nullptr; r.out_pinned = nullptr; r.bgra = false; r.band_begin = r.band_end = 0; r.device_input = nullptr;
-    job->Setup(r); job->Run(r); DecodeResult fr; DecodeFinish(job, &fr);
-    if (fr.status != Status::Ok) { res->status = fr.status; res->message = fr.message; res->info = info; return; }
+    std::shared_ptr<DecodeJob> job = StartJob(r, st, false); job->Run(r); const DecodeResult fr = DecodeFinish(job);
     const int W = int(m.xsize), H = int(m.ysize), C = info.num_channels, cc = int(m.num_color_channels()); const size_t canvas_bytes = size_t(W) * H * C * sizeof(float);
     DevBuf canvas; canvas.Alloc(canvas_bytes);
     if (!ref_only && slots[cb.source].valid) CUDA_OK(cudaMemcpyAsync(canvas.p, slots[cb.source].buf.p, canvas_bytes, cudaMemcpyDeviceToDevice, st)); else CUDA_OK(cudaMemsetAsync(canvas.p, 0, canvas_bytes, st));
@@ -751,8 +741,8 @@ static void DecodeLayered(const DecodeRequest& req, size_t pos, cudaStream_t st,
       uint8_t* host = nullptr;
       if (!req.device_output) { host = req.out_pinned; if (!host) { job->h_layer_out.Alloc(out_bytes, true); host = job->h_layer_out.as<uint8_t>(); } CUDA_OK(cudaMemcpyAsync(host, d_final, out_bytes, cudaMemcpyDeviceToHost, st)); }
       CUDA_OK(cudaStreamSynchronize(st));
-      info.frame_name = fh.name; res->status = Status::Ok; res->info = info; res->pixels = req.device_output ? d_final : host; res->pixel_bytes = out_bytes;
-      res->out_width = ori >= 5 ? uint32_t(H) : uint32_t(W); res->out_height = ori >= 5 ? uint32_t(W) : uint32_t(H); res->job = job; return;
+      DecodeResult res; info.frame_name = fh.name; res.info = info; res.pixels = req.device_output ? d_final : host; res.pixel_bytes = out_bytes;
+      res.out_width = ori >= 5 ? uint32_t(H) : uint32_t(W); res.out_height = ori >= 5 ? uint32_t(W) : uint32_t(H); res.job = job; return res;
     }
     CUDA_OK(cudaStreamSynchronize(st));   // the frame's buffers go back to the pools with the job
     const bool can_ref = ref_only || (!fh.is_last && (fh.duration == 0 || fh.save_as_reference != 0));
@@ -763,33 +753,18 @@ static void DecodeLayered(const DecodeRequest& req, size_t pos, cudaStream_t st,
 }
 
 DecodeResult DecodeOnGpu(const DecodeRequest& req) {
-  DecodeResult res; cudaStream_t st = nullptr;
-  std::string why; if (!req.data) { res.status = Status::NullParameter; return res; }
-  if (SignatureCheck(req.data, req.size) == 0) { res.status = Status::InvalidFileSignature; return res; }
-  if (!CudaAvailable(&why)) { res.status = Status::DecodeError; res.message = why; return res; }
-  if (cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) != cudaSuccess) { res.status = Status::DecodeError; res.message = "cudaStreamCreate failed"; return res; }
-  {
-    std::shared_ptr<DecodeJob> job;
-    // timing events are cheap; always record so callers can read stage times
-    DecodeRequest r2 = req; (void)r2;
-    job = std::shared_ptr<DecodeJob>(); DecodeResult tmp;
-    // enqueue with stage timing enabled
-    struct Timed { static void Enable(DecodeJob* j) { j->timed = true; for (int i = 0; i < 7; i++) cudaEventCreate(&j->ev[i]); } };
-    try {
-      job = std::make_shared<DecodeJob>(); job->stream = st; Timed::Enable(job.get());
-      res.status = ParseHeadersInto(req.data, req.size, &job->hd, &job->info, &res.message);
-      if (res.status == Status::Ok) {
-        size_t first_pos = 0; const bool plain = FirstFrameIsPlain(job->hd, &first_pos);
-        if (plain || req.band_begin || req.band_end) { job->Setup(req); job->Run(req); DecodeFinish(job, &res); }
-        else { job.reset(); DecodeLayered(req, first_pos, st, &res); }
-      }
-    } catch (const std::bad_alloc&) { res.status = Status::OutOfMemory; }
-    catch (const std::exception& e) { res.status = Status::DecodeError; res.message = e.what(); if (job) res.info = job->info; }
-    if (res.status != Status::Ok) cudaStreamSynchronize(st);
-  }
-  // the stream must outlive the job's pending work; everything was synchronised above
-  cudaStreamDestroy(st);
-  return res;
+  if (!req.data) throw StatusError(DecoderStatus_NullParameter);
+  if (SignatureCheck(req.data, req.size) == 0) throw StatusError(DecoderStatus_InvalidFileSignature);
+  std::string why; JXLG_CHECK(CudaAvailable(&why), why);
+  cudaStream_t st = nullptr; JXLG_CHECK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking) == cudaSuccess, "cudaStreamCreate failed");
+  struct Stream { cudaStream_t s; ~Stream() { cudaStreamDestroy(s); } } stream{st};   // outlives the job below, and with it the job's pending work
+  std::shared_ptr<DecodeJob> job;
+  try {
+    size_t layered_pos = 0;
+    job = StartJob(req, st, true, req.band_begin || req.band_end ? nullptr : &layered_pos);
+    if (layered_pos) return DecodeLayered(req, *job, layered_pos, st);
+    job->Run(req); return DecodeFinish(job);
+  } catch (...) { cudaStreamSynchronize(st); throw; }   // the job gives its buffers back only after its work has drained
 }
 
 bool DecodeDebugPlanes(const std::shared_ptr<DecodeJob>& job, int which, std::vector<float>* out, int* xpad, int* ypad) {

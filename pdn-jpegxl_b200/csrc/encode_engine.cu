@@ -22,11 +22,6 @@ namespace jxlgpu {
 
 namespace {
 
-// Device buffers come from the engine's caching pool (cudaMalloc / cudaFree cost more than most encoder kernels; cudaFree also synchronises).
-// A buffer goes back to the pool only after the work that uses it has been synchronised (the sessions sync their stream before they let go).
-struct Buf { void* p = nullptr; size_t n = 0; void* pool = nullptr; void Alloc(size_t b) { Free(); n = b ? b : 1; p = DeviceGet(n, &pool); } void Free() { if (p) DevicePut(p, n, pool); p = nullptr; } ~Buf() { Free(); }
-  Buf() {} Buf(const Buf&) = delete; Buf& operator=(const Buf&) = delete; template <class T> T* as() const { return static_cast<T*>(p); } };
-
 // ---- fixed MA trees (same shape the decoder kernels walk; BFS layout as DecodeTree allocates it)
 struct TreeBuilder {
   struct Tmp { int prop; int32_t split; int l, r; int pred; }; std::vector<Tmp> n;
@@ -129,16 +124,6 @@ namespace {
 
 const size_t kNumAcCtx = size_t(495) * 15;
 
-// Everything that depends on the frame only (size, options, pixel format), never on pixels.
-struct EncPlan {
-  bool lossless = false, is_gray = false, has_alpha = false; int ncolor = 3, num_ec = 0, nplanes = 0;
-  ImageMetadata m; FrameHeader fh;
-  Tree tree; std::vector<Token> tree_tokens; EncCode tree_code; size_t nleaves = 0; std::vector<uint16_t> leaf_lut;
-  EncOptions mopt, aopt; uint32_t global_scale = 1, quant_lf = 16; float q_ac = 1;
-  bool groups_have_modular = false, global_has_modular = false, single = false, aq = false, cfl = false; GroupHeader plain, gheader;
-  size_t HistWords() const { return (nleaves + (lossless ? 0 : kNumAcCtx)) * kEncAlphabet; }
-};
-
 EncPlan MakePlan(uint32_t xs, uint32_t ys, uint32_t flags, const EncodeRequest& req) {
   EncPlan p; p.lossless = req.lossless;
   p.is_gray = !(flags & 1) && req.icc_size == 0; p.has_alpha = (flags & 2) != 0;
@@ -189,33 +174,7 @@ std::vector<std::vector<uint64_t>> TrimmedHist(const uint64_t* flat, size_t num_
 
 }  // namespace
 
-// kind: 0 global Modular stream, 1 LF group, 2 pass group. The payload is either owned (`bytes`) or a view into a band's serialised blob.
-struct BandSection { uint32_t kind = 0, index = 0; uint64_t bits = 0; std::vector<uint8_t> bytes; const uint8_t* view = nullptr; size_t view_n = 0;
-  const uint8_t* data() const { return view ? view : bytes.data(); } size_t size() const { return view ? view_n : bytes.size(); } };
-
-class BandEncoder {
- public:
-  explicit BandEncoder(const EncodeRequest& r) : req(r) {}
-  ~BandEncoder() { if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); } }
-  uint32_t Begin();                                         // -> flags of this band (bit 0: a non-gray pixel, bit 1: a non-opaque pixel)
-  std::vector<uint64_t> Tokenize(uint32_t frame_flags);     // -> this band's histograms, [context][kEncAlphabet] (Modular contexts, then AC contexts)
-  std::vector<BandSection> Finish(const std::vector<uint64_t>& frame_hist);
-  int64_t DebugStage(int32_t which, void* out, int64_t capacity, int64_t* dims4);   // JxlB200BandEncoderDebugStage
-  const EncPlan& Plan() const { return plan; }
-  float device_ms = 0;
-
- private:
-  struct Timer { cudaEvent_t a, b; cudaStream_t s; float* acc; Timer(cudaStream_t st_, float* acc_) : s(st_), acc(acc_) { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a, s); }
-    ~Timer() { cudaEventRecord(b, s); cudaEventSynchronize(b); float ms = 0; cudaEventElapsedTime(&ms, a, b); *acc += ms; cudaEventDestroy(a); cudaEventDestroy(b); } };
-  EncodeRequest req; cudaStream_t st = nullptr; EncPlan plan; DEncFrame e; FrameHeader fb;   // fb: frame header of the band taken as an image of its own (group / LF-group layout)
-  uint32_t frame_h = 0, lf_group0 = 0, group0 = 0;      // frame height; index of the band's first LF group / first group in the frame
-  const uint8_t* d_bgra = nullptr;                       // first row of the band itself (halo rows lie before it)
-  Buf d_in, d_flags, d_e, d_xyb, d_tmp1, d_tmp2, d_planes, d_lf, d_lfq, d_coeffs, d_nz, d_dq, d_order, d_tokens, d_account, d_lut, d_modstreams, d_streams, d_hist_m, d_hist_a, d_bytes, d_bits, d_gabframe, d_srclut, d_hfm, d_ytox, d_ytob, d_stats;
-  std::vector<DEncModStream> mod_streams; std::vector<DEncStream> m_streams, a_streams; std::vector<uint32_t> ac_counts;
-  uint32_t first_lf_stream = 0, first_group_stream = 0, max_mod_tokens = 0; uint64_t byte_cursor = 0;
-  std::vector<std::vector<Token>> hfmeta_tokens; std::vector<uint32_t> hfmeta_nb;
-  bool stages_valid = false;                             // between Tokenize and Finish: k_enc_ans overwrites the token words in place
-};
+size_t EncPlan::HistWords() const { return (nleaves + (lossless ? 0 : kNumAcCtx)) * kEncAlphabet; }
 
 uint32_t BandEncoder::Begin() {
   std::string why; JXLG_CHECK(CudaAvailable(&why), why);
@@ -514,25 +473,18 @@ std::vector<uint8_t> AssembleFile(const EncPlan& plan, const std::vector<uint64_
 }
 
 EncodeResult EncodeOnGpu(const EncodeRequest& req) {
-  EncodeResult res;
-  if (!req.bgra) { res.status = EncStatus::NullParameter; return res; }
-  try {
-    std::string why; if (!CudaAvailable(&why)) { res.status = EncStatus::EncodeError; res.message = why; return res; }
-    BandEncoder enc(req);
-    const uint32_t flags = enc.Begin();
-    const std::vector<uint64_t> hist = enc.Tokenize(flags);
-    const std::vector<BandSection> secs = enc.Finish(hist);
-    std::vector<const BandSection*> ptrs; for (const BandSection& s : secs) ptrs.push_back(&s);
-    res.file = AssembleFile(enc.Plan(), hist, ptrs, req);
-    res.pixel_format = enc.Plan().is_gray ? (enc.Plan().has_alpha ? 1 : 0) : (enc.Plan().has_alpha ? 3 : 2); res.times.total = enc.device_ms;
-  } catch (const std::bad_alloc&) { res.status = EncStatus::OutOfMemory; }
-  catch (const std::exception& ex) { res.status = EncStatus::EncodeError; res.message = ex.what(); }
+  if (!req.bgra) throw StatusError(EncoderStatus_NullParameter);
+  std::string why; JXLG_CHECK(CudaAvailable(&why), why);
+  BandEncoder enc(req);
+  const uint32_t flags = enc.Begin();
+  const std::vector<uint64_t> hist = enc.Tokenize(flags);
+  const std::vector<BandSection> secs = enc.Finish(hist);
+  std::vector<const BandSection*> ptrs; for (const BandSection& s : secs) ptrs.push_back(&s);
+  EncodeResult res; res.file = AssembleFile(enc.Plan(), hist, ptrs, req); res.times.total = enc.device_ms;
   return res;
 }
 
-// ---- band sessions behind the C ABI (JxlB200BandEncoder*)
-struct BandSession { std::unique_ptr<BandEncoder> enc; std::vector<uint8_t> icc, exif, xmp; EncodeRequest req; };
-
+// ---- the section blob a band session hands to AssembleBands
 static std::vector<uint8_t> SerializeSections(const std::vector<BandSection>& secs) {
   std::vector<uint8_t> out; auto put = [&](const void* p, size_t n) { const uint8_t* b = static_cast<const uint8_t*>(p); out.insert(out.end(), b, b + n); };
   const uint32_t magic = 0x4253584a, count = uint32_t(secs.size()); put(&magic, 4); put(&count, 4);
@@ -546,33 +498,13 @@ static std::vector<BandSection> ParseSections(const uint8_t* p, size_t n) {
   return out;
 }
 
-BandSession* BandEncoderCreate(const EncodeRequest& r, uint32_t* flags, EncStatus* status, std::string* message) {
-  std::unique_ptr<BandSession> s(new BandSession); s->req = r;
-  try {
-    if (r.icc_size) { s->icc.assign(r.icc, r.icc + r.icc_size); s->req.icc = s->icc.data(); }   // the session outlives the call: keep copies of the metadata
-    s->req.exif = nullptr; s->req.exif_size = 0; s->req.xmp = nullptr; s->req.xmp_size = 0;
-    s->enc.reset(new BandEncoder(s->req)); *flags = s->enc->Begin(); *status = EncStatus::Ok; return s.release();
-  } catch (const std::bad_alloc&) { *status = EncStatus::OutOfMemory; } catch (const std::exception& ex) { *status = EncStatus::EncodeError; *message = ex.what(); }
-  return nullptr;
-}
-EncStatus BandEncoderTokenize(BandSession* s, uint32_t frame_flags, std::vector<uint64_t>* hist, std::string* message) {
-  try { *hist = s->enc->Tokenize(frame_flags); return EncStatus::Ok; } catch (const std::bad_alloc&) { return EncStatus::OutOfMemory; } catch (const std::exception& ex) { *message = ex.what(); return EncStatus::EncodeError; }
-}
-EncStatus BandEncoderFinish(BandSession* s, const uint64_t* hist, size_t words, std::vector<uint8_t>* sections, float* device_ms, std::string* message) {
-  try { std::vector<uint64_t> h(hist, hist + words); *sections = SerializeSections(s->enc->Finish(h)); if (device_ms) *device_ms = s->enc->device_ms; return EncStatus::Ok; }
-  catch (const std::bad_alloc&) { return EncStatus::OutOfMemory; } catch (const std::exception& ex) { *message = ex.what(); return EncStatus::EncodeError; }
-}
-void BandEncoderDestroy(BandSession* s) { delete s; }
-int64_t BandEncoderDebugStage(BandSession* s, int32_t which, void* out, int64_t capacity, int64_t* dims4, std::string* message) {
-  try { return s->enc->DebugStage(which, out, capacity, dims4); } catch (const std::exception& ex) { *message = ex.what(); return 0; }
-}
-EncStatus AssembleBands(const EncodeRequest& frame, uint32_t frame_flags, const uint64_t* hist, size_t words, const uint8_t* const* blobs, const size_t* sizes, size_t count, std::vector<uint8_t>* file, std::string* message) {
-  try {
-    EncPlan plan = MakePlan(frame.width, frame.height, frame_flags, frame); std::vector<uint64_t> h(hist, hist + words);
-    std::vector<std::vector<BandSection>> all; for (size_t i = 0; i < count; i++) all.push_back(ParseSections(blobs[i], sizes[i]));
-    std::vector<const BandSection*> ptrs; for (auto& v : all) for (auto& s : v) ptrs.push_back(&s);
-    *file = AssembleFile(plan, h, ptrs, frame); return EncStatus::Ok;
-  } catch (const std::bad_alloc&) { return EncStatus::OutOfMemory; } catch (const std::exception& ex) { *message = ex.what(); return EncStatus::EncodeError; }
+std::vector<uint8_t> BandEncoder::FinishBlob(const std::vector<uint64_t>& frame_hist) { return SerializeSections(Finish(frame_hist)); }
+
+std::vector<uint8_t> AssembleBands(const EncodeRequest& frame, uint32_t frame_flags, const uint64_t* hist, size_t words, const uint8_t* const* blobs, const size_t* sizes, size_t count) {
+  EncPlan plan = MakePlan(frame.width, frame.height, frame_flags, frame); std::vector<uint64_t> h(hist, hist + words);
+  std::vector<std::vector<BandSection>> all; for (size_t i = 0; i < count; i++) all.push_back(ParseSections(blobs[i], sizes[i]));
+  std::vector<const BandSection*> ptrs; for (auto& v : all) for (auto& s : v) ptrs.push_back(&s);
+  return AssembleFile(plan, h, ptrs, frame);
 }
 
 }  // namespace jxlgpu

@@ -19,6 +19,11 @@ namespace jxlgpu {
 struct Error : std::runtime_error {
   explicit Error(const std::string& s) : std::runtime_error(s) {}
 };
+// A failure the C ABI reports with its own status (a DecoderStatus or EncoderStatus) instead of DecodeError / EncodeError.
+struct StatusError : Error {
+  int32_t status;
+  explicit StatusError(int32_t st, const std::string& s = std::string()) : Error(s), status(st) {}
+};
 #define JXLG_CHECK(c, msg) do { if (!(c)) throw ::jxlgpu::Error(msg); } while (0)
 
 // U32 distribution descriptor: Val(c) | Bits(n) | BitsOffset(n, off)   (SURVEY A.2)
