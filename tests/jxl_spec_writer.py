@@ -241,10 +241,23 @@ def passes(b, num_passes=1, shifts=(), downsample=(), last_pass=()):
 FLAG_NOISE, FLAG_PATCHES, FLAG_SPLINES, FLAG_USE_LF_FRAME, FLAG_SKIP_LF_SMOOTHING = 1, 2, 16, 32, 128
 
 
+RESTORATION_SIGMA = ("quant_mul", "pass0_sigma_scale", "pass2_sigma_scale", "border_sad_mul")
+
+
 def frame_header(b, modular, num_extra=0, xyb_encoded=False, flags=0, group_size_shift=1, num_passes=1, pass_shifts=(), name=b"",
-                 x_qm_scale=3, b_qm_scale=2, crop=None, canvas=None, blend=None, ec_blend=None, is_last=True, save_as_reference=0, gab=False, epf_iters=0):
-    """A regular frame without restoration filters. Defaults: full size, last, blend mode Replace. crop = (x0, y0, width, height) with
-    canvas = (image width, image height); blend / ec_blend[i] = dict(mode, alpha_channel, clamp, source) (F.2: BlendingInfo)."""
+                 x_qm_scale=3, b_qm_scale=2, crop=None, canvas=None, blend=None, ec_blend=None, is_last=True, save_as_reference=0, gab=False, epf_iters=0,
+                 restoration=None):
+    """A regular frame, by default without restoration filters. Defaults: full size, last, blend mode Replace. crop = (x0, y0, width, height) with
+    canvas = (image width, image height); blend / ec_blend[i] = dict(mode, alpha_channel, clamp, source) (F.2: BlendingInfo).
+    restoration: the RestorationFilter fields written instead of the defaults, where the syntax has them (gaborish weights only with gab, the
+    EPF fields only with epf_iters > 0), every value F16-exact:
+      all_default=True: the one-bit form (gaborish on with default weights, two EPF iterations; gab and epf_iters must say so);
+      gab_w: 6 values (x_w1, x_w2, y_w1, y_w2, b_w1, b_w2); sharp_lut: 8 values (VarDCT only);
+      channel_scale: 3 values, with zero_flush: the two 16-bit fields after them, which decoders skip (non-zero bits by default);
+      quant_mul (VarDCT only), pass0_sigma_scale, pass2_sigma_scale, border_sad_mul: all four together;
+      sigma_for_modular (Modular only; 1.0 when absent)."""
+    r = dict(restoration or {})
+    assert not set(r) - {"all_default", "gab_w", "sharp_lut", "channel_scale", "zero_flush", "sigma_for_modular"} - set(RESTORATION_SIGMA), r
     b.bool(False)                 # all_default
     b.u(2, 0)                     # frame_type: regular
     b.u(1, 1 if modular else 0)   # encoding
@@ -296,19 +309,41 @@ def frame_header(b, modular, num_extra=0, xyb_encoded=False, flags=0, group_size
     b.u32((("val", 0), ("bits", 4), ("bo", 5, 16), ("bo", 10, 48)), len(name))
     for ch in name:
         b.u(8, ch)
-    # RestorationFilter: not all_default (the default switches gaborish and two EPF iterations on); default weights and parameters
-    b.bool(False)
+    # RestorationFilter (all_default switches gaborish with its default weights and two EPF iterations on)
+    def f16s(key, n):
+        vals = list(r[key])
+        assert len(vals) == n, (key, vals)
+        for v in vals:
+            b.f16(f16_exact(float(v)))
+
+    b.bool(bool(r.get("all_default")))
+    if r.get("all_default"):
+        assert gab and epf_iters == 2 and set(r) == {"all_default"}
+        b.u64(0)                  # frame header extensions
+        return
     b.bool(gab)
     if gab:
-        b.bool(False)             # gab_custom
+        b.bool("gab_w" in r)      # gab_custom
+        if "gab_w" in r:
+            f16s("gab_w", 6)
     b.u(2, epf_iters)
     if epf_iters:
         if not modular:
-            b.bool(False)         # epf_sharp_custom
-        b.bool(False)             # epf_weight_custom
-        b.bool(False)             # epf_sigma_custom
+            b.bool("sharp_lut" in r)            # epf_sharp_custom
+            if "sharp_lut" in r:
+                f16s("sharp_lut", 8)
+        b.bool("channel_scale" in r)            # epf_weight_custom
+        if "channel_scale" in r:
+            f16s("channel_scale", 3)
+            for v in r.get("zero_flush", (0.4375, 0.625)):
+                b.f16(f16_exact(float(v)))      # two 16-bit fields no decoder uses
+        sigma = [k for k in RESTORATION_SIGMA if k in r and not (modular and k == "quant_mul")]
+        assert not sigma or len(sigma) == len(RESTORATION_SIGMA) - int(modular), "the sigma fields go together: %s" % sigma
+        b.bool(bool(sigma))                     # epf_sigma_custom
+        for k in sigma:
+            b.f16(f16_exact(float(r[k])))
         if modular:
-            b.f16(1.0)            # epf_sigma_for_modular
+            b.f16(f16_exact(float(r.get("sigma_for_modular", 1.0))))
     b.u64(0)                      # restoration filter extensions
     b.u64(0)                      # frame header extensions
 
@@ -1295,7 +1330,7 @@ class BlockCtxMap:
 
 def vardct_frame(xsize, ysize, lfq, blocks, ytox, ytob, coeffs, sharp=None, lf_dequant=None, global_scale=32768, quant_lf=64, extra_precision=0,
                  bctx=None, cfl=None, tables=None, presets=None, orders=None, pass_shift=None, code="ans", opsin=None, skip_smoothing=True,
-                 gab=False, epf_iters=0, x_qm_scale=3, b_qm_scale=2, wrong=None):
+                 gab=False, epf_iters=0, restoration=None, x_qm_scale=3, b_qm_scale=2, bits=8, exp_bits=0, color=None, orientation=1, wrong=None):
     """A complete XYB VarDCT image (codestream) whose every integer is the caller's:
       lfq: quantised LF, three (X, Y, B) integer arrays of yb x xb cells (row-major nested lists or numpy);
       blocks: [(by, bx, strategy, hf_mul)] covering every cell once, strategies from VARBLOCK, never across a 256-px group border;
@@ -1310,7 +1345,9 @@ def vardct_frame(xsize, ysize, lfq, blocks, ytox, ytob, coeffs, sharp=None, lf_d
       natural[perm[k]].
     code: "ans" (clustered ANS, 8 clusters), "prefix" (simple prefix codes; every value must be <= 3) or "lz77" (ANS + LZ77 copies at
       distances 1 .. 160).
-    opsin = (inverse matrix, bias, quant_bias) as image_metadata(). wrong: one of WRONG_RULES."""
+    opsin = (inverse matrix, bias, quant_bias) as image_metadata(); bits, exp_bits, color, orientation: the image's as image_metadata(), which
+    set the output's sample type, transfer function and orientation. gab, epf_iters, restoration: the restoration filters as frame_header().
+    wrong: one of WRONG_RULES."""
     import oracle_py                                    # natural coefficient orders only (jxlo_natural_order); everything else is this writer's
     import numpy as np
     assert wrong is None or wrong in WRONG_RULES
@@ -1453,10 +1490,11 @@ def vardct_frame(xsize, ysize, lfq, blocks, ytox, ytob, coeffs, sharp=None, lf_d
     b = Bits()
     b.u(16, 0x0AFF)
     size_header(b, xsize, ysize)
-    image_metadata(b, xyb_encoded=True, opsin=opsin)
+    image_metadata(b, bits=bits, exp_bits=exp_bits, xyb_encoded=True, orientation=orientation, color=color, opsin=opsin)
     b.pad_to_byte()
     frame_header(b, modular=False, xyb_encoded=True, flags=FLAG_SKIP_LF_SMOOTHING if skip_smoothing else 0, num_passes=npasses,
-                 pass_shifts=(pass_shift,) if npasses == 2 else (), x_qm_scale=x_qm_scale, b_qm_scale=b_qm_scale, gab=gab, epf_iters=epf_iters)
+                 pass_shifts=(pass_shift,) if npasses == 2 else (), x_qm_scale=x_qm_scale, b_qm_scale=b_qm_scale, gab=gab, epf_iters=epf_iters,
+                 restoration=restoration)
     single = ngroups == 1 and npasses == 1
     sections = []
     s = Bits()

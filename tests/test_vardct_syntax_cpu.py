@@ -8,6 +8,8 @@ import pytest
 import dec_reference as ref
 import jxl_spec_writer as jw
 import vardct_syntax_cases as vc
+from test_gpu_stages import TF_SRGB, orient, xyb_to_output
+from test_gpu_vardct_syntax import FILTER_F32_REL
 
 FP32_REL = 2e-6        # the oracle computes in fp32: relative to each channel's range
 
@@ -26,7 +28,8 @@ def _rel(got, want):
 def test_oracle_decodes_the_writers_integers(oracle, name):
     d, c = _decode(oracle, name)
     xb, yb = c["xb"], c["yb"]
-    assert (d.width, d.height, d.xpad, d.ypad) == (c["w"], c["h"], 8 * xb, 8 * yb)
+    w, h = (c["h"], c["w"]) if c["kw"]["orientation"] >= 5 else (c["w"], c["h"])     # the oriented image's size
+    assert (d.width, d.height, d.xpad, d.ypad) == (w, h, 8 * xb, 8 * yb)
     assert np.array_equal(d.stages["coeffs"].reshape(3, -1, 64), c["coeffs"])
     assert np.count_nonzero(c["coeffs"]) > 0
     assert np.array_equal(d.stages["lfq"], np.stack(c["lfq"]))
@@ -40,11 +43,16 @@ def test_oracle_decodes_the_writers_integers(oracle, name):
     assert (d.global_scale, d.quant_lf, d.x_qm_scale, d.b_qm_scale) == (kw["global_scale"], kw["quant_lf"], kw["x_qm_scale"], kw["b_qm_scale"])
 
 
-@pytest.mark.parametrize("name", [n for n in vc.NAMES if not vc.SPECS[n][2].get("smoothing")])
+@pytest.mark.parametrize("name", vc.NAMES)
 def test_oracle_lf_matches_float64(oracle, name):
     d, c = _decode(oracle, name)
     kw = c["kw"]
     want = ref.lf_planes(c["lfq"], kw["lf_dequant"], kw["global_scale"], kw["quant_lf"], kw["extra_precision"], kw["cfl"])
+    if not kw["skip_smoothing"]:
+        raw = want
+        want = ref.lf_smoothing(raw, kw["lf_dequant"], kw["global_scale"], kw["quant_lf"])
+        changed = np.abs(want - raw) > 1e-6 * np.abs(raw).max()
+        assert changed[:, 1:-1, 1:-1].mean() > 0.2, "smoothing changes too few LF samples of %s" % name
     err = _rel(d.stages["lf"], want)
     assert np.all(err <= FP32_REL), err
 
@@ -113,3 +121,68 @@ def test_mode6_table_from_library_parameters_equals_the_library_table(oracle):
 def test_raw_dequantisation_tables_are_refused(oracle):
     with pytest.raises(oracle.OracleError, match="RAW"):
         oracle.decode(vc.raw_table_file())
+
+
+# ------------------------------------------------------------------------------------------------ restoration filters
+def _restore(c, planes, switches=()):
+    kw = c["kw"]
+    return ref.restore(planes, c["w"], c["h"], kw["gab"], kw["epf_iters"], kw["restoration"], c["sharp"], c["blocks"], kw["global_scale"], switches)
+
+
+@pytest.mark.parametrize("name", vc.FILTER_NAMES)
+def test_oracle_filters_match_float64(oracle, name):
+    """The oracle's gaborish and EPF stages, fed with its own reconstruction, against the float64 reference (each stage on its own)."""
+    d, c = _decode(oracle, name)
+    kw, w, h = c["kw"], c["w"], c["h"]
+    st = {k: d.stages[k].reshape(3, d.ypad, d.xpad)[:, :h, :w] for k in ("idct", "gab", "epf")}
+    gab = ref.gaborish(st["idct"], ref.restoration_params(kw["restoration"])["gab_w"]) if kw["gab"] else st["idct"].astype(np.float64)
+    assert np.all(_rel(st["gab"], gab) <= FP32_REL), _rel(st["gab"], gab)
+    epf = ref.restore(st["gab"], w, h, False, kw["epf_iters"], kw["restoration"], c["sharp"], c["blocks"], kw["global_scale"])
+    assert np.all(_rel(st["epf"], epf) <= FP32_REL), _rel(st["epf"], epf)
+
+
+def test_filter_cases_sit_away_from_the_skip_threshold():
+    """EPF is continuous in its inputs except where a cell's inv_sigma crosses the skip threshold: no cell lies within 1e-4 of it, and every
+    EPF case with more than one cell has both filtered and skipped cells (the single-cell frames are filtered)."""
+    for name in vc.FILTER_NAMES:
+        c = vc._ints(name)
+        kw = c["kw"]
+        if not kw["epf_iters"]:
+            continue
+        isg = ref.inv_sigma(c["sharp"], c["blocks"], kw["global_scale"], ref.restoration_params(kw["restoration"]))
+        assert np.abs(isg / ref.MIN_INV_SIGMA - 1).min() > 1e-4, name
+        skipped = int((isg < ref.MIN_INV_SIGMA).sum())
+        assert 0 < skipped < isg.size if isg.size > 1 else skipped == 0, (name, skipped, isg.size)
+
+
+def test_filter_cases_carry_custom_and_default_parameters():
+    o = {n: vc.SPECS[n][2] for n in vc.FILTER_NAMES}
+    r = vc.RESTORATION
+    assert len(set(r["gab_w"][0::2])) == 3 and len(set(r["gab_w"][1::2])) == 3
+    lut = list(r["sharp_lut"])
+    assert 0.0 in lut and lut != sorted(lut) and any(r[k] != ref.DEFAULT_RESTORATION[k] for k in ("quant_mul", "border_sad_mul"))
+    assert r["pass0_sigma_scale"] != ref.DEFAULT_RESTORATION["pass0_sigma_scale"] and r["pass2_sigma_scale"] != ref.DEFAULT_RESTORATION["pass2_sigma_scale"]
+    assert [n for n in o if not o[n].get("restoration")] == ["gab_epf1"]
+    assert [n for n in o if (o[n].get("restoration") or {}).get("all_default")] == ["all_default_224x100"]
+    assert any(o[n].get("epf") == 3 and -(-vc.SPECS[n][1] // 256) >= 3 for n in o)
+
+
+def _output(c, xyb):
+    kw = c["kw"]
+    inv, bias, _ = kw["opsin"]
+    tf = (kw["color"] or {}).get("tf", TF_SRGB)
+    return orient(xyb_to_output(xyb, tf=tf, opsin_inv=inv, opsin_bias=[-v for v in bias]), kw["orientation"])
+
+
+@pytest.mark.parametrize("switch", ref.SWITCHES)
+def test_each_filter_rule_matters(oracle, switch):
+    """Each rule of the reference, applied differently, moves some case's output samples by at least 20x the bound the GPU's samples are held
+    to (FILTER_F32_REL, relative to max(|sample|, 1e-3)): the cases can tell each rule from its alternative."""
+    worst = 0.0
+    for name in vc.FILTER_NAMES:
+        d, c = _decode(oracle, name)
+        idct = d.stages["idct"].reshape(3, d.ypad, d.xpad).astype(np.float64)
+        real = _output(c, _restore(c, idct))
+        moved = _output(c, _restore(c, idct, (switch,)))
+        worst = max(worst, float((np.abs(moved - real) / np.maximum(np.abs(real), 1e-3)).max()))
+    assert worst >= 20 * FILTER_F32_REL, "%s moves the output by %.3g at most" % (switch, worst)

@@ -28,6 +28,15 @@ TABLES_DCT8_SINGLE = {0: [[40.0 * 64], [10.0 * 64], [6.0 * 64]]}
 LF_THR = ([-20], [0, 60], [10])
 QF_THR = [2, 5, 40, 121]
 HF_MULS = [1, 2, 3, 5, 6, 40, 41, 121, 122, 200, 256]  # the thresholds themselves (a >= / > difference), both ends of the range
+# Restoration parameters no encoder writes (F16-exact): distinct gaborish weights per channel, a non-monotone sharpness LUT with zeros,
+# channel scales, sigma scales and border multiplier away from the defaults, non-zero bits in the two skipped 16-bit fields
+RESTORATION = dict(gab_w=(0.125, 0.0625, 0.09375, 0.03125, 0.15625, 0.046875), sharp_lut=(0.0, 0.75, 0.25, 1.25, 0.0, 0.5, 1.0, 0.375),
+                   channel_scale=(32.0, 6.5, 2.5), zero_flush=(0.4375, 0.625), quant_mul=0.53125, pass0_sigma_scale=0.75, pass2_sigma_scale=5.0,
+                   border_sad_mul=0.5)
+# Small coefficients and LF (XYB within about +-1): larger samples would leave the colour conversion's cube and opsin matrix to cancel
+# values of 1e4 in linear light, and the rendered samples could no longer be held to fp32 level
+FILTERED = dict(strategies=[0, 0, 4, 7], bctx=True, cfl=True, tables=TABLES, orders=True, opsin=True, amp=1, lf_amp=40, global_scale=3000,
+                quant_lf=20, restoration=RESTORATION)
 
 
 def block_ctx_map(rng, n=8):
@@ -114,9 +123,33 @@ SPECS = {
     # adaptive LF smoothing on
     "smoothing": (264, 200, dict(strategies=[0, 0, 4, 7], bctx=True, cfl=True, lf_dequant=True, tables=TABLES, orders=True, opsin=True, amp=15,
                                  smoothing=True, global_scale=3000, quant_lf=20)),
-    # gaborish + one EPF iteration: the wide TMA render kernel with a custom opsin matrix
+    # gaborish + one EPF iteration: the wide TMA render kernel with a custom opsin matrix and the default filter parameters
     "gab_epf1": (256, 160, dict(strategies=[0, 0, 4, 7], bctx=True, cfl=True, tables=TABLES, orders=True, opsin=True, amp=15, gab=True, epf=1,
                                 global_scale=3000, quant_lf=20)),
+    # Restoration filters with the custom parameters (RESTORATION) unless noted; the render kernel each case selects is in
+    # test_gpu_vardct_syntax.RENDER_KERNEL. Sizes at 32k +- 1 and 64k +- 1, widths of 4k (k_render<.., true>) and not.
+    "epf1_260x97": (260, 97, dict(FILTERED, epf=1)),
+    "epf1_95x63": (95, 63, dict(FILTERED, epf=1)),
+    "epf2_128x65": (128, 65, dict(FILTERED, epf=2)),
+    "epf2_161x33": (161, 33, dict(FILTERED, epf=2)),
+    "epf3_132x67": (132, 67, dict(FILTERED, epf=3)),
+    "gab_192x129": (192, 129, dict(FILTERED, gab=True)),
+    "gab_127x95": (127, 95, dict(FILTERED, gab=True)),
+    # the one-bit all_default form: gaborish and two EPF iterations with the default parameters, adaptive LF smoothing on
+    "all_default_224x100": (224, 100, dict(FILTERED, gab=True, epf=2, restoration=dict(all_default=True), smoothing=True)),
+    # 3 group rows (band decodes), the 7-px halo of gaborish + EPF 3 across the group and band borders
+    "bands_300x530": (300, 530, dict(FILTERED, gab=True, epf=3)),
+    # frames smaller than the 7-px (or 4-px) halo: it reflects more than once
+    "tiny_1x1": (1, 1, dict(FILTERED, strategies=[0], epf=3)),
+    "tiny_5x3": (5, 3, dict(FILTERED, strategies=[0], gab=True, epf=2)),
+    "tiny_9x7": (9, 7, dict(FILTERED, strategies=[0], gab=True, epf=3, global_scale=500)),   # a coarser quantiser: one of its two cells is filtered
+    # the wide kernel with custom parameters: interior (TMA) tiles, and a frame without one
+    "wide_193x161": (193, 161, dict(FILTERED, gab=True, epf=1)),
+    "wide_129x63": (129, 63, dict(FILTERED, gab=True, epf=1)),
+    # other outputs of gaborish + EPF 1 (k_render<1,1,false>): 16-bit samples in orientation 6, and DCT8-only f32 linear samples
+    # (the case the float64 chain runs from the writer's integers alone)
+    "u16_orient6_200x136": (200, 136, dict(FILTERED, gab=True, epf=1, bits=16, orientation=6)),
+    "dct8_f32_linear": (203, 150, dict(FILTERED, strategies=[0], gab=True, epf=1, bits=32, exp_bits=8, color=dict(tf=jw.TF_LINEAR))),
 }
 
 
@@ -127,6 +160,14 @@ def raw_table_file():
     return jw.vardct_frame(c["w"], c["h"], c["lfq"], c["blocks"], c["ytox"], c["ytob"], c["coeffs"], **kw)
 
 
+def smooth_lf_field(rng, c, xb, yb):
+    """Quantised LF of channel c for a case with adaptive LF smoothing: a smooth field plus 0 / +-1 noise in about half the cells, so that
+    the smoothing gate takes all three of its branches (smoothed, blended, kept) in many cells; random LF would keep every sample."""
+    y, x = np.mgrid[0:yb, 0:xb]
+    noise = rng.integers(-1, 2, (yb, xb)) * (rng.random((yb, xb)) < 0.5)
+    return np.round(30 * np.sin(x / 6.0 + c) + 20 * np.cos(y / 5.0 - c) + 0.5 * x).astype(np.int64) + noise
+
+
 def _ints(name):
     """The integers of case `name` (seeded by its name): dict(w, h, xb, yb, lfq, blocks, ytox, ytob, sharp, coeffs, kwargs for vardct_frame)."""
     w, h, o = SPECS[name]
@@ -134,7 +175,8 @@ def _ints(name):
     xb, yb = -(-w // 8), -(-h // 8)
     yt, xt = -(-yb // 8), -(-xb // 8)
     smooth_lf = o.get("smoothing")
-    lfq = [rng.integers(-40, 41, (yb, xb)) if smooth_lf else rng.integers(-300, 301, (yb, xb)) for _ in range(3)]
+    lf_amp = o.get("lf_amp", 300)
+    lfq = [smooth_lf_field(rng, c, xb, yb) if smooth_lf else rng.integers(-lf_amp, lf_amp + 1, (yb, xb)) for c in range(3)]
     blocks = layout(rng, xb, yb, o["strategies"])
     ytox, ytob = rng.integers(-128, 128, (yt, xt)), rng.integers(-128, 128, (yt, xt))
     ytox.flat[0], ytob.flat[-1] = -128, 127
@@ -150,7 +192,8 @@ def _ints(name):
               presets=[g % 3 for g in range(ngroups)] if o.get("presets") and ngroups > 1 else None,
               orders=permutations(rng, used_orders, npasses) if o.get("orders") else None, pass_shift=o.get("pass_shift"), code=o.get("code", "ans"),
               opsin=OPSIN if o.get("opsin") else None, skip_smoothing=not smooth_lf, gab=bool(o.get("gab")), epf_iters=o.get("epf", 0),
-              x_qm_scale=o.get("x_qm_scale", 3), b_qm_scale=o.get("b_qm_scale", 2))
+              restoration=o.get("restoration"), x_qm_scale=o.get("x_qm_scale", 3), b_qm_scale=o.get("b_qm_scale", 2), bits=o.get("bits", 8),
+              exp_bits=o.get("exp_bits", 0), color=o.get("color"), orientation=o.get("orientation", 1))
     return dict(w=w, h=h, xb=xb, yb=yb, lfq=lfq, blocks=blocks, ytox=ytox, ytob=ytob, sharp=sharp, coeffs=coeffs, kw=kw)
 
 
@@ -163,3 +206,4 @@ def case(name, wrong=None):
 
 
 NAMES = list(SPECS)
+FILTER_NAMES = [n for n in NAMES if SPECS[n][2].get("gab") or SPECS[n][2].get("epf")]
