@@ -41,9 +41,12 @@ template <class Result, class Request> Result WithTimes(Result (*call)(const Req
 
 // The one place where the engine's exceptions become what a C caller sees. `body` returns the status of a call that did not throw;
 // a failure becomes StatusError's status, OutOfMemory, or DecodeError / EncodeError, with the exception's text in ErrorInfo.
+// The thread's CUDA error state is cleared when a call enters and when it leaves: a runtime call that failed and was reported (an invalid
+// device index) or was unchecked on purpose would otherwise be read by the launch check of a later call and fail that call instead.
 struct Decoding { static const int32_t kOutOfMemory = DecoderStatus_OutOfMemory, kError = DecoderStatus_DecodeError; };
 struct Encoding { static const int32_t kOutOfMemory = EncoderStatus_OutOfMemory, kError = EncoderStatus_EncodeError; };
 template <class Codec, class F> int32_t Guard(ErrorInfo* ei, F&& body) {
+  struct ClearCudaError { ClearCudaError() { cudaGetLastError(); } ~ClearCudaError() { cudaGetLastError(); } } clear;
   try { return body(); }
   catch (const StatusError& e) { SetErrorMessage(ei, std::string(e.what())); return e.status; }
   catch (const std::bad_alloc&) { return Codec::kOutOfMemory; }
@@ -269,7 +272,7 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
       for (int i = 0; i < count; i++) in_off[i + 1] = in_off[i] + ((a.dataSizes[begin + i] + 63) & ~size_t(63));
       pin_bytes = in_off[count] + 64; pin = PinnedGet(pin_bytes); in_ready.resize(size_t(count), nullptr);
       for (int i = 0; i < count; i++) {
-        cudaMemcpyAsync(static_cast<uint8_t*>(pin) + in_off[i], a.datas[begin + i], a.dataSizes[begin + i], cudaMemcpyDeviceToHost, copy_stream);
+        CUDA_OK(cudaMemcpyAsync(static_cast<uint8_t*>(pin) + in_off[i], a.datas[begin + i], a.dataSizes[begin + i], cudaMemcpyDeviceToHost, copy_stream));
         if (cudaEventCreateWithFlags(&in_ready[i], cudaEventDisableTiming) != cudaSuccess || cudaEventRecord(in_ready[i], copy_stream) != cudaSuccess)
           throw std::runtime_error("cannot read device inputs");
       }
@@ -307,7 +310,8 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
       if (st != DecoderStatus_Ok) { record(f.idx, st, ei.errorMessage); f.job.reset(); done++; }
       return st == DecoderStatus_Ok;
     };
-    auto idle = [](const Bundle& b) { return cudaStreamQuery(b.stream) != cudaErrorNotReady; };
+    // A busy stream answers cudaErrorNotReady, which is cleared so that the launch checks of this thread do not report it as a failure.
+    auto idle = [](const Bundle& b) { const cudaError_t e = cudaStreamQuery(b.stream); if (e == cudaErrorNotReady) cudaGetLastError(); return e != cudaErrorNotReady; };
     auto jobs_of = [](Bundle& b) { std::vector<std::shared_ptr<DecodeJob>> v; for (auto& it : b.items) v.push_back(it->job); return v; };
     auto next_phase = [&](Bundle& b, int phase) {   // enqueue `phase` for every image of the bundle; images that fail are finished and dropped
       for (size_t k = 0; k < b.items.size();) {
@@ -353,7 +357,7 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
           const int li = next++, i = begin + li;
           std::unique_ptr<InFlight> f(new InFlight); f->idx = i;
           DecodeRequest req; req.bgra = a.bgra != 0; req.device_output = !a.hostOutputs; req.size = a.dataSizes[i]; req.out_capacity = a.outputBytes[i]; req.ac_lanes = batch_lanes;
-          if (a.hostInputs) req.data = a.datas[i]; else { cudaEventSynchronize(in_ready[li]); req.data = host_in + in_off[li]; req.device_input = a.datas[i]; }
+          if (a.hostInputs) req.data = a.datas[i]; else { CUDA_OK(cudaEventSynchronize(in_ready[li])); req.data = host_in + in_off[li]; req.device_input = a.datas[i]; }
           if (!a.hostOutputs) { req.out_device = a.outputs[i]; f->direct = true; } else if (out_is_pinned[li]) { req.out_pinned = a.outputs[i]; f->direct = true; }
           if (reserve_sets == 0 && a.count >= 32) for (int spin = 0; spin < 40000 && !g_pools_warm[cur_dev & 63].load(); spin++) std::this_thread::sleep_for(std::chrono::microseconds(50));   // at most 2 s, first batch only
           bool layered = false;
@@ -500,7 +504,7 @@ JxlB200BandEncoder* JxlB200BandEncoderCreate(int32_t device, const BitmapData* b
 EncoderStatus JxlB200BandEncoderTokenize(JxlB200BandEncoder* enc, uint32_t frameFlags, uint64_t** hist, size_t* histWords, ErrorInfo* errorInfo) {
   if (!enc || !hist || !histWords) return EncoderStatus_NullParameter;
   return Guard<Encoding>(errorInfo, [&] {
-    if (enc->device >= 0) cudaSetDevice(enc->device);
+    JXLG_CHECK(enc->device < 0 || cudaSetDevice(enc->device) == cudaSuccess, "cudaSetDevice failed");
     const std::vector<uint64_t> h = enc->enc->Tokenize(frameFlags);
     *hist = static_cast<uint64_t*>(CopyOut(h.data(), h.size() * 8)); *histWords = h.size(); return EncoderStatus_Ok;
   });
@@ -508,7 +512,7 @@ EncoderStatus JxlB200BandEncoderTokenize(JxlB200BandEncoder* enc, uint32_t frame
 EncoderStatus JxlB200BandEncoderFinish(JxlB200BandEncoder* enc, const uint64_t* frameHist, size_t histWords, uint8_t** sections, size_t* sectionBytes, float* deviceMs, ErrorInfo* errorInfo) {
   if (!enc || !frameHist || !sections || !sectionBytes) return EncoderStatus_NullParameter;
   return Guard<Encoding>(errorInfo, [&] {
-    if (enc->device >= 0) cudaSetDevice(enc->device);
+    JXLG_CHECK(enc->device < 0 || cudaSetDevice(enc->device) == cudaSuccess, "cudaSetDevice failed");
     const std::vector<uint8_t> blob = enc->enc->FinishBlob(std::vector<uint64_t>(frameHist, frameHist + histWords)); if (deviceMs) *deviceMs = enc->enc->device_ms;
     *sections = static_cast<uint8_t*>(CopyOut(blob.data(), blob.size())); *sectionBytes = blob.size(); return EncoderStatus_Ok;
   });
@@ -516,7 +520,7 @@ EncoderStatus JxlB200BandEncoderFinish(JxlB200BandEncoder* enc, const uint64_t* 
 int64_t JxlB200BandEncoderDebugStage(JxlB200BandEncoder* enc, int32_t which, void* out, int64_t capacityBytes, int64_t* dims4, ErrorInfo* errorInfo) {
   if (!enc) { SetErrorMessage(errorInfo, "null parameter"); return 0; }
   int64_t n = 0;
-  Guard<Encoding>(errorInfo, [&] { if (enc->device >= 0) cudaSetDevice(enc->device); n = enc->enc->DebugStage(which, out, capacityBytes, dims4); return EncoderStatus_Ok; });
+  Guard<Encoding>(errorInfo, [&] { JXLG_CHECK(enc->device < 0 || cudaSetDevice(enc->device) == cudaSuccess, "cudaSetDevice failed"); n = enc->enc->DebugStage(which, out, capacityBytes, dims4); return EncoderStatus_Ok; });
   return n;
 }
 void JxlB200BandEncoderDestroy(JxlB200BandEncoder* enc) {

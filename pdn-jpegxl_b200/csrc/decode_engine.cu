@@ -29,8 +29,6 @@ static inline double NowMs() { return std::chrono::duration<double, std::milli>(
 void DumpHostTrace() { if (!g_trace.n) return; fprintf(stderr, "[jxlb200] host ms/image: headers %.2f setup %.2f lfglobal %.2f hfglobal %.2f alloc+upload %.2f blob %.2f launch %.2f\n", g_trace.t[0] / g_trace.n, g_trace.t[1] / g_trace.n, g_trace.t[2] / g_trace.n, g_trace.t[3] / g_trace.n, g_trace.t[4] / g_trace.n, g_trace.t[5] / g_trace.n, g_trace.t[6] / g_trace.n); g_trace = HostTrace(); }
 
 // ---------------------------------------------------------------- small utilities
-#define CUDA_OK(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) throw Error(std::string("CUDA: ") + cudaGetErrorString(e_) + " at " #expr); } while (0)
-
 bool CudaAvailable(std::string* why) {
   int n = 0; cudaError_t e = cudaGetDeviceCount(&n);
   if (e != cudaSuccess || n == 0) { if (why) *why = std::string("no usable CUDA device (") + (e != cudaSuccess ? cudaGetErrorString(e) : "device count is 0") + "); the engine has no CPU fallback"; cudaGetLastError(); return false; }
@@ -580,10 +578,10 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
   const DFrame* d = d_frame.as<DFrame>();
   if (timed) cudaEventRecord(ev[0], stream);
   // global Modular stream
-  if (global_has_data) { LaunchModularGlobal(d, h, after_lfglobal, uint32_t(global_decoded), stream); CountLaunch(); }
+  if (global_has_data) LaunchModularGlobal(d, h, after_lfglobal, uint32_t(global_decoded), stream);
   else if (single) { uint64_t* slot = reinterpret_cast<uint64_t*>(h_misc.as<uint8_t>() + 2 * sizeof(DFrame)); slot[0] = after_lfglobal; CUDA_OK(cudaMemcpyAsync(h.end_bitpos, slot, 8, cudaMemcpyHostToDevice, stream)); }
   if (!vardct && !single && mod_has_lf_level) LaunchModLfGroups(h, stream);   // Modular frames: channels of shift >= 3 live in the LF-group sections
-  if (vardct) { if (defer_entropy && !single) lf_pending = true; else { LaunchLfGroups(d, h, stream); CountLaunch(); } }
+  if (vardct) { if (defer_entropy && !single) lf_pending = true; else LaunchLfGroups(d, h, stream); }
   else if (single) { /* Modular frame, single section: LF group and HfGlobal parts are empty; groups continue where the global stream ended */ CUDA_OK(cudaMemcpyAsync(h.end_bitpos + 2, h.end_bitpos, 8, cudaMemcpyDeviceToDevice, stream)); }
   if (single && vardct) {   // HfGlobal follows the LF group in the same bit stream: need its end position on the host
     uint64_t pos[3] = {0, 0, 0}; CUDA_OK(cudaMemcpyAsync(h_err.p, d_err.p, 64, cudaMemcpyDeviceToHost, stream)); CUDA_OK(cudaStreamSynchronize(stream));
@@ -599,10 +597,10 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
 void DecodeJob::RunAc() {
   const bool vardct = h.encoding == 0; const DFrame* d = d_frame.as<DFrame>(); double tt = NowMs();
   if (timed) cudaEventRecord(ev[1], stream);
-  if (vardct) { bool smooth = h.lf_src == h.lf_tmp; LaunchLfDequant(d, h, smooth, stream); CountLaunch(smooth ? 2 : 1); }
+  if (vardct) LaunchLfDequant(d, h, h.lf_src == h.lf_tmp, stream);
   if (vardct) CUDA_OK(cudaMemsetAsync(d_coeffs.p, 0, coeffs_bytes, stream));
   if (defer_entropy && vardct && h.num_passes == 1 && h.ac_fast && !(h.num_mod_channels > h.first_group_channel)) ac_pending = true;
-  else for (uint32_t p = 0; p < h.num_passes; p++) CountLaunch(LaunchAcGroups(d, h, int(p), ac_lanes, stream));
+  else for (uint32_t p = 0; p < h.num_passes; p++) LaunchAcGroups(d, h, int(p), ac_lanes, stream);
   if (timed) cudaEventRecord(ev[2], stream);
   g_trace.t[6] += NowMs() - tt;
 }
@@ -640,7 +638,7 @@ static bool FirstFrameIsPlain(const Headers& hd, size_t* first_pos) {
 // a file whose first frame is not plain is left for compositing: the job holds only its headers, and *layered_pos receives that frame's position.
 static std::shared_ptr<DecodeJob> StartJob(const DecodeRequest& req, cudaStream_t stream, bool timed, size_t* layered_pos = nullptr) {
   std::shared_ptr<DecodeJob> job = std::make_shared<DecodeJob>(); job->stream = stream;
-  if (timed) { job->timed = true; for (int i = 0; i < 7; i++) cudaEventCreate(&job->ev[i]); }
+  if (timed) { job->timed = true; for (int i = 0; i < 7; i++) cudaEventCreate(&job->ev[i]); }   // stage timing only: ev calls are not checked
   double t0 = NowMs(); ParseHeadersInto(req.data, req.size, &job->hd, &job->info); g_trace.t[0] += NowMs() - t0;
   if (layered_pos && !FirstFrameIsPlain(job->hd, layered_pos)) return job;
   if (layered_pos) *layered_pos = 0;
@@ -669,7 +667,7 @@ void DecodeEnqueuePhase(const std::shared_ptr<DecodeJob>& job, int phase) {
 void DecodeBundleLaunch(const std::vector<std::shared_ptr<DecodeJob>>& jobs, int phase) {
   for (int kind = 0; kind < 2; kind++) {   // LF: narrow / wide Modular kernels; AC: one kind
     DFrameSet set; set.n = 0; cudaStream_t st = nullptr; int lanes = 1;
-    auto flush = [&]() { if (!set.n) return; if (phase == 1) LaunchLfGroupsMulti(set, kind == 0, st); else LaunchAcGroupsMulti(set, lanes, st); CountLaunch(); set.n = 0; };
+    auto flush = [&]() { if (!set.n) return; if (phase == 1) LaunchLfGroupsMulti(set, kind == 0, st); else LaunchAcGroupsMulti(set, lanes, st); set.n = 0; };
     for (const auto& j : jobs) {
       if (!j) continue;
       if (phase == 1) { if (!j->lf_pending || LfNarrow(j->h) != (kind == 0)) continue; }

@@ -81,13 +81,12 @@ __global__ void __launch_bounds__(256) k_finalize_canvas_bgra(const float* __res
 
 void LaunchBlendLayer(float* canvas, const float* frame, int W, int H, int fw, int fh, int x0, int y0, int C, int cc, uint32_t cmode, uint32_t amode, bool cclamp, bool aclamp, bool premultiplied, cudaStream_t st) {
   if (fw <= 0 || fh <= 0) return; dim3 grid((fw + 255) / 256, fh);
-  k_blend_layer<<<grid, 256, 0, st>>>(canvas, frame, W, H, fw, fh, x0, y0, C, cc, cmode, amode, cclamp, aclamp, premultiplied); CountLaunch();
+  Launch<k_blend_layer>(grid, 256, 0, st, canvas, frame, W, H, fw, fh, x0, y0, C, cc, cmode, amode, cclamp, aclamp, premultiplied);
 }
 void LaunchFinalizeCanvas(const float* canvas, uint8_t* out, int W, int H, int C, int cc, bool premultiplied, uint32_t sample_type, uint32_t orientation, bool bgra, cudaStream_t st) {
   dim3 grid((W + 255) / 256, H);
-  if (bgra) k_finalize_canvas_bgra<<<grid, 256, 0, st>>>(canvas, reinterpret_cast<uint32_t*>(out), W, H, C, cc, premultiplied, orientation);
-  else k_finalize_canvas<<<grid, 256, 0, st>>>(canvas, out, W, H, C, cc, premultiplied, sample_type, orientation);
-  CountLaunch();
+  if (bgra) Launch<k_finalize_canvas_bgra>(grid, 256, 0, st, canvas, reinterpret_cast<uint32_t*>(out), W, H, C, cc, premultiplied, orientation);
+  else Launch<k_finalize_canvas>(grid, 256, 0, st, canvas, out, W, H, C, cc, premultiplied, sample_type, orientation);
 }
 
 }  // namespace jxlgpu

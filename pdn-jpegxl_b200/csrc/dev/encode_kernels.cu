@@ -15,7 +15,7 @@
 namespace jxlgpu {
 
 __device__ __constant__ float kSrgbLut[256];
-void UploadSrgbLut(const float* lut) { cudaMemcpyToSymbol(kSrgbLut, lut, 256 * sizeof(float)); }
+void UploadSrgbLut(const float* lut) { CUDA_OK(cudaMemcpyToSymbol(kSrgbLut, lut, 256 * sizeof(float))); }
 
 __global__ void k_enc_scan(const uint8_t* __restrict__ bgra, uint32_t w, uint32_t h, uint32_t stride, uint32_t* flags) {
   uint32_t x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y; uint32_t f = 0;
@@ -312,24 +312,24 @@ __global__ void __launch_bounds__(256) k_enc_compact(const uint8_t* __restrict__
   for (uint64_t i = threadIdx.x; i < nvec; i += 256) d[i] = s[i];
 }
 void EncLaunchCompact(const uint8_t* src, const DEncStream* streams, uint32_t nstreams, const uint64_t* bits, const uint64_t* dst_off, uint8_t* dst, cudaStream_t st) {
-  if (!nstreams) return; k_enc_compact<<<nstreams, 256, 0, st>>>(src, streams, bits, dst_off, dst); CountLaunch();
+  if (!nstreams) return; Launch<k_enc_compact>(nstreams, 256, 0, st, src, streams, bits, dst_off, dst);
 }
-void EncLaunchScan(const uint8_t* bgra, uint32_t w, uint32_t h, uint32_t stride, uint32_t* flags, cudaStream_t st) { dim3 grid((w + 255) / 256, h); k_enc_scan<<<grid, 256, 0, st>>>(bgra, w, h, stride, flags); CountLaunch(); }
-void EncLaunchToXyb(const DEncFrame* d, const DEncFrame& h, const uint8_t* bgra, cudaStream_t st) { dim3 blk(32, 8), grid((h.xpad + 31) / 32, (h.ext_rows + 7) / 8); k_enc_to_xyb<<<grid, blk, 0, st>>>(d, bgra); CountLaunch(); }
-void EncLaunchToPlanes(const DEncFrame* d, const DEncFrame& h, const uint8_t* bgra, cudaStream_t st) { dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8); k_enc_to_planes<<<grid, blk, 0, st>>>(d, bgra); CountLaunch(); }
-void EncLaunchSharpen(float* cur, const float* orig, const float* blur, size_t n, cudaStream_t st) { k_enc_sharpen<<<unsigned((n + 255) / 256), 256, 0, st>>>(cur, orig, blur, n); CountLaunch(); }
+void EncLaunchScan(const uint8_t* bgra, uint32_t w, uint32_t h, uint32_t stride, uint32_t* flags, cudaStream_t st) { dim3 grid((w + 255) / 256, h); Launch<k_enc_scan>(grid, 256, 0, st, bgra, w, h, stride, flags); }
+void EncLaunchToXyb(const DEncFrame* d, const DEncFrame& h, const uint8_t* bgra, cudaStream_t st) { dim3 blk(32, 8), grid((h.xpad + 31) / 32, (h.ext_rows + 7) / 8); Launch<k_enc_to_xyb>(grid, blk, 0, st, d, bgra); }
+void EncLaunchToPlanes(const DEncFrame* d, const DEncFrame& h, const uint8_t* bgra, cudaStream_t st) { dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8); Launch<k_enc_to_planes>(grid, blk, 0, st, d, bgra); }
+void EncLaunchSharpen(float* cur, const float* orig, const float* blur, size_t n, cudaStream_t st) { Launch<k_enc_sharpen>(unsigned((n + 255) / 256), 256, 0, st, cur, orig, blur, n); }
 void EncLaunchBlockParams(const DEncFrame* d, const DEncFrame& h, cudaStream_t st) {
-  const uint32_t cells = h.xb * h.yb, tiles = h.xt * h.yt; k_enc_block_stats<<<(cells + 63) / 64, 64, 0, st>>>(d); k_enc_tile_params<<<(tiles + 3) / 4, 128, 0, st>>>(d); CountLaunch(2);
+  const uint32_t cells = h.xb * h.yb, tiles = h.xt * h.yt; Launch<k_enc_block_stats>((cells + 63) / 64, 64, 0, st, d); Launch<k_enc_tile_params>((tiles + 3) / 4, 128, 0, st, d);
 }
-void EncLaunchDct8(const DEncFrame* d, const DEncFrame& h, cudaStream_t st) { uint32_t cells = h.xb * h.yb; k_enc_dct8<<<(cells + 63) / 64, 64, 0, st>>>(d); k_enc_lf_quant<<<(cells + 255) / 256, 256, 0, st>>>(d); CountLaunch(2); }
+void EncLaunchDct8(const DEncFrame* d, const DEncFrame& h, cudaStream_t st) { uint32_t cells = h.xb * h.yb; Launch<k_enc_dct8>((cells + 63) / 64, 64, 0, st, d); Launch<k_enc_lf_quant>((cells + 255) / 256, 256, 0, st, d); }
 void EncLaunchModTokens(const DEncFrame* d, const DEncModStream* streams, uint32_t nstreams, uint32_t max_tokens, const int32_t* planes, uint32_t pw, uint32_t ph, uint32_t nch, const uint16_t* leaf_lut, cudaStream_t st) {
-  if (!nstreams || !max_tokens) return; dim3 grid((max_tokens + 255) / 256, nstreams); k_enc_mod_tokens<<<grid, 256, 0, st>>>(d, streams, planes, pw, ph, nch, leaf_lut); CountLaunch();
+  if (!nstreams || !max_tokens) return; dim3 grid((max_tokens + 255) / 256, nstreams); Launch<k_enc_mod_tokens>(grid, 256, 0, st, d, streams, planes, pw, ph, nch, leaf_lut);
 }
-void EncLaunchAcTokens(const DEncFrame* d, const DEncFrame& h, cudaStream_t st) { if (!h.num_groups) return; k_enc_ac_tokens<<<h.num_groups, 1024, 0, st>>>(d); CountLaunch(); }
+void EncLaunchAcTokens(const DEncFrame* d, const DEncFrame& h, cudaStream_t st) { if (!h.num_groups) return; Launch<k_enc_ac_tokens>(h.num_groups, 1024, 0, st, d); }
 void EncLaunchHistogram(const uint2* tokens, const DEncStream* streams, uint32_t nstreams, uint32_t max_count, uint32_t* hist, cudaStream_t st) {
-  if (!nstreams || !max_count) return; dim3 grid((max_count + 255) / 256, nstreams); k_enc_histogram<<<grid, 256, 0, st>>>(tokens, streams, hist); CountLaunch();
+  if (!nstreams || !max_count) return; dim3 grid((max_count + 255) / 256, nstreams); Launch<k_enc_histogram>(grid, 256, 0, st, tokens, streams, hist);
 }
-void EncLaunchPrefix(const DEncFrame* d, const DEncStream* streams, uint32_t nstreams, const DEncCode* code, uint32_t bits_off, cudaStream_t st) { if (!nstreams) return; k_enc_prefix<<<(nstreams + 3) / 4, 128, 0, st>>>(d, streams, nstreams, code, bits_off); CountLaunch(); }
-void EncLaunchAns(const DEncFrame* d, const DEncStream* streams, uint32_t nstreams, const DEncCode* code, uint32_t bits_off, cudaStream_t st) { if (!nstreams) return; k_enc_ans<<<(nstreams + 3) / 4, 128, 0, st>>>(d, streams, nstreams, code, bits_off); CountLaunch(); }
+void EncLaunchPrefix(const DEncFrame* d, const DEncStream* streams, uint32_t nstreams, const DEncCode* code, uint32_t bits_off, cudaStream_t st) { if (!nstreams) return; Launch<k_enc_prefix>((nstreams + 3) / 4, 128, 0, st, d, streams, nstreams, code, bits_off); }
+void EncLaunchAns(const DEncFrame* d, const DEncStream* streams, uint32_t nstreams, const DEncCode* code, uint32_t bits_off, cudaStream_t st) { if (!nstreams) return; Launch<k_enc_ans>((nstreams + 3) / 4, 128, 0, st, d, streams, nstreams, code, bits_off); }
 
 }  // namespace jxlgpu

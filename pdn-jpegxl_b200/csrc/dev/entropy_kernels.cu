@@ -492,47 +492,39 @@ __global__ void k_modular_global(const __grid_constant__ DFrame f, uint64_t star
   SetError(f.err, md.rd.err);
 }
 
-static void EnsureSmemAttr() { static bool done[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (done[dev & 63]) return; done[dev & 63] = true;   // function attributes are per device
-  cudaFuncSetAttribute(k_lf_group_multi<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_lf_group_multi<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_ac_vardct_multi<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  cudaFuncSetAttribute(k_lf_group<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_lf_group<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_ac_vardct<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_mod_group<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_mod_group<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_modular_global, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-  cudaFuncSetAttribute(k_mod_lf_group<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); cudaFuncSetAttribute(k_mod_lf_group<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024); }
-void LaunchLfGroups(const DFrame* d, const DFrame& h, cudaStream_t st) { EnsureSmemAttr(); if (!h.num_lf_groups) return; const bool narrow = LfNarrow(h);
-  if (narrow) k_lf_group<true><<<h.num_lf_groups + h.lf_cta_offset, 32, h.lf_smem, st>>>(h); else k_lf_group<false><<<h.num_lf_groups + h.lf_cta_offset, 32, h.lf_smem, st>>>(h); }
+void LaunchLfGroups(const DFrame* d, const DFrame& h, cudaStream_t st) { if (!h.num_lf_groups) return; const bool narrow = LfNarrow(h);
+  if (narrow) Launch<k_lf_group<true>>(h.num_lf_groups + h.lf_cta_offset, 32, h.lf_smem, st, h); else Launch<k_lf_group<false>>(h.num_lf_groups + h.lf_cta_offset, 32, h.lf_smem, st, h); }
 // Bundle launches (JxlB200DecodeBatch): the images of `set` share one stream; all must be VarDCT, multi-section, of the same kind
 // (narrow Modular path for LF; single pass + shared-memory ANS tables for AC) — the caller checks with BundleCompatible*.
 bool LfNarrow(const DFrame& h) { return !h.uses_wp; }   // the image's bit depth (mod_wide) does not matter for LF groups: see LfGroupBody
 void LaunchLfGroupsMulti(const DFrameSet& set, bool narrow, cudaStream_t st) {
-  EnsureSmemAttr(); uint32_t smem = 0; for (uint32_t i = 0; i < set.n; i++) smem = std::max(smem, set.f[i].lf_smem); const unsigned grid = set.first[set.n] + set.cta_offset;
-  if (narrow) k_lf_group_multi<true><<<grid, 32, smem, st>>>(set); else k_lf_group_multi<false><<<grid, 32, smem, st>>>(set);
+  uint32_t smem = 0; for (uint32_t i = 0; i < set.n; i++) smem = std::max(smem, set.f[i].lf_smem); const unsigned grid = set.first[set.n] + set.cta_offset;
+  if (narrow) Launch<k_lf_group_multi<true>>(grid, 32, smem, st, set); else Launch<k_lf_group_multi<false>>(grid, 32, smem, st, set);
 }
 void LaunchAcGroupsMulti(const DFrameSet& set, int lanes, cudaStream_t st) {   // every frame: encoding 0, num_passes 1, ac_fast
-  EnsureSmemAttr(); uint32_t smem = 0; for (uint32_t i = 0; i < set.n; i++) smem = std::max(smem, set.f[i].ac_smem);
+  uint32_t smem = 0; for (uint32_t i = 0; i < set.n; i++) smem = std::max(smem, set.f[i].ac_smem);
   // Occupancy cap: a padded shared-memory request bounds the AC CTAs resident per SM, which leaves registers and shared memory for the
   // tile kernels (reconstruction, render) of images that are further along (they otherwise queue behind ~70 ms entropy CTAs).
   if (lanes >= 8) smem = std::max(smem, kAcBatchSmem);
-  k_ac_vardct_multi<true><<<set.first[set.n] + set.cta_offset, 32 * AcWarpsFor(lanes), smem, st>>>(set, lanes);
+  Launch<k_ac_vardct_multi<true>>(set.first[set.n] + set.cta_offset, 32 * AcWarpsFor(lanes), smem, st, set, lanes);
 }
 void LaunchLfDequant(const DFrame* d, const DFrame& h, bool smooth, cudaStream_t st) {
-  size_t plane = size_t(h.xb) * h.yb; unsigned blocks = unsigned((plane + 255) / 256); k_lf_dequant<<<blocks, 256, 0, st>>>(d); if (smooth) k_lf_smooth<<<blocks, 256, 0, st>>>(d);
+  size_t plane = size_t(h.xb) * h.yb; unsigned blocks = unsigned((plane + 255) / 256); Launch<k_lf_dequant>(blocks, 256, 0, st, d); if (smooth) Launch<k_lf_smooth>(blocks, 256, 0, st, d);
 }
-// Returns the number of kernels launched. `lanes`: sections per warp for the AC walk (power of two, 1..32).
+// `lanes`: sections per warp for the AC walk (power of two, 1..32).
 int AcCtas(const DFrame& h, int lanes) { const unsigned per_cta = unsigned(AcWarpsFor(lanes) * lanes); return int((h.num_groups + per_cta - 1) / per_cta); }
-int LaunchAcGroups(const DFrame* d, const DFrame& h, int pass, int lanes, cudaStream_t st) {
-  EnsureSmemAttr(); int n = 0;
+void LaunchAcGroups(const DFrame* d, const DFrame& h, int pass, int lanes, cudaStream_t st) {
   if (h.encoding == 0) {
     const unsigned nw = unsigned(AcWarpsFor(lanes)), per_cta = nw * unsigned(lanes), ctas = (h.num_groups + per_cta - 1) / per_cta;
-    if (h.ac_fast) k_ac_vardct<true><<<ctas + h.ac_cta_offset, 32 * nw, h.ac_smem, st>>>(h, pass, lanes); else k_ac_vardct<false><<<ctas + h.ac_cta_offset, 32 * nw, 0, st>>>(h, pass, lanes);
-    n++;
+    if (h.ac_fast) Launch<k_ac_vardct<true>>(ctas + h.ac_cta_offset, 32 * nw, h.ac_smem, st, h, pass, lanes); else Launch<k_ac_vardct<false>>(ctas + h.ac_cta_offset, 32 * nw, 0, st, h, pass, lanes);
   }
   if (h.num_mod_channels > h.first_group_channel) { const unsigned ctas = (h.num_groups + kModGroupsPerCta - 1) / kModGroupsPerCta;
-    if (!h.uses_wp && !h.mod_wide) k_mod_group<true><<<ctas, 32 * kModGroupsPerCta, h.lf_smem, st>>>(h, pass); else k_mod_group<false><<<ctas, 32 * kModGroupsPerCta, h.lf_smem, st>>>(h, pass); n++; }
-  return n;
+    if (!h.uses_wp && !h.mod_wide) Launch<k_mod_group<true>>(ctas, 32 * kModGroupsPerCta, h.lf_smem, st, h, pass); else Launch<k_mod_group<false>>(ctas, 32 * kModGroupsPerCta, h.lf_smem, st, h, pass); }
 }
 void LaunchModLfGroups(const DFrame& h, cudaStream_t st) {
-  EnsureSmemAttr(); if (!h.num_lf_groups) return; const unsigned ctas = (h.num_lf_groups + kModGroupsPerCta - 1) / kModGroupsPerCta;
-  if (!h.uses_wp && !h.mod_wide) k_mod_lf_group<true><<<ctas, 32 * kModGroupsPerCta, h.lf_smem, st>>>(h); else k_mod_lf_group<false><<<ctas, 32 * kModGroupsPerCta, h.lf_smem, st>>>(h);
-  CountLaunch();
+  if (!h.num_lf_groups) return; const unsigned ctas = (h.num_lf_groups + kModGroupsPerCta - 1) / kModGroupsPerCta;
+  if (!h.uses_wp && !h.mod_wide) Launch<k_mod_lf_group<true>>(ctas, 32 * kModGroupsPerCta, h.lf_smem, st, h); else Launch<k_mod_lf_group<false>>(ctas, 32 * kModGroupsPerCta, h.lf_smem, st, h);
 }
-void LaunchModularGlobal(const DFrame* d, const DFrame& h, uint64_t start_bitpos, uint32_t num_channels, cudaStream_t st) { EnsureSmemAttr(); k_modular_global<<<1, 32, h.lf_smem, st>>>(h, start_bitpos, num_channels); }
+void LaunchModularGlobal(const DFrame* d, const DFrame& h, uint64_t start_bitpos, uint32_t num_channels, cudaStream_t st) { Launch<k_modular_global>(1, 32, h.lf_smem, st, h, start_bitpos, num_channels); }
 
 }  // namespace jxlgpu

@@ -38,10 +38,9 @@ __global__ void __launch_bounds__(256) k_split_layers(const T* __restrict__ src,
 template <typename T>
 static void SplitT(const void* src, void* color, uint8_t* alpha, size_t npix, int format, bool has_alpha, cudaStream_t st) {
   const unsigned grid = unsigned((npix + 255) / 256); const T* s = static_cast<const T*>(src); T* c = static_cast<T*>(color);
-  if (format == 0) { if (has_alpha) k_split_layers<T, 1, 3, true><<<grid, 256, 0, st>>>(s, c, alpha, npix); else k_split_layers<T, 1, 3, false><<<grid, 256, 0, st>>>(s, c, alpha, npix); }
-  else if (format == 1) { if (has_alpha) k_split_layers<T, 3, 3, true><<<grid, 256, 0, st>>>(s, c, alpha, npix); else k_split_layers<T, 3, 3, false><<<grid, 256, 0, st>>>(s, c, alpha, npix); }
-  else { if (has_alpha) k_split_layers<T, 4, 4, true><<<grid, 256, 0, st>>>(s, c, alpha, npix); else k_split_layers<T, 4, 4, false><<<grid, 256, 0, st>>>(s, c, alpha, npix); }
-  CountLaunch();
+  if (format == 0) { if (has_alpha) Launch<k_split_layers<T, 1, 3, true>>(grid, 256, 0, st, s, c, alpha, npix); else Launch<k_split_layers<T, 1, 3, false>>(grid, 256, 0, st, s, c, alpha, npix); }
+  else if (format == 1) { if (has_alpha) Launch<k_split_layers<T, 3, 3, true>>(grid, 256, 0, st, s, c, alpha, npix); else Launch<k_split_layers<T, 3, 3, false>>(grid, 256, 0, st, s, c, alpha, npix); }
+  else { if (has_alpha) Launch<k_split_layers<T, 4, 4, true>>(grid, 256, 0, st, s, c, alpha, npix); else Launch<k_split_layers<T, 4, 4, false>>(grid, 256, 0, st, s, c, alpha, npix); }
 }
 
 // format: DecoderImageFormat (0 Gray, 1 Rgb, 2 Cmyk); sample_type: 0 u8, 1 u16, 2 f16, 3 f32

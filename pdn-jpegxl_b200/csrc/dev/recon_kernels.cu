@@ -12,17 +12,12 @@
 #include "kernels.h"
 #include "enc_frame.cuh"
 #include "idct_tables.inc"
-#include <atomic>
 #include <cuda_fp16.h>
 #include <cuda.h>
 #include <cmath>
 #include <stdexcept>
 
 namespace jxlgpu {
-
-static std::atomic<int> g_launches{0};
-int LaunchCount() { return g_launches.load(); }
-void CountLaunch(int n) { g_launches.fetch_add(n); }
 
 void FillDeviceTables(DTables* t) {
   for (int l = 0; l <= 8; l++) { int n = 1 << l; float* c = t->cosines + CosOff(l);
@@ -874,14 +869,12 @@ __global__ void k_output_int(const DFrame* fp) {
 }
 
 void LaunchReconstruct(const DFrame* d, const DFrame& h, cudaStream_t st) {
-  static bool attr[64] = {false}; const size_t smem16 = size_t(kReconWarps) * 3 * 16 * 20 * sizeof(float), smem32 = size_t(kReconWarps) * 3 * 32 * 36 * sizeof(float); int dev = 0; cudaGetDevice(&dev);
-  if (!attr[dev & 63]) { cudaFuncSetAttribute(k_reconstruct<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem32)); attr[dev & 63] = true; }
+  const size_t smem16 = size_t(kReconWarps) * 3 * 16 * 20 * sizeof(float), smem32 = size_t(kReconWarps) * 3 * 32 * 36 * sizeof(float);
   { const int items = int(h.num_groups) * 32; const int grid = std::min(items, 148 * 3); const size_t d8smem = size_t(2) * 3 * 32 * kD8Stride * sizeof(float);
-    static bool attr8[64] = {false}; if (!attr8[dev & 63]) { cudaFuncSetAttribute(k_reconstruct_dct8, cudaFuncAttributeMaxDynamicSharedMemorySize, int(d8smem)); attr8[dev & 63] = true; }
-    k_reconstruct_dct8<<<grid, 256, d8smem, st>>>(h, items); }
-  k_reconstruct<16><<<h.num_groups * 4, kReconWarps * 32, smem16, st>>>(d); k_reconstruct<32><<<h.num_groups * 4, kReconWarps * 32, smem32, st>>>(d); CountLaunch(3);
+    Launch<k_reconstruct_dct8>(grid, 256, d8smem, st, h, items); }
+  Launch<k_reconstruct<16>>(h.num_groups * 4, kReconWarps * 32, smem16, st, d); Launch<k_reconstruct<32>>(h.num_groups * 4, kReconWarps * 32, smem32, st, d);
 }
-void LaunchGaborishPlanes(const DFrame* d, const DFrame& h, const float* src, float* dst, cudaStream_t st) { dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8); k_gaborish<<<grid, blk, 0, st>>>(d, src, dst); CountLaunch(); }
+void LaunchGaborishPlanes(const DFrame* d, const DFrame& h, const float* src, float* dst, cudaStream_t st) { dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8); Launch<k_gaborish>(grid, blk, 0, st, d, src, dst); }
 // TMA descriptor of the three XYB planes as one rank-3 fp32 tensor {xpad, ypad, 3}, box {72, 38, 3}: one bulk copy fetches a whole
 // tile-plus-halo into the dense [plane][row][72] layout the filters read. The tensor starts at the planes' first allocated row (XybFirstRow),
 // so a band's map covers exactly its ypad rows. The driver entry point is looked up at run time (no libcuda link).
@@ -897,8 +890,6 @@ static bool EncodeXybTensorMap(const DFrame& h, CUtensorMap* out) {
 // k_render_wide_tma for the RGB8 or opaque BGRA32 output of a frame with gaborish + one EPF iteration
 static void LaunchRenderWide(const DFrame& h, bool bgra, cudaStream_t st) {
   const size_t smem = size_t(3) * kRfBuf * sizeof(float);
-  { static bool attr[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (!attr[dev & 63]) {
-      cudaFuncSetAttribute(k_render_wide_tma<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); cudaFuncSetAttribute(k_render_wide_tma<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); attr[dev & 63] = true; } }
   const int ntx = int(h.xsize + 63) / 64;
   // tile rows of the output rows: a band's out_y0 is a multiple of the group size, hence of the 32-row tile height
   const int t0 = h.band_on ? int(h.out_y0 / 32) * ntx : 0, t1 = int(((h.band_on ? h.out_y1 : h.ysize) + 31) / 32) * ntx;
@@ -906,14 +897,12 @@ static void LaunchRenderWide(const DFrame& h, bool bgra, cudaStream_t st) {
   // Tile (64, 32) is the first that can be interior: a frame smaller than 132 x 67 has no interior tile, issues no copy and gets the zero map.
   if (WideTileInterior(h, 64, 32) && !EncodeXybTensorMap(h, &tmap)) throw std::runtime_error("cuTensorMapEncodeTiled failed for the render kernel's XYB planes");
   const int grid = std::min(t1 - t0, 148 * 2);
-  if (bgra) k_render_wide_tma<1, true><<<grid, 256, smem, st>>>(h, tmap, ntx, t0, t1); else k_render_wide_tma<1, false><<<grid, 256, smem, st>>>(h, tmap, ntx, t0, t1);
+  if (bgra) Launch<k_render_wide_tma<1, true>>(grid, 256, smem, st, h, tmap, ntx, t0, t1); else Launch<k_render_wide_tma<1, false>>(grid, 256, smem, st, h, tmap, ntx, t0, t1);
 }
 // gaborish + EPF + colour in one pass over the frame (VarDCT frames with at least one restoration filter)
 template <int GAB, int EPF> static void LaunchRenderT(const DFrame& h, cudaStream_t st) {
   constexpr int H = GAB + (EPF == 3 ? 3 : 0) + (EPF >= 1 ? 2 : 0) + (EPF >= 2 ? 1 : 0), D = 32 + 2 * H; size_t smem = (size_t(EPF ? 8 : 6) * D * D + 64) * sizeof(float);
   constexpr bool kWide = GAB == 1 && EPF == 1;   // RGB8 output of these filters takes k_render_wide_tma, so k_render<1, 1, true> is never built
-  { static bool attr[64] = {false}; int dev = 0; cudaGetDevice(&dev); if (!attr[dev & 63]) { cudaFuncSetAttribute(k_render<GAB, EPF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-      if constexpr (!kWide) cudaFuncSetAttribute(k_render<GAB, EPF, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)); attr[dev & 63] = true; } }
   const DOutput& o = h.out;
   const bool rgb8 = !o.bgra && o.sample_type == 0 && o.num_channels == 3 && o.color_channels == 3 && o.alpha_plane < 0 && o.black_plane < 0 && !o.premultiplied && o.orientation == 1;
   dim3 grid((h.xsize + 31) / 32, (h.ysize + 31) / 32);
@@ -921,16 +910,15 @@ template <int GAB, int EPF> static void LaunchRenderT(const DFrame& h, cudaStrea
     // opaque BGRA32 surface of an 8-bit RGB image (JxlB200LoadImageBgra, BASELINE config 2): the same kernel with a 16-byte store per 4 pixels
     const bool fast_bgra = o.bgra && o.color_channels == 3 && o.alpha_plane < 0 && o.black_plane < 0 && !o.premultiplied && o.orientation == 1 && (reinterpret_cast<uintptr_t>(h.out_px) & 15) == 0;
     if (rgb8 || fast_bgra) LaunchRenderWide(h, fast_bgra, st);   // rows that are not 4-byte aligned fall back to byte stores inside the kernel
-    else k_render<1, 1, false><<<grid, 256, smem, st>>>(h);
+    else Launch<k_render<1, 1, false>>(grid, 256, smem, st, h);
   } else {
     const bool fast = rgb8 && (size_t(h.xsize) * 3) % 4 == 0 && (reinterpret_cast<uintptr_t>(h.out_px) & 3) == 0;
-    if (fast) k_render<GAB, EPF, true><<<grid, 256, smem, st>>>(h); else k_render<GAB, EPF, false><<<grid, 256, smem, st>>>(h);
+    if (fast) Launch<k_render<GAB, EPF, true>>(grid, 256, smem, st, h); else Launch<k_render<GAB, EPF, false>>(grid, 256, smem, st, h);
   }
-  CountLaunch();
 }
 bool LaunchFusedRender(const DFrame* d, const DFrame& h, cudaStream_t st) {
   if (h.encoding != 0 || (!h.lpf.gab && !h.lpf.epf_iters)) return false;
-  if (h.lpf.epf_iters) { size_t n = size_t(h.xb) * h.yb; k_inv_sigma<<<unsigned((n + 255) / 256), 256, 0, st>>>(d); CountLaunch(); }
+  if (h.lpf.epf_iters) { size_t n = size_t(h.xb) * h.yb; Launch<k_inv_sigma>(unsigned((n + 255) / 256), 256, 0, st, d); }
   const int g = h.lpf.gab ? 1 : 0;
   switch (g * 4 + int(h.lpf.epf_iters)) {
     case 1: LaunchRenderT<0, 1>(h, st); break; case 2: LaunchRenderT<0, 2>(h, st); break; case 3: LaunchRenderT<0, 3>(h, st); break;
@@ -968,20 +956,18 @@ __global__ void k_unsqueeze(const DFrame* fp, uint32_t op_index) {
 void LaunchInverseRct(const DFrame* d, const DFrame& h, const DModOp* ops, cudaStream_t st) {   // every inverse transform of the global Modular image, in execution order
   for (uint32_t i = 0; i < h.num_ops; i++) {
     const DModOp& op = ops[i]; const size_t n = size_t(op.w) * op.h;
-    if (op.kind == 2) { const unsigned threads = op.rct_type ? op.h : op.w; if (!threads) continue; k_unsqueeze<<<(threads + 63) / 64, 64, 0, st>>>(d, i); CountLaunch(); continue; }
+    if (op.kind == 2) { const unsigned threads = op.rct_type ? op.h : op.w; if (!threads) continue; Launch<k_unsqueeze>((threads + 63) / 64, 64, 0, st, d, i); continue; }
     if (!n) continue;
-    if (op.kind == 0) k_inverse_rct<<<unsigned((n + 255) / 256), 256, 0, st>>>(d, i);
-    else if (op.nb_deltas == 0) k_inverse_palette<<<dim3(unsigned((n + 255) / 256), op.num_c), 256, 0, st>>>(d, i);
-    else k_inverse_palette_delta<<<op.num_c, 32, 0, st>>>(d, i);
-    CountLaunch();
+    if (op.kind == 0) Launch<k_inverse_rct>(unsigned((n + 255) / 256), 256, 0, st, d, i);
+    else if (op.nb_deltas == 0) Launch<k_inverse_palette>(dim3(unsigned((n + 255) / 256), op.num_c), 256, 0, st, d, i);
+    else Launch<k_inverse_palette_delta>(op.num_c, 32, 0, st, d, i);
   }
 }
 void LaunchOutput(const DFrame* d, const DFrame& h, cudaStream_t st) {
   dim3 blk(32, 8), grid((h.xsize + 31) / 32, (h.ysize + 7) / 8);
   bool int_path = h.encoding == 1 && !h.color.xyb_encoded && h.out.exp_bits == 0 && h.out.black_plane < 0 && !h.out.premultiplied && (h.out.sample_type == 0 ? h.out.bits == 8 : (h.out.sample_type == 1 && h.out.bits == 16)) &&
                   (h.out.alpha_plane < 0 || (h.out.alpha_bits == h.out.bits && h.out.alpha_exp_bits == 0 && h.out_ch[h.out.alpha_plane].hshift == 0));
-  if (int_path) k_output_int<<<grid, blk, 0, st>>>(d); else k_output<<<grid, blk, 0, st>>>(h, h.xyb);
-  CountLaunch();
+  if (int_path) Launch<k_output_int>(grid, blk, 0, st, d); else Launch<k_output>(grid, blk, 0, st, h, h.xyb);
 }
 
 }  // namespace jxlgpu

@@ -18,8 +18,6 @@
 
 namespace jxlgpu {
 
-#define CUDA_OK(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) throw Error(std::string("CUDA: ") + cudaGetErrorString(e_) + " at " #expr); } while (0)
-
 namespace {
 
 // ---- fixed MA trees (same shape the decoder kernels walk; BFS layout as DecodeTree allocates it)
@@ -375,15 +373,18 @@ std::vector<BandSection> BandEncoder::Finish(const std::vector<uint64_t>& frame_
     DeviceEncCode dm, da; UploadEncCode(codes.mcode, &dm, st); if (!lossless) UploadEncCode(codes.acode, &da, st);
     const DEncFrame* de = d_e.as<DEncFrame>(); const DEncStream* d_m = d_streams.as<DEncStream>(); const DEncStream* d_a = d_m + m_streams.size();
     // the Modular streams (few and long: an LF group is one serial stream of 196 608 tokens) and the AC streams (many) are independent: two CUDA streams
-    cudaStream_t st2 = nullptr; cudaEvent_t ready = nullptr, done2 = nullptr; CUDA_OK(cudaStreamCreateWithFlags(&st2, cudaStreamNonBlocking)); cudaEventCreateWithFlags(&ready, cudaEventDisableTiming); cudaEventCreateWithFlags(&done2, cudaEventDisableTiming);
-    cudaEventRecord(ready, st); cudaStreamWaitEvent(st2, ready, 0);
+    // Released also when a call below throws, after the side stream's work has drained (its kernels use this encoder's buffers).
+    struct Side { cudaStream_t st2 = nullptr; cudaEvent_t ready = nullptr, done2 = nullptr;
+      ~Side() { if (st2) { cudaStreamSynchronize(st2); cudaStreamDestroy(st2); } if (ready) cudaEventDestroy(ready); if (done2) cudaEventDestroy(done2); } } side;
+    cudaStream_t& st2 = side.st2; CUDA_OK(cudaStreamCreateWithFlags(&st2, cudaStreamNonBlocking)); CUDA_OK(cudaEventCreateWithFlags(&side.ready, cudaEventDisableTiming)); CUDA_OK(cudaEventCreateWithFlags(&side.done2, cudaEventDisableTiming));
+    CUDA_OK(cudaEventRecord(side.ready, st)); CUDA_OK(cudaStreamWaitEvent(st2, side.ready, 0));
     const uint32_t nm = uint32_t(m_streams.size());
     if (codes.mcode.use_prefix) EncLaunchPrefix(de, d_m, nm, dm.desc.as<DEncCode>(), 0, st); else EncLaunchAns(de, d_m, nm, dm.desc.as<DEncCode>(), 0, st);
     if (!lossless) { if (codes.acode.use_prefix) EncLaunchPrefix(de, d_a, ng, da.desc.as<DEncCode>(), nm, st2); else EncLaunchAns(de, d_a, ng, da.desc.as<DEncCode>(), nm, st2); }
-    cudaEventRecord(done2, st2); cudaStreamWaitEvent(st, done2, 0);
+    CUDA_OK(cudaEventRecord(side.done2, st2)); CUDA_OK(cudaStreamWaitEvent(st, side.done2, 0));
     if (nm) CUDA_OK(cudaMemcpyAsync(bits_m.data(), e.stream_bits, size_t(nm) * 8, cudaMemcpyDeviceToHost, st));
     if (!lossless) CUDA_OK(cudaMemcpyAsync(bits_a.data(), e.stream_bits + nm, size_t(ng) * 8, cudaMemcpyDeviceToHost, st));
-    CUDA_OK(cudaStreamSynchronize(st)); cudaStreamDestroy(st2); cudaEventDestroy(ready); cudaEventDestroy(done2);
+    CUDA_OK(cudaStreamSynchronize(st));
     // dense copy of what was written: stream k (Modular streams first, then AC) lands at dense_off[k] of `bytes`
     const size_t ns = size_t(nm) + (lossless ? 0 : ng); dense_off.assign(ns + 1, 0);
     for (size_t k = 0; k < ns; k++) { const uint64_t b = k < nm ? bits_m[k] : bits_a[k - nm]; dense_off[k + 1] = dense_off[k] + ((b + 7) / 8 + 15) / 16 * 16; }

@@ -126,6 +126,7 @@ class BandEncoder {
   float device_ms = 0;
 
  private:
+  // device_ms only: its calls are not checked
   struct Timer { cudaEvent_t a, b; cudaStream_t s; float* acc; Timer(cudaStream_t st_, float* acc_) : s(st_), acc(acc_) { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a, s); }
     ~Timer() { cudaEventRecord(b, s); cudaEventSynchronize(b); float ms = 0; cudaEventElapsedTime(&ms, a, b); *acc += ms; cudaEventDestroy(a); cudaEventDestroy(b); } };
   EncodeRequest req; cudaStream_t st = nullptr; EncPlan plan; DEncFrame e; FrameHeader fb;   // fb: frame header of the band taken as an image of its own (group / LF-group layout)

@@ -226,6 +226,23 @@ def test_band_decode_stitches_to_the_full_frame(gpu, oracle, kw):
         gpu.decode_band(data, 0, rows + 1)
 
 
+def test_call_after_an_invalid_device_index_succeeds(gpu, oracle):
+    """A call given a device index that does not exist fails with its own status. The runtime keeps that failure in the thread's error
+    state; the next call on the same thread must not read it as a refused kernel launch of its own."""
+    img = oracle.synthetic_image(300, 200, seed=4)
+    data = oracle.encode(img, effort=7, distance=1.0)
+    ref = _decode_gpu(gpu, data).layer_data.color
+    bgra = np.concatenate([img[..., ::-1], np.full(img.shape[:2] + (1,), 255, np.uint8)], axis=2)
+    bad = 4096
+    with pytest.raises(gpu.FormatException) as e:
+        gpu.decode_band(data, 0, 1, device=bad)
+    assert e.value.status == "InvalidParameter"
+    assert np.array_equal(_decode_gpu(gpu, data).layer_data.color, ref)
+    with pytest.raises(gpu.FormatException, match="cudaSetDevice"):
+        gpu.BandEncoder(bgra, 200, 0, 0, 0, gpu.EncoderOptions(quality=90, effort=3), device=bad)
+    assert oracle.psnr(oracle.decode(gpu.encode_to_memory(bgra, gpu.EncoderOptions(quality=90, effort=3))).pixels, img) > 30.0
+
+
 def test_large_batch_uses_bundles_and_wide_warps(gpu, oracle):
     """64+ files with 32+ streams is the configuration bench.py measures: two images per entropy launch and 16 AC sections per warp.
     Every output must equal the single-image decode of the same file."""

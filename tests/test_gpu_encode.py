@@ -126,3 +126,20 @@ def test_band_encoder_rejects_misaligned_bands(gpu, oracle):
         gpu.BandEncoder(img[1000:2500], 2500, 1000, 0, 0, opts)           # a band must start on an LF-group row
     with pytest.raises(gpu.FormatException, match="halo"):
         gpu.BandEncoder(img[2048:2500], 2500, 2048, 0, 0, opts)           # and bring the 8 rows above it
+
+
+def test_refused_launch_fails_the_save(gpu):
+    """A 64 x 65 536 bitmap is taller than the grid of the colour / alpha scan can reach (grid.y <= 65 535): the runtime refuses that
+    launch before it reaches the device. SaveImage must fail with EncodeError rather than write the image as gray and opaque."""
+    w, h = 64, 65536
+    y, x = np.mgrid[0:h, 0:w]
+    bgra = np.stack([(x * 4) % 256, y % 256, (x + y) % 256, 255 - y % 7], axis=-1).astype(np.uint8)
+    out = io.BytesIO()
+    try:
+        gpu.JpegXLSave.Save(bgra, out, lossless=True)
+    except gpu.FormatException as e:
+        assert e.status == "EncodeError" and "CUDA" in str(e), (e.status, str(e))
+        return
+    image = gpu.DecoderImage()
+    gpu.JpegXLNative.LoadImage(out.getvalue(), image)
+    assert np.array_equal(image.layer_data.color, bgra[..., 2::-1]) and np.array_equal(image.layer_data.transparency, bgra[..., 3])
