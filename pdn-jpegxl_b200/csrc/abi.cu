@@ -16,7 +16,6 @@
 #include <thread>
 #include <map>
 #include <chrono>
-#include <cstdio>
 #include <mutex>
 #include <atomic>
 #include <stdexcept>
@@ -161,7 +160,7 @@ DecoderStatus JxlB200LoadImageBgra(const uint8_t* data, size_t dataSize, uint8_t
 DecoderStatus JxlB200LoadImageLayers(const uint8_t* data, size_t dataSize, uint8_t* color, size_t colorBytes, uint8_t* transparency, size_t transparencyBytes,
                                      int32_t* info6, ErrorInfo* errorInfo) {
   if (!data || !color) return DecoderStatus_NullParameter;
-  void* d_color = nullptr; void* d_alpha = nullptr; void* pool_c = nullptr; void* pool_a = nullptr; size_t bytes_c = 0, bytes_a = 0;   // cached device buffers (engine pool)
+  Buf d_color, d_alpha;
   const DecoderStatus rc = Guard<Decoding>(errorInfo, [&] {
     DecodeRequest req; req.data = data; req.size = dataSize; req.device_output = true; const DecodeResult res = WithTimes(DecodeOnGpu, req);
     const ParsedInfo& pi = res.info; const size_t npix = size_t(res.out_width) * res.out_height; const size_t bps = pi.sample_type == 0 ? 1 : pi.sample_type == 3 ? 4 : 2;
@@ -169,17 +168,16 @@ DecoderStatus JxlB200LoadImageLayers(const uint8_t* data, size_t dataSize, uint8
     const size_t dst_ch = pi.format == 2 ? 4 : 3, need_color = npix * dst_ch * bps, need_alpha = pi.has_alpha ? npix : 0;
     if (info6) { info6[0] = int32_t(res.out_width); info6[1] = int32_t(res.out_height); info6[2] = pi.format; info6[3] = pi.sample_type; info6[4] = pi.has_alpha ? 1 : 0; info6[5] = int32_t(dst_ch); }
     if (colorBytes < need_color || (pi.has_alpha && (!transparency || transparencyBytes < need_alpha))) { SetErrorMessage(errorInfo, "layer buffers too small"); return DecoderStatus_InvalidParameter; }
-    bytes_c = need_color ? need_color : 1; bytes_a = need_alpha ? need_alpha : 1; d_color = DeviceGet(bytes_c, &pool_c); d_alpha = DeviceGet(bytes_a, &pool_a);   // throw std::bad_alloc when the device is full
+    d_color.Alloc(need_color); d_alpha.Alloc(need_alpha);
     {
-      LaunchSplitLayers(res.pixels, d_color, static_cast<uint8_t*>(d_alpha), npix, pi.format, pi.sample_type, pi.has_alpha, 0);
-      cudaError_t e = cudaMemcpy(color, d_color, need_color, cudaMemcpyDeviceToHost);
-      if (e == cudaSuccess && need_alpha) e = cudaMemcpy(transparency, d_alpha, need_alpha, cudaMemcpyDeviceToHost);
+      LaunchSplitLayers(res.pixels, d_color.p, d_alpha.as<uint8_t>(), npix, pi.format, pi.sample_type, pi.has_alpha, 0);
+      cudaError_t e = cudaMemcpy(color, d_color.p, need_color, cudaMemcpyDeviceToHost);
+      if (e == cudaSuccess && need_alpha) e = cudaMemcpy(transparency, d_alpha.p, need_alpha, cudaMemcpyDeviceToHost);
       JXLG_CHECK(e == cudaSuccess, std::string("CUDA: ") + cudaGetErrorString(e));
     }
     return DecoderStatus_Ok;
   });
-  if (d_color || d_alpha) cudaDeviceSynchronize();   // the split kernel ran on the default stream; the copies above were synchronous
-  DevicePut(d_color, bytes_c, pool_c); DevicePut(d_alpha, bytes_a, pool_a);
+  if (d_color.p || d_alpha.p) cudaDeviceSynchronize();   // the split kernel ran on the default stream (the copies above were synchronous): drained before the buffers go back to the pool
   return rc;
 }
 
@@ -249,7 +247,7 @@ static int64_t PaceReserve(int dev, int64_t step_ns) {   // -> earliest start ti
 static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int nstreams, int batch_lanes, int bundle_size, size_t reserve_sets, ShardResult* out) {
   const int count = end - begin;
   if (count <= 0) return;
-  void* pin = nullptr; size_t pin_bytes = 0;
+  Buf pin;   // outlives the catch blocks below, which wait for the copies into it
   std::vector<cudaEvent_t> in_ready;
   struct EventGuard { std::vector<cudaEvent_t>& v; ~EventGuard() { for (cudaEvent_t e : v) if (e) cudaEventDestroy(e); } } in_ready_guard{in_ready};
   std::vector<uint8_t> finished(size_t(count), 0);
@@ -270,13 +268,13 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     // are queued up front on their own stream, one event per file, and a file is only waited for when its turn to be parsed comes.
     if (!a.hostInputs) {
       for (int i = 0; i < count; i++) in_off[i + 1] = in_off[i] + ((a.dataSizes[begin + i] + 63) & ~size_t(63));
-      pin_bytes = in_off[count] + 64; pin = PinnedGet(pin_bytes); in_ready.resize(size_t(count), nullptr);
+      pin.Alloc(in_off[count] + 64, true); in_ready.resize(size_t(count), nullptr);
       for (int i = 0; i < count; i++) {
-        CUDA_OK(cudaMemcpyAsync(static_cast<uint8_t*>(pin) + in_off[i], a.datas[begin + i], a.dataSizes[begin + i], cudaMemcpyDeviceToHost, copy_stream));
+        CUDA_OK(cudaMemcpyAsync(pin.as<uint8_t>() + in_off[i], a.datas[begin + i], a.dataSizes[begin + i], cudaMemcpyDeviceToHost, copy_stream));
         if (cudaEventCreateWithFlags(&in_ready[i], cudaEventDisableTiming) != cudaSuccess || cudaEventRecord(in_ready[i], copy_stream) != cudaSuccess)
           throw std::runtime_error("cannot read device inputs");
       }
-      host_in = static_cast<uint8_t*>(pin);
+      host_in = pin.as<uint8_t>();
     }
     // host outputs that are page-locked receive the pixels directly (no staging copy)
     std::vector<uint8_t> out_is_pinned(size_t(count), 0);
@@ -284,8 +282,6 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
       cudaPointerAttributes at;
       if (cudaPointerGetAttributes(&at, a.outputs[begin + i]) == cudaSuccess && at.type == cudaMemoryTypeHost) out_is_pinned[i] = 1; else cudaGetLastError();
     }
-    const bool trace = getenv("JXLB200_TRACE") != nullptr; double t_enq = 0, t_ret = 0, t_idle = 0, acc_t[5] = {0, 0, 0, 0, 0};
-    auto now = []() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     // Three-phase pipeline per image (LF entropy | AC entropy | reconstruction + render): a phase is enqueued only once the image's
     // stream has drained, so a kernel waiting on a 40 ms predecessor never sits at the head of a hardware queue shared with other
     // streams (there are 32 queues). Images travel in bundles of `bundle_size` that share a stream and whose LF / AC entropy kernels
@@ -293,14 +289,11 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     // q1/q2/q3 hold the bundles whose phase 1/2/3 is running.
     struct Bundle { std::vector<std::unique_ptr<InFlight>> items; cudaStream_t stream = nullptr; };
     std::deque<std::unique_ptr<Bundle>> q1, q2, q3; int next = 0, done = 0;
-    const double t_start = now(); double ph_first[3] = {-1, -1, -1}, ph_last[3] = {0, 0, 0};   // trace: when the first / last bundle left phase 1, 2, 3
-    auto stamp = [&](int ph) { const double t = now() - t_start; if (ph_first[ph] < 0) ph_first[ph] = t; ph_last[ph] = t; };
     auto finish = [&](InFlight& f, const DecodeResult& res) {   // records a decoded image
       DecoderStatus st = DecoderStatus_Ok;
       if (res.pixel_bytes > a.outputBytes[f.idx]) st = DecoderStatus_InvalidParameter;
       else if (!f.direct) memcpy(a.outputs[f.idx], res.pixels, res.pixel_bytes);
       record(f.idx, st, std::string());
-      if (trace) { const StageTimes& t = res.times; acc_t[0] += t.lf; acc_t[1] += t.ac; acc_t[2] += t.recon; acc_t[3] += t.filters + t.output; acc_t[4] += t.total; }
       f.job.reset(); done++;
     };
     // Runs one step of an image (enqueue, a later phase, finish). A failure is recorded for the image and drops it (false).
@@ -326,17 +319,17 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
         if (!idle(*q3[k])) { k++; continue; }
         Bundle& b = *q3[k];
         for (auto& f : b.items) step(*f, [&] { finish(*f, DecodeFinish(f->job)); });
-        free_streams.push_back(b.stream); q3.erase(q3.begin() + k); progressed = true; stamp(2);
+        free_streams.push_back(b.stream); q3.erase(q3.begin() + k); progressed = true;
       }
       for (size_t k = 0; k < std::min(kWindow, q2.size());) {
         if (!idle(*q2[k])) { k++; continue; }
-        std::unique_ptr<Bundle> b = std::move(q2[k]); q2.erase(q2.begin() + k); progressed = true; stamp(1);
+        std::unique_ptr<Bundle> b = std::move(q2[k]); q2.erase(q2.begin() + k); progressed = true;
         next_phase(*b, 3);
         if (b->items.empty()) free_streams.push_back(b->stream); else q3.push_back(std::move(b));
       }
       for (size_t k = 0; k < std::min(kWindow, q1.size());) {
         if (!idle(*q1[k])) { k++; continue; }
-        std::unique_ptr<Bundle> b = std::move(q1[k]); q1.erase(q1.begin() + k); progressed = true; stamp(0);
+        std::unique_ptr<Bundle> b = std::move(q1[k]); q1.erase(q1.begin() + k); progressed = true;
         next_phase(*b, 2);
         if (b->items.empty()) free_streams.push_back(b->stream); else q2.push_back(std::move(b));
       }
@@ -347,11 +340,10 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     int64_t pace_ns = 0, launch_at = 0;
     if (a.hostOutputs && a.count >= 64) pace_ns = int64_t(double(a.outputBytes[begin]) / kPaceGBps);
     while (done < count) {
-      double t0 = now(); bool progressed = advance(); t_ret += now() - t0;
+      const bool progressed = advance();
       if (pace_ns && next < count && !free_streams.empty() && launch_at == 0) launch_at = PaceReserve(cur_dev, pace_ns * std::min(bundle_size, count - next));
       if (next < count && !free_streams.empty() && (launch_at == 0 || SteadyNs() >= launch_at)) {
         launch_at = 0;
-        t0 = now();
         std::unique_ptr<Bundle> b(new Bundle); b->stream = free_streams.back(); free_streams.pop_back();
         for (int k = 0; k < bundle_size && next < count; k++) {
           const int li = next++, i = begin + li;
@@ -369,14 +361,9 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
           if (f->job) b->items.push_back(std::move(f));
         }
         if (bundle_size > 1) DecodeBundleLaunch(jobs_of(*b), 1);
-        t_enq += now() - t0;
         if (b->items.empty()) free_streams.push_back(b->stream); else q1.push_back(std::move(b));
-      } else if (!progressed) { t0 = now(); std::this_thread::sleep_for(std::chrono::microseconds(20)); t_idle += now() - t0; }
+      } else if (!progressed) std::this_thread::sleep_for(std::chrono::microseconds(20));
     }
-    if (trace) { DumpHostTrace(); if (slot == 0) DumpPoolStats(); }
-    if (trace && acc_t[4] > 0) fprintf(stderr, "[jxlb200] shard %d GPU ms/image under load (JXLB200_TRACE=2 events): lf %.2f ac %.2f recon %.2f render %.2f total %.2f\n", slot, acc_t[0] / count, acc_t[1] / count, acc_t[2] / count, acc_t[3] / count, acc_t[4] / count);
-    if (trace) fprintf(stderr, "[jxlb200] shard %d phase exits, ms after shard start (first .. last bundle): LF %.1f .. %.1f, AC %.1f .. %.1f, tiles %.1f .. %.1f\n", slot, ph_first[0], ph_last[0], ph_first[1], ph_last[1], ph_first[2], ph_last[2]);
-    if (trace) fprintf(stderr, "[jxlb200] shard %d, %d images: host parse + LF phase %.2f ms (%.2f ms/image), polling + later phases + retire %.2f ms, idle (GPU-bound) %.2f ms\n", slot, count, t_enq, t_enq / std::max(count, 1), t_ret, t_idle);
   } catch (const std::exception& e) {   // a failure of the shard itself (streams, input copies): every image not finished yet fails with it
     // Work may still be running on this shard's streams and writing into caller-owned buffers: wait for it before returning them.
     cudaDeviceSynchronize(); cudaGetLastError();
@@ -386,7 +373,6 @@ static void RunBatchShard(const BatchArgs& a, int slot, int begin, int end, int 
     cudaDeviceSynchronize(); cudaGetLastError();
     for (int i = begin; i < end; i++) if (!finished[size_t(i - begin)]) record(i, DecoderStatus_DecodeError, "batch decode failed");
   }
-  if (pin) PinnedPut(pin, pin_bytes);
 }
 
 // A batch in flight: owns copies of the caller's pointer arrays, the per-file statuses and the shard threads.

@@ -14,19 +14,11 @@
 #include <dlfcn.h>
 #include <map>
 #include <mutex>
-#include <chrono>
 #include <atomic>
 #include <memory>
 #include <functional>
-#include <cstdio>
 
 namespace jxlgpu {
-
-// host-side phase timers (JXLB200_TRACE=1): where the serial CPU time of an enqueue goes
-struct HostTrace { double t[8] = {0}; int n = 0; };
-static thread_local HostTrace g_trace;
-static inline double NowMs() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-void DumpHostTrace() { if (!g_trace.n) return; fprintf(stderr, "[jxlb200] host ms/image: headers %.2f setup %.2f lfglobal %.2f hfglobal %.2f alloc+upload %.2f blob %.2f launch %.2f\n", g_trace.t[0] / g_trace.n, g_trace.t[1] / g_trace.n, g_trace.t[2] / g_trace.n, g_trace.t[3] / g_trace.n, g_trace.t[4] / g_trace.n, g_trace.t[5] / g_trace.n, g_trace.t[6] / g_trace.n); g_trace = HostTrace(); }
 
 // ---------------------------------------------------------------- small utilities
 bool CudaAvailable(std::string* why) {
@@ -36,18 +28,20 @@ bool CudaAvailable(std::string* why) {
 }
 
 // Caching allocators (device + pinned host). cudaMalloc / cudaHostAlloc cost milliseconds; a decode is a handful of ms.
+// The shard threads of a batch take and return buffers concurrently: every access to the maps and the cached byte count holds mu_,
+// and no allocation runs under it.
 class Pool {
  public:
   explicit Pool(bool pinned) : pinned_(pinned) {}
   void* Get(size_t bytes) {
     size_t sz = Round(bytes); { std::lock_guard<std::mutex> lk(mu_); auto it = free_.find(sz); if (it != free_.end() && !it->second.empty()) { void* p = it->second.back(); it->second.pop_back(); cached_ -= sz; return p; } }
-    misses_++; { std::lock_guard<std::mutex> lk(mu_); miss_sizes_[sz]++; } void* p = nullptr; cudaError_t e = pinned_ ? cudaHostAlloc(&p, sz, cudaHostAllocDefault) : cudaMalloc(&p, sz);
-    if (e != cudaSuccess) { cudaGetLastError(); Trim(); e = pinned_ ? cudaHostAlloc(&p, sz, cudaHostAllocDefault) : cudaMalloc(&p, sz); }
+    void* p = nullptr; cudaError_t e = Malloc(&p, sz);
+    if (e != cudaSuccess) { cudaGetLastError(); Trim(); e = Malloc(&p, sz); }
     if (e != cudaSuccess) { cudaGetLastError(); throw std::bad_alloc(); }
     { std::lock_guard<std::mutex> lk(mu_); total_[sz]++; }
     return p;
   }
-  void Put(void* p, size_t bytes) { if (!p) return; size_t sz = Round(bytes); std::lock_guard<std::mutex> lk(mu_); free_[sz].push_back(p); cached_ += sz; if (cached_ > Limit()) TrimLocked(); }
+  void Put(void* p, size_t bytes) { if (!p) return; size_t sz = Round(bytes); std::lock_guard<std::mutex> lk(mu_); free_[sz].push_back(p); cached_ += sz; if (cached_ > LimitLocked()) TrimLocked(); }
   void Trim() { std::lock_guard<std::mutex> lk(mu_); TrimLocked(); }
   // Makes sure `count` buffers of this size class are cached (batch start: the first image tells the sizes; allocating them one
   // by one while the GPU is busy stalls the enqueue thread for milliseconds each and takes many batches to converge).
@@ -55,31 +49,26 @@ class Pool {
   // reservation runs, so counting only the free ones would allocate a fresh set on every batch.
   void Reserve(size_t bytes, size_t count) {
     const size_t sz = Round(bytes); size_t have; { std::lock_guard<std::mutex> lk(mu_); have = total_[sz]; }
-    for (; have < count; have++) { if (cached_ + sz > Limit()) return; void* p = nullptr; cudaError_t e = pinned_ ? cudaHostAlloc(&p, sz, cudaHostAllocDefault) : cudaMalloc(&p, sz); if (e != cudaSuccess) { cudaGetLastError(); return; }
+    for (; have < count; have++) {
+      { std::lock_guard<std::mutex> lk(mu_); if (cached_ + sz > LimitLocked()) return; }
+      void* p = nullptr; if (Malloc(&p, sz) != cudaSuccess) { cudaGetLastError(); return; }
       std::lock_guard<std::mutex> lk(mu_); free_[sz].push_back(p); cached_ += sz; total_[sz]++; }
   }
- private:
   // size classes: powers of two from 4 KiB up to 16 MiB (files of different sizes then share every small bucket, so the first image of
   // a batch can reserve for all of them), eighths of a power of two above (the big planes, whose size depends on the dimensions only)
-  public: static size_t Round(size_t b) { if (b <= 4096) return 4096; int k = 63 - __builtin_clzll(b - 1); if (b <= (size_t(16) << 20)) return size_t(2) << k; k = 63 - __builtin_clzll(b); size_t g = size_t(1) << (k - 3); return (b + g - 1) / g * g; }
-  private: void TrimLocked() { trims_++; for (auto& kv : free_) { for (void* p : kv.second) { if (pinned_) cudaFreeHost(p); else cudaFree(p); } total_[kv.first] -= std::min(total_[kv.first], kv.second.size()); } free_.clear(); cached_ = 0; }
-  size_t Limit() { if (!limit_) { size_t fr = 0, tot = 0; if (pinned_ || cudaMemGetInfo(&fr, &tot) != cudaSuccess) { cudaGetLastError(); limit_ = size_t(32) << 30; } else limit_ = tot / 4 * 3; } return limit_; }
-  public: size_t misses_ = 0, trims_ = 0; std::map<size_t, size_t> miss_sizes_; std::string MissReport() { std::lock_guard<std::mutex> lk(mu_); std::string r; for (auto& kv : miss_sizes_) { r += " " + std::to_string(kv.first >> 10) + "K:" + std::to_string(kv.second) + "(free " + std::to_string(free_[kv.first].size()) + ")"; } return r; } size_t Cached() const { return cached_; }
+  static size_t Round(size_t b) { if (b <= 4096) return 4096; int k = 63 - __builtin_clzll(b - 1); if (b <= (size_t(16) << 20)) return size_t(2) << k; k = 63 - __builtin_clzll(b); size_t g = size_t(1) << (k - 3); return (b + g - 1) / g * g; }
  private:
-  bool pinned_; std::mutex mu_; std::map<size_t, std::vector<void*>> free_; std::map<size_t, size_t> total_; size_t cached_ = 0; size_t limit_ = 0;
+  size_t LimitLocked() { if (!limit_) { size_t fr = 0, tot = 0; if (pinned_ || cudaMemGetInfo(&fr, &tot) != cudaSuccess) { cudaGetLastError(); limit_ = size_t(32) << 30; } else limit_ = tot / 4 * 3; } return limit_; }
+  cudaError_t Malloc(void** p, size_t sz) { return pinned_ ? cudaHostAlloc(p, sz, cudaHostAllocDefault) : cudaMalloc(p, sz); }
+  void TrimLocked() { for (auto& kv : free_) { for (void* p : kv.second) { if (pinned_) cudaFreeHost(p); else cudaFree(p); } total_[kv.first] -= std::min(total_[kv.first], kv.second.size()); } free_.clear(); cached_ = 0; }
+  bool pinned_; std::mutex mu_; std::map<size_t, std::vector<void*>> free_; std::map<size_t, size_t> total_; size_t cached_ = 0, limit_ = 0;
 };
 static Pool& DevPool() {   // one pool per device: a cached buffer must never cross devices
   static std::mutex mu; static std::map<int, std::unique_ptr<Pool>> pools; int dev = 0; cudaGetDevice(&dev); std::lock_guard<std::mutex> lk(mu); auto& p = pools[dev]; if (!p) p.reset(new Pool(false)); return *p; }
 static Pool& HostPool() { static Pool p(true); return p; }
 void TrimPools() { DevPool().Trim(); HostPool().Trim(); }
-void DumpPoolStats() { Pool& d = DevPool(); Pool& h = HostPool(); fprintf(stderr, "[jxlb200] pools: device misses %zu trims %zu cached %.1f GB; pinned misses %zu trims %zu cached %.2f GB\n", d.misses_, d.trims_, d.Cached() / 1e9, h.misses_, h.trims_, h.Cached() / 1e9); fprintf(stderr, "[jxlb200] device miss sizes:%s\n", d.MissReport().c_str()); }
-void* PinnedGet(size_t bytes) { return HostPool().Get(bytes ? bytes : 1); }
-void* DeviceGet(size_t bytes, void** pool_token) { Pool& p = DevPool(); *pool_token = &p; return p.Get(bytes ? bytes : 1); }   // the current device's pool
-void DevicePut(void* ptr, size_t bytes, void* pool_token) { if (ptr && pool_token) static_cast<Pool*>(pool_token)->Put(ptr, bytes ? bytes : 1); }
-void PinnedPut(void* p, size_t bytes) { HostPool().Put(p, bytes ? bytes : 1); }
-
-struct DevBuf { void* p = nullptr; size_t n = 0; bool host = false; Pool* pool = nullptr; void Alloc(size_t bytes, bool pinned = false) { Free(); host = pinned; n = bytes ? bytes : 1; pool = pinned ? &HostPool() : &DevPool(); p = pool->Get(n); } void Free() { if (p) pool->Put(p, n); p = nullptr; n = 0; } ~DevBuf() { Free(); } DevBuf() {} DevBuf(const DevBuf&) = delete; DevBuf& operator=(const DevBuf&) = delete;
-  void Swap(DevBuf& o) { std::swap(p, o.p); std::swap(n, o.n); std::swap(host, o.host); std::swap(pool, o.pool); } template <class T> T* as() const { return static_cast<T*>(p); } };
+void Buf::Alloc(size_t bytes, bool pinned) { Free(); n = bytes ? bytes : 1; pool = pinned ? &HostPool() : &DevPool(); p = pool->Get(n); }
+void Buf::Free() { if (p) pool->Put(p, n); p = nullptr; n = 0; }
 
 static const DTables* DeviceTables() {
   static std::mutex mu; static std::map<int, DTables*> per_dev; std::lock_guard<std::mutex> lk(mu); int dev = 0; CUDA_OK(cudaGetDevice(&dev));
@@ -223,7 +212,7 @@ LayeredStill::LayeredStill() : Error("layered (multi-frame) files are decoded by
 class DecodeJob {
  public:
   Headers hd; ParsedInfo info; FrameHeader fh; Toc toc; DFrame h; Blob blob; bool bgra = false, device_output = false, layer = false; DLocalTree global_local = DLocalTree(); std::vector<DModOp> ops_host; bool mod_has_lf_level = false; uint64_t mod_total_ints = 0;   /* int32 samples of all Modular planes: coded channels + the outputs of palette expansions */
-  DevBuf d_frame, d_blob, d_comp, d_lfq, d_lf, d_lf_tmp, d_acs, d_qf, d_sharp, d_lfidx, d_ytox, d_ytob, d_hfmeta, d_coeffs, d_xyb, d_xyb_tmp, d_sigma, d_mod, d_wp, d_out, d_err, h_out, h_err, h_comp, h_blob, h_misc, d_gother, d_nz, d_acend, d_lz, d_gpal, d_layer_out, h_layer_out;   /* *_layer_out: the finished canvas of a layered file (owned by the job of the frame that is shown) */
+  Buf d_frame, d_blob, d_comp, d_lfq, d_lf, d_lf_tmp, d_acs, d_qf, d_sharp, d_lfidx, d_ytox, d_ytob, d_hfmeta, d_coeffs, d_xyb, d_xyb_tmp, d_sigma, d_mod, d_wp, d_out, d_err, h_out, h_err, h_comp, h_blob, h_misc, d_gother, d_nz, d_acend, d_lz, d_gpal, d_layer_out, h_layer_out;   /* *_layer_out: the finished canvas of a layered file (owned by the job of the frame that is shown) */
   std::function<void()> ac_budget; int ac_lanes = 1; bool phased = false; size_t coeffs_bytes = 0, xyb_row_shift = 0;
   bool defer_entropy = false, lf_pending = false, ac_pending = false;   // bundle mode: the LF / AC entropy launch is left to DecodeBundleLaunch*
   cudaStream_t stream = nullptr; cudaEvent_t ev[8] = {nullptr}; bool timed = false; size_t out_bytes = 0; size_t comp_size = 0; const uint8_t* frame_ptr = nullptr; size_t frame_off = 0;
@@ -233,10 +222,10 @@ class DecodeJob {
 
   void Setup(const DecodeRequest& req);
   void RunLf(const DecodeRequest& req); void RunAc(); void RunRender();
-  void ReservePools(size_t count) { DevBuf* all[] = {&d_frame, &d_blob, &d_comp, &d_lfq, &d_lf, &d_lf_tmp, &d_acs, &d_qf, &d_sharp, &d_lfidx, &d_ytox, &d_ytob, &d_hfmeta, &d_coeffs, &d_xyb, &d_xyb_tmp, &d_sigma, &d_mod, &d_wp, &d_out, &d_err, &h_out, &h_err, &h_comp, &h_blob, &h_misc, &d_gother, &d_nz, &d_acend};
+  void ReservePools(size_t count) { Buf* all[] = {&d_frame, &d_blob, &d_comp, &d_lfq, &d_lf, &d_lf_tmp, &d_acs, &d_qf, &d_sharp, &d_lfidx, &d_ytox, &d_ytob, &d_hfmeta, &d_coeffs, &d_xyb, &d_xyb_tmp, &d_sigma, &d_mod, &d_wp, &d_out, &d_err, &h_out, &h_err, &h_comp, &h_blob, &h_misc, &d_gother, &d_nz, &d_acend};
     // several buffers of a job share a size class (the small ones all round to 4 KiB): reserve count x multiplicity per class
     std::map<std::pair<Pool*, size_t>, size_t> mult;
-    for (DevBuf* b : all) if (b->p && b->pool) mult[std::make_pair(b->pool, Pool::Round(b->n))]++;
+    for (Buf* b : all) if (b->p && b->pool) mult[std::make_pair(b->pool, Pool::Round(b->n))]++;
     for (auto& kv : mult) kv.first.first->Reserve(kv.first.second, (count + 1) * kv.second); }
   void Run(const DecodeRequest& req) { RunLf(req); RunAc(); RunRender(); }
   void ParseLfGlobal(BitReader& br); uint32_t AddTree(const Tree& t, uint32_t* uses_wp); DLocalTree ParseLocalTree(BitReader& br, size_t pixels);
@@ -527,11 +516,9 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
   const ByteSpan& cs = hd.ci.codestream; const bool vardct = h.encoding == 0; const size_t nsec = toc.size.size(); const bool single = nsec == 1;
   const size_t nlog = size_t(h.num_passes) * h.num_groups + h.num_lf_groups + 2;
   // host parse: LfGlobal (+ HfGlobal when it has its own section)
-  double tt = NowMs();
-  BitReader lfg(cs.data() + frame_off + toc.offset[0], toc.size[0]); ParseLfGlobal(lfg); JXLG_CHECK(!lfg.overrun, "LfGlobal truncated"); g_trace.t[2] += NowMs() - tt; tt = NowMs();
+  BitReader lfg(cs.data() + frame_off + toc.offset[0], toc.size[0]); ParseLfGlobal(lfg); JXLG_CHECK(!lfg.overrun, "LfGlobal truncated");
   uint64_t base_bits = uint64_t(frame_off) * 8; uint64_t after_lfglobal = (uint64_t(frame_off) + toc.offset[0]) * 8 + lfg.pos;
   if (!single && vardct) { BitReader hb(cs.data() + frame_off + toc.offset[1 + h.num_lf_groups], toc.size[1 + h.num_lf_groups]); ParseHfGlobal(hb); JXLG_CHECK(!hb.overrun, "HfGlobal truncated"); }
-  g_trace.t[3] += NowMs() - tt; tt = NowMs();
   {  // shared-memory budgets for the staged tables (host knows the exact sizes)
     auto code_bytes = [](const DCode& c) { return ((c.num_clusters * 4 + 15) & ~15u) + ((c.num_ctx + 15) & ~15u) + (c.use_prefix ? 0u : (((c.num_clusters << c.log_alpha) * 8 + 15) & ~15u)); };
     uint32_t modb = has_tree ? code_bytes(h.mod_code) + ((h.tree_size * 16 + 15) & ~15u) : 0;
@@ -543,7 +530,6 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
       for (uint32_t p = 0; p < h.num_passes; p++) prefix |= h.ac_code[p].lz77 != 0;   // LZ77 streams take the generic reader too
       h.ac_smem = acb + 64; h.ac_fast = (!prefix && h.ac_smem <= 96 * 1024) ? 1 : 0; if (!h.ac_fast) h.ac_smem = 0; };
     if (vardct && !single) ac_budget();
-    { static const bool tr = getenv("JXLB200_TRACE") != nullptr; static std::atomic<int> shown{0}; if (tr && shown.fetch_add(1) < 2) fprintf(stderr, "[jxlb200] table staging: lf_smem %u B, ac_smem %u B (ac_fast %u), AC clusters %u, log_alpha %u\n", h.lf_smem, h.ac_smem, h.ac_fast, h.ac_code[0].num_clusters, h.ac_code[0].log_alpha); }
   }
   // ---- sub-bitstreams with their own MA tree. Group sections of Modular frames start with their Modular header, so the host can parse the tree and
   // the code that follow it (VarDCT frames keep their group-local Modular data behind the AC coefficients, where only the device knows the position).
@@ -572,9 +558,9 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
   std::vector<uint64_t> sec(2 * nlog + 2, 0);
   for (size_t i = 0; i < nlog; i++) { size_t t = single ? 0 : i; sec[i] = base_bits + uint64_t(toc.offset[t]) * 8; sec[nlog + i] = base_bits + uint64_t(toc.offset[t] + toc.size[t]) * 8; }
   h.sec_off = blob.Add(sec.data(), sec.size() * 8);
-  AllocateAndUpload(req); g_trace.t[4] += NowMs() - tt; tt = NowMs();
+  AllocateAndUpload(req);
   auto upload_blob = [&]() { blob.b.resize((blob.b.size() + 31) / 16 * 16, 0); if (d_blob.n < blob.b.size() + 16) d_blob.Alloc(std::max<size_t>(blob.b.size() * 2, 1 << 16)); h.blob = d_blob.as<uint8_t>(); h_blob.Alloc(blob.b.size(), true); memcpy(h_blob.p, blob.b.data(), blob.b.size()); CUDA_OK(cudaMemcpyAsync(d_blob.p, h_blob.p, blob.b.size(), cudaMemcpyHostToDevice, stream)); UploadFrame(); };
-  upload_blob(); g_trace.t[5] += NowMs() - tt; tt = NowMs();
+  upload_blob();
   const DFrame* d = d_frame.as<DFrame>();
   if (timed) cudaEventRecord(ev[0], stream);
   // global Modular stream
@@ -590,24 +576,22 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
     BitReader hb(cs.data(), cs.size()); hb.pos = size_t(pos[1]); ParseHfGlobal(hb); JXLG_CHECK(!hb.overrun, "HfGlobal truncated"); uint64_t after = hb.pos; ac_budget();
     upload_blob(); { uint64_t* slot = reinterpret_cast<uint64_t*>(h_misc.as<uint8_t>() + 2 * sizeof(DFrame)) + 1; slot[0] = after; CUDA_OK(cudaMemcpyAsync(h.end_bitpos + 2, slot, 8, cudaMemcpyHostToDevice, stream)); }
   }
-  g_trace.t[6] += NowMs() - tt;
 }
 
 // Phase 2: LF dequantisation (+ adaptive smoothing) and the AC / group-Modular entropy kernels.
 void DecodeJob::RunAc() {
-  const bool vardct = h.encoding == 0; const DFrame* d = d_frame.as<DFrame>(); double tt = NowMs();
+  const bool vardct = h.encoding == 0; const DFrame* d = d_frame.as<DFrame>();
   if (timed) cudaEventRecord(ev[1], stream);
   if (vardct) LaunchLfDequant(d, h, h.lf_src == h.lf_tmp, stream);
   if (vardct) CUDA_OK(cudaMemsetAsync(d_coeffs.p, 0, coeffs_bytes, stream));
   if (defer_entropy && vardct && h.num_passes == 1 && h.ac_fast && !(h.num_mod_channels > h.first_group_channel)) ac_pending = true;
   else for (uint32_t p = 0; p < h.num_passes; p++) LaunchAcGroups(d, h, int(p), ac_lanes, stream);
   if (timed) cudaEventRecord(ev[2], stream);
-  g_trace.t[6] += NowMs() - tt;
 }
 
 // Phase 3: dequant + IDCT, restoration filters, colour transform, pack, and the copy back to the host.
 void DecodeJob::RunRender() {
-  const bool vardct = h.encoding == 0; const DFrame* d = d_frame.as<DFrame>(); double tt = NowMs();
+  const bool vardct = h.encoding == 0; const DFrame* d = d_frame.as<DFrame>();
   if (vardct && !d_xyb_tmp.p) {   // phased job: the LF phase has drained, its flag word is already in host memory
     const bool big_blocks = h_err.as<volatile uint32_t>()[12] != 0;   // written by k_lf_group straight into this page-locked word
     if (big_blocks) { d_xyb_tmp.Alloc(size_t(h.xpad) * h.ypad * 3 * 4); h.xyb_tmp = d_xyb_tmp.as<float>() - xyb_row_shift; UploadFrame(); }
@@ -622,7 +606,6 @@ void DecodeJob::RunRender() {
   if (!device_output) CUDA_OK(cudaMemcpyAsync(ext_out_pinned ? ext_out_pinned : h_out.as<uint8_t>(), h.out_px, out_bytes, cudaMemcpyDeviceToHost, stream));
   CUDA_OK(cudaMemcpyAsync(h_err.p, d_err.p, 64, cudaMemcpyDeviceToHost, stream));
   if (timed) cudaEventRecord(ev[6], stream);
-  g_trace.t[6] += NowMs() - tt; g_trace.n++;
 }
 
 // Position of the first frame after an optional preview frame, and whether that frame is a plain single-frame image.
@@ -639,18 +622,17 @@ static bool FirstFrameIsPlain(const Headers& hd, size_t* first_pos) {
 static std::shared_ptr<DecodeJob> StartJob(const DecodeRequest& req, cudaStream_t stream, bool timed, size_t* layered_pos = nullptr) {
   std::shared_ptr<DecodeJob> job = std::make_shared<DecodeJob>(); job->stream = stream;
   if (timed) { job->timed = true; for (int i = 0; i < 7; i++) cudaEventCreate(&job->ev[i]); }   // stage timing only: ev calls are not checked
-  double t0 = NowMs(); ParseHeadersInto(req.data, req.size, &job->hd, &job->info); g_trace.t[0] += NowMs() - t0;
+  ParseHeadersInto(req.data, req.size, &job->hd, &job->info);
   if (layered_pos && !FirstFrameIsPlain(job->hd, layered_pos)) return job;
   if (layered_pos) *layered_pos = 0;
-  t0 = NowMs(); job->Setup(req); g_trace.t[1] += NowMs() - t0;
+  job->Setup(req);
   return job;
 }
 
 std::shared_ptr<DecodeJob> DecodeEnqueue(const DecodeRequest& req, cudaStream_t stream, bool lf_phase_only, bool defer_entropy) {
   if (!req.data) throw StatusError(DecoderStatus_NullParameter);
   std::string why; JXLG_CHECK(CudaAvailable(&why), why);
-  static const bool batch_times = getenv("JXLB200_TRACE") != nullptr && atoi(getenv("JXLB200_TRACE")) >= 2;
-  std::shared_ptr<DecodeJob> job = StartJob(req, stream, batch_times);
+  std::shared_ptr<DecodeJob> job = StartJob(req, stream, false);
   job->phased = lf_phase_only; job->defer_entropy = defer_entropy && lf_phase_only;
   if (lf_phase_only) job->RunLf(req); else job->Run(req);
   return job;
@@ -693,7 +675,6 @@ DecodeResult DecodeFinish(const std::shared_ptr<DecodeJob>& job) {
   cudaError_t e = cudaStreamSynchronize(job->stream);
   if (e != cudaSuccess) throw Error(std::string("CUDA: ") + cudaGetErrorString(e));
   uint32_t de = *job->h_err.as<uint32_t>();
-  { static const bool dbg = getenv("JXLB200_TRACE") != nullptr; if (dbg && job->timed) fprintf(stderr, "[jxlb200] LF group 0: LF coefficients %u kcycles, HF metadata %u kcycles\n", job->h_err.as<uint32_t>()[13], job->h_err.as<uint32_t>()[14]); }
   JXLG_CHECK(de == 0, DevErrorText(de));
   DecodeResult r;
   r.info = job->info; r.pixels = job->device_output ? job->h.out_px : (job->ext_out_pinned ? job->ext_out_pinned : job->h_out.as<uint8_t>()); r.pixel_bytes = job->out_bytes; r.out_width = job->h.out.out_w; r.out_height = job->h.band_on ? job->h.out_y1 - job->h.out_y0 : job->h.out.out_h; r.job = job;
@@ -709,7 +690,7 @@ DecodeResult DecodeFinish(const std::shared_ptr<DecodeJob>& job) {
 // patches (rejected) and are skipped.
 // `head` holds the file's headers.
 static DecodeResult DecodeLayered(const DecodeRequest& req, const DecodeJob& head, size_t pos, cudaStream_t st) {
-  struct SlotBuf { DevBuf buf; bool valid = false; }; SlotBuf slots[4]; ParsedInfo info = head.info;
+  struct SlotBuf { Buf buf; bool valid = false; }; SlotBuf slots[4]; ParsedInfo info = head.info;
   const ImageMetadata& m = head.hd.meta; const ByteSpan& cs = head.hd.ci.codestream;
   for (int guard = 0; guard < 4096; guard++) {
     JXLG_CHECK(pos < cs.size(), "JxlDecoderProcessInput needs more input, but it already received the entire image.");
@@ -725,7 +706,7 @@ static DecodeResult DecodeLayered(const DecodeRequest& req, const DecodeJob& hea
     DecodeRequest r = req; r.layer = true; r.layer_pos = pos; r.device_output = true; r.out_device = nullptr; r.out_pinned = nullptr; r.bgra = false; r.band_begin = r.band_end = 0; r.device_input = nullptr;
     std::shared_ptr<DecodeJob> job = StartJob(r, st, false); job->Run(r); const DecodeResult fr = DecodeFinish(job);
     const int W = int(m.xsize), H = int(m.ysize), C = info.num_channels, cc = int(m.num_color_channels()); const size_t canvas_bytes = size_t(W) * H * C * sizeof(float);
-    DevBuf canvas; canvas.Alloc(canvas_bytes);
+    Buf canvas; canvas.Alloc(canvas_bytes);
     if (!ref_only && slots[cb.source].valid) CUDA_OK(cudaMemcpyAsync(canvas.p, slots[cb.source].buf.p, canvas_bytes, cudaMemcpyDeviceToDevice, st)); else CUDA_OK(cudaMemsetAsync(canvas.p, 0, canvas_bytes, st));
     const bool premul = alpha >= 0 && m.ec[alpha].alpha_associated;
     LaunchBlendLayer(canvas.as<float>(), reinterpret_cast<const float*>(fr.pixels), W, H, int(fh.xsize), int(fh.ysize), ref_only ? 0 : fh.x0, ref_only ? 0 : fh.y0, C, cc,

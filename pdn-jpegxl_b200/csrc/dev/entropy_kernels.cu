@@ -85,7 +85,7 @@ __device__ __forceinline__ void LfGroupBody(const DFrame& f, const int g) {
   const uint64_t* sec = SecBitPos(f); const uint32_t nsec = f.num_passes * f.num_groups + f.num_lf_groups + 2; const bool single = (f.num_groups == 1 && f.num_passes == 1);
   const uint64_t end = single ? sec[nsec] : sec[nsec + 1 + g];
   int32_t* wp = f.wp_scratch + size_t(g) * WPScratchInts(kMaxWpWidth);
-  const size_t plane = size_t(f.xb) * f.yb; const int lf_sid = 1 + g; long long dbg_t0 = 0;
+  const size_t plane = size_t(f.xb) * f.yb; const int lf_sid = 1 + g;
   // ---- part A (lane 0): section start, LF-coefficient sub-bitstream header
   if (lane == 0) {
     sh_ok = 0; sh_nb = 0;
@@ -95,7 +95,7 @@ __device__ __forceinline__ void LfGroupBody(const DFrame& f, const int g) {
     f.hfmeta_scratch[size_t(f.num_lf_groups) * kHfMetaScratchInts + g] = int32_t(extra_prec);
     const bool ok = ReadGroupHeaderDev(md, f);
     if (ok) md.rd.Init(md.cv);
-    sh_hdr_ok = ok ? 1 : 0; dbg_t0 = clock64();
+    sh_hdr_ok = ok ? 1 : 0;
   }
   __syncwarp();
   // ---- part B (whole warp): the three LF-coefficient channels; stream channel order is Y, X, B (A.8 LfGroup)
@@ -114,11 +114,7 @@ __device__ __forceinline__ void LfGroupBody(const DFrame& f, const int g) {
   // ---- part C (lane 0): HF metadata
   if (lane == 0) {
     bool ok = sh_hdr_ok != 0;
-    if (ok) {
-      if (!md.rd.FinalOk(md.cv)) md.rd.err = md.rd.err ? md.rd.err : kErrAnsFinal;
-      if (g == 0) f.err[13] = uint32_t((clock64() - dbg_t0) >> 10);   // debug: kilo-cycles spent on the LF coefficients of LF group 0
-    }
-    const long long dbg_t1 = clock64();
+    if (ok && !md.rd.FinalOk(md.cv)) md.rd.err = md.rd.err ? md.rd.err : kErrAnsFinal;
     // (Modular LF-group channels — extra channels with dim_shift >= 3 — are rejected on the host.)
     if (ok && !md.rd.err) {
       uint32_t nb = md.rd.br.Read(CeilLog2Dev(uint32_t(w * h))) + 1; sh_nb = nb;
@@ -131,7 +127,6 @@ __device__ __forceinline__ void LfGroupBody(const DFrame& f, const int g) {
         if (!md.rd.FinalOk(md.cv)) md.rd.err = md.rd.err ? md.rd.err : kErrAnsFinal;
       }
     }
-    if (g == 0) f.err[14] = uint32_t((clock64() - dbg_t1) >> 10);   // debug: kilo-cycles spent on its HF metadata
     uint64_t pos = md.rd.br.BitPos(); if (pos > end) md.rd.err = md.rd.err ? md.rd.err : kErrOverrun;
     if (single) f.end_bitpos[1] = pos;
     SetError(f.err, md.rd.err); sh_ok = (ok && !md.rd.err) ? 1 : 0;
@@ -198,14 +193,17 @@ __device__ __forceinline__ void LfGroupBody(const DFrame& f, const int g) {
 
 // The first-wave CTA->SM mapping is deterministic, so concurrent images would stack their few LF CTAs on the same SMs:
 // each launch prepends `lf_cta_offset` empty CTAs to land on different SMs.
+// Register budget: one warp per CTA, at least 12 CTAs per SM (a 256-image batch of 12 MP files keeps about 7 LF CTAs on each SM), which
+// allows up to 168 registers. Left to ptxas's default target, the narrow variants get 96 and spill around the decode calls.
+constexpr int kLfMinCtasPerSm = 12;
 template <bool kNarrow>
-__global__ void __launch_bounds__(32) k_lf_group(const __grid_constant__ DFrame f) {
+__global__ void __launch_bounds__(32, kLfMinCtasPerSm) k_lf_group(const __grid_constant__ DFrame f) {
   if (blockIdx.x < f.lf_cta_offset) return;
   LfGroupBody<kNarrow>(f, int(blockIdx.x - f.lf_cta_offset));
 }
 // Several images per launch (DFrameSet): the image is found from the CTA index.
 template <bool kNarrow>
-__global__ void __launch_bounds__(32) k_lf_group_multi(const __grid_constant__ DFrameSet s) {
+__global__ void __launch_bounds__(32, kLfMinCtasPerSm) k_lf_group_multi(const __grid_constant__ DFrameSet s) {
   if (blockIdx.x < s.cta_offset) return;
   const uint32_t cta = blockIdx.x - s.cta_offset; uint32_t img = 0; while (img + 1 < s.n && cta >= s.first[img + 1]) img++;
   LfGroupBody<kNarrow>(s.f[img], int(cta - s.first[img]));

@@ -61,7 +61,6 @@ DecodeResult DecodeOnGpu(const DecodeRequest& req);
 std::shared_ptr<DecodeJob> DecodeEnqueue(const DecodeRequest& req, cudaStream_t stream, bool lf_phase_only, bool defer_entropy);
 void DecodeBundleLaunch(const std::vector<std::shared_ptr<DecodeJob>>& jobs, int phase);   // phase 1: pending LF launches, 2: pending AC launches (jobs share one stream)
 void DecodeEnqueuePhase(const std::shared_ptr<DecodeJob>& job, int phase);   // phase 2: AC entropy kernels, 3: reconstruction + render; on failure the job's stream has drained
-void DumpPoolStats();
 void DecodeReservePools(const std::shared_ptr<DecodeJob>& job, size_t count);   // pre-populate the caching pools with `count` more sets of this job's buffers
 ParsedInfo DecodeBandLayout(const uint8_t* data, size_t size);
 DecodeResult DecodeFinish(const std::shared_ptr<DecodeJob>& job);
@@ -73,11 +72,14 @@ bool DecodeDebugCoeffs(const std::shared_ptr<DecodeJob>& job, std::vector<int16_
 
 bool CudaAvailable(std::string* why);
 void TrimPools();
-void DumpHostTrace();
-void* PinnedGet(size_t bytes);            // cached page-locked host memory (cudaHostAlloc costs far more than a decode)
-void PinnedPut(void* p, size_t bytes);
-void* DeviceGet(size_t bytes, void** pool_token);   // cached device memory of the current device (the encoder allocates ~25 buffers per call)
-void DevicePut(void* p, size_t bytes, void* pool_token);
+
+// A buffer from the engine's caching pools: device memory of the device current at Alloc, or page-locked host memory with pinned = true
+// (cudaMalloc / cudaHostAlloc cost more than a decode or most encoder kernels; cudaFree also synchronises). It goes back to the pool it
+// came from, and only after the work that uses it has been synchronised (the jobs and sessions sync their stream before they let go).
+class Pool;
+struct Buf { void* p = nullptr; size_t n = 0; Pool* pool = nullptr; void Alloc(size_t bytes, bool pinned = false); void Free();   // Alloc throws std::bad_alloc when the pool cannot get the memory
+  void Swap(Buf& o) { std::swap(p, o.p); std::swap(n, o.n); std::swap(pool, o.pool); } template <class T> T* as() const { return static_cast<T*>(p); }
+  Buf() {} ~Buf() { Free(); } Buf(const Buf&) = delete; Buf& operator=(const Buf&) = delete; };
 
 // ---- encoder
 struct EncodeRequest {
@@ -91,11 +93,6 @@ struct EncodeRequest {
 };
 struct EncodeResult { std::vector<uint8_t> file; StageTimes times; };
 EncodeResult EncodeOnGpu(const EncodeRequest& req);
-
-// Device buffers come from the engine's caching pool (cudaMalloc / cudaFree cost more than most encoder kernels; cudaFree also synchronises).
-// A buffer goes back to the pool only after the work that uses it has been synchronised (the sessions sync their stream before they let go).
-struct Buf { void* p = nullptr; size_t n = 0; void* pool = nullptr; void Alloc(size_t b) { Free(); n = b ? b : 1; p = DeviceGet(n, &pool); } void Free() { if (p) DevicePut(p, n, pool); p = nullptr; } ~Buf() { Free(); }
-  Buf() {} Buf(const Buf&) = delete; Buf& operator=(const Buf&) = delete; template <class T> T* as() const { return static_cast<T*>(p); } };
 
 // Everything that depends on the frame only (size, options, pixel format), never on pixels.
 struct EncPlan {
