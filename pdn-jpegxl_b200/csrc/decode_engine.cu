@@ -216,7 +216,7 @@ class DecodeJob {
   std::function<void()> ac_budget; int ac_lanes = 1; bool phased = false; size_t coeffs_bytes = 0, xyb_row_shift = 0;
   bool defer_entropy = false, lf_pending = false, ac_pending = false;   // bundle mode: the LF / AC entropy launch is left to DecodeBundleLaunch*
   cudaStream_t stream = nullptr; cudaEvent_t ev[8] = {nullptr}; bool timed = false; size_t out_bytes = 0; size_t comp_size = 0; const uint8_t* frame_ptr = nullptr; size_t frame_off = 0;
-  bool has_tree = false; Tree tree; Code tree_code; GroupHeader gheader; size_t global_decoded = 0; uint64_t global_data_bitpos = 0; bool global_has_data = false;
+  bool has_tree = false; Tree tree; Code tree_code; uint64_t global_data_bitpos = 0; bool global_has_data = false;
   std::vector<Code> ac_codes; uint32_t hf_blob_mark = 0; uint32_t frame_uploads = 0; uint8_t* ext_out_device = nullptr; uint8_t* ext_out_pinned = nullptr;
   ~DecodeJob() { for (auto& e : ev) if (e) cudaEventDestroy(e); }
 
@@ -251,6 +251,85 @@ DLocalTree DecodeJob::ParseLocalTree(BitReader& br, size_t pixels) {
   return lt;
 }
 
+// The global Modular image: its channels as coded (the forward side of every transform its header lists, SURVEY.md A.7; libjxl's MetaApply)
+// and the inverse transforms as device ops.
+struct ModPlan {
+  std::vector<DModChannel> coded, out;   // the channels as coded / the image's own channels after the inverse transforms, each with its plane
+  std::vector<DModOp> ops;               // the inverse transforms in the order the kernels run them: last transform first
+  size_t global_channels = 0;            // coded channels [0, global_channels) are held by the global section
+  bool has_lf_level = false;             // some later channel is coded in the LF-group sections
+  uint64_t total_ints = 0;               // int32 samples of all planes: coded channels + the outputs of the ops
+};
+// The walk keeps channel identities (indices into `geo`), not positions. An RCT works in place on three of them; a palette consumes
+// begin..end and creates an index and a palette channel; a squeeze step creates an average and a residual channel for each channel it
+// consumes. Every op outputs the channels its transform consumed, so each channel is either coded or made by exactly one op.
+static ModPlan PlanModularImage(const ImageMetadata& m, const FrameHeader& fh, const GroupHeader& gh) {
+  std::vector<DModChannel> geo;   // every channel the forward transforms pass through; the image's own channels first
+  if (fh.encoding == 1) { JXLG_CHECK(!m.xyb_encoded, "XYB-encoded Modular frames are not supported"); int nc = m.ce.color_space == kCsGray ? 1 : 3; for (int c = 0; c < nc; c++) geo.push_back(DModChannel{fh.xsize, fh.ysize, 0, 0, 0}); }
+  for (size_t i = 0; i < m.ec.size(); i++) { JXLG_CHECK(fh.ec_upsampling[i] == 1, "upsampling is not supported"); uint32_t s = m.ec[i].dim_shift; geo.push_back(DModChannel{DivCeil(fh.xsize, 1u << s), DivCeil(fh.ysize, 1u << s), s, s, 0}); }
+  JXLG_CHECK(geo.size() <= 8, "too many Modular channels"); const size_t num_image_channels = geo.size();
+  std::vector<uint32_t> ch(num_image_channels); for (size_t i = 0; i < ch.size(); i++) ch[i] = uint32_t(i);   // the channel list
+  auto add = [&](DModChannel c) { geo.push_back(c); return uint32_t(geo.size() - 1); };
+  ModPlan plan; std::vector<DModOp>& ops = plan.ops;
+  // an op goes in front of the ops of earlier transforms; `at` keeps the channels of one squeeze step in order
+  auto new_op = [&](uint32_t kind, size_t at) -> DModOp& { JXLG_CHECK(ops.size() < 1024, "too many Modular transform steps"); DModOp& o = *ops.insert(ops.begin() + at, DModOp()); o.kind = kind; return o; };
+  int nb_meta = 0;
+  for (const Transform& t : gh.transforms) {
+    if (t.id == 0) {
+      JXLG_CHECK(t.begin_c + 3 <= ch.size(), "RCT channel range"); const DModChannel a = geo[ch[t.begin_c]];
+      for (int k = 1; k < 3; k++) JXLG_CHECK(geo[ch[t.begin_c + k]].w == a.w && geo[ch[t.begin_c + k]].h == a.h, "RCT channel sizes");
+      DModOp& op = new_op(0, 0); op.rct_type = t.rct_type; op.w = a.w; op.h = a.h; for (int k = 0; k < 3; k++) op.p[k] = ch[t.begin_c + k];
+      continue;
+    }
+    if (t.id == 1) {
+      const uint32_t end_c = t.begin_c + t.num_c - 1; JXLG_CHECK(t.num_c >= 1 && t.num_c <= 4 && end_c < ch.size(), "palette channel range"); const DModChannel first = geo[ch[t.begin_c]];
+      for (uint32_t c = t.begin_c + 1; c <= end_c; c++) { const DModChannel& o = geo[ch[c]]; JXLG_CHECK(o.w == first.w && o.h == first.h && o.hshift == first.hshift && o.vshift == first.vshift, "palette channel sizes"); }
+      if (int(t.begin_c) < nb_meta) { JXLG_CHECK(int(end_c) < nb_meta, "palette across the meta-channel boundary"); nb_meta += 2 - int(t.num_c); } else nb_meta += 1;
+      JXLG_CHECK(t.nb_deltas == 0 || t.predictor != 6, "delta palettes with the weighted predictor are not supported");
+      DModOp& op = new_op(1, 0); op.num_c = t.num_c; op.pal_w = t.nb_colors + t.nb_deltas; op.nb_deltas = t.nb_deltas; op.predictor = t.predictor; op.w = first.w; op.h = first.h;
+      for (uint32_t k = 0; k < t.num_c; k++) op.out[k] = ch[t.begin_c + k];
+      op.p[0] = add(first); op.p[1] = add(DModChannel{op.pal_w, t.num_c, 0, 0, 0});   // the palette itself: one row per colour channel, always coded in the global section
+      ch.erase(ch.begin() + t.begin_c + 1, ch.begin() + end_c + 1); ch[t.begin_c] = uint32_t(op.p[0]); ch.insert(ch.begin(), uint32_t(op.p[1]));
+      continue;
+    }
+    // Squeeze: every step halves its channels (average, shift + 1) and appends / inserts the residual channels
+    std::vector<SqueezeParams> steps = t.squeezes;
+    if (steps.empty()) {   // default parameters (libjxl's DefaultSqueezeParameters): chroma first when the first two channels match, then alternate until <= 8 x 8
+      const int nb = int(ch.size()) - nb_meta; JXLG_CHECK(nb > 0, "squeeze without channels"); uint32_t w = geo[ch[nb_meta]].w, hh = geo[ch[nb_meta]].h;
+      if (nb > 2 && geo[ch[nb_meta + 1]].w == w && geo[ch[nb_meta + 1]].h == hh) { SqueezeParams p; p.horizontal = true; p.in_place = false; p.begin_c = uint32_t(nb_meta + 1); p.num_c = 2; steps.push_back(p); p.horizontal = false; steps.push_back(p); }
+      SqueezeParams p; p.begin_c = uint32_t(nb_meta); p.num_c = uint32_t(nb); p.in_place = true;
+      if (!(w > hh)) { if (hh > 8) { p.horizontal = false; steps.push_back(p); hh = (hh + 1) / 2; } }
+      while (w > 8 || hh > 8) { if (w > 8) { p.horizontal = true; steps.push_back(p); w = (w + 1) / 2; } if (hh > 8) { p.horizontal = false; steps.push_back(p); hh = (hh + 1) / 2; } }
+    }
+    for (const SqueezeParams& sq : steps) {
+      const uint32_t end_c = sq.begin_c + sq.num_c - 1; JXLG_CHECK(sq.num_c >= 1 && end_c < ch.size(), "squeeze channel range"); JXLG_CHECK(int(sq.begin_c) >= nb_meta, "squeeze of meta channels is not supported");
+      const size_t offset = sq.in_place ? size_t(end_c) + 1 : ch.size();
+      for (uint32_t c = sq.begin_c; c <= end_c; c++) {
+        const DModChannel in = geo[ch[c]]; DModChannel a = in, r;
+        if (sq.horizontal) { a.w = (in.w + 1) / 2; a.hshift++; r = DModChannel{in.w - a.w, a.h, a.hshift, a.vshift, 0}; }
+        else { a.h = (in.h + 1) / 2; a.vshift++; r = DModChannel{a.w, in.h - a.h, a.hshift, a.vshift, 0}; }
+        JXLG_CHECK(a.hshift < 30 && a.vshift < 30, "squeeze depth");
+        DModOp& op = new_op(2, c - sq.begin_c); op.rct_type = sq.horizontal ? 1 : 0; op.w = a.w; op.h = a.h; op.num_c = r.w; op.pal_w = r.h; op.out[0] = ch[c];
+        op.p[0] = ch[c] = add(a); op.p[1] = add(r); ch.insert(ch.begin() + offset + (c - sq.begin_c), uint32_t(op.p[1]));
+      }
+    }
+  }
+  JXLG_CHECK(ch.size() <= 255, "too many Modular channels");
+  // planes: the coded channels in coded order, then the outputs of the ops in the order they run; p[] and out[] turn from channels into planes
+  uint64_t off = 0; for (uint32_t id : ch) { DModChannel& c = geo[id]; c.plane_off = off; off += uint64_t(c.w) * c.h; plan.coded.push_back(c); }
+  for (DModOp& op : ops) {
+    const uint32_t nout = op.kind == 0 ? 0 : op.kind == 1 ? op.num_c : 1;
+    for (uint32_t k = 0; k < nout; k++) { DModChannel& c = geo[op.out[k]]; c.plane_off = off; off += uint64_t(c.w) * c.h; op.out[k] = c.plane_off; }
+    for (int k = 0; k < (op.kind == 0 ? 3 : 2); k++) op.p[k] = geo[op.p[k]].plane_off;
+  }
+  plan.out.assign(geo.begin(), geo.begin() + num_image_channels); plan.total_ints = off;
+  // which channels the global section holds: meta channels always, then every channel up to the first one larger than a group
+  const std::vector<DModChannel>& cc = plan.coded; size_t c = 0; for (; c < cc.size(); c++) if (int(c) >= nb_meta && (cc[c].w > fh.group_dim || cc[c].h > fh.group_dim)) break;
+  plan.global_channels = c;
+  for (size_t i = c; i < cc.size(); i++) if (std::min(cc[i].hshift, cc[i].vshift) >= 3 && cc[i].w && cc[i].h) plan.has_lf_level = true;   // coded in the LF-group sections
+  return plan;
+}
+
 void DecodeJob::ParseLfGlobal(BitReader& br) {
   const ImageMetadata& m = hd.meta;
   JXLG_CHECK(!(fh.flags & (kFlagPatches | kFlagSplines | kFlagNoise)), "patches/splines/noise are not supported");
@@ -282,102 +361,26 @@ void DecodeJob::ParseLfGlobal(BitReader& br) {
     uint32_t uses_wp = 0; h.tree_off = AddTree(tree, &uses_wp); h.tree_size = uint32_t(tree.size()); h.uses_wp = uses_wp; h.mod_code = blob.AddCode(tree_code);
   }
   h.has_tree = has_tree;
-  // global Modular image: colour channels (Modular frames) + extra channels
-  std::vector<DModChannel> ch;
-  if (fh.encoding == 1) { JXLG_CHECK(!m.xyb_encoded, "XYB-encoded Modular frames are not supported"); int nc = m.ce.color_space == kCsGray ? 1 : 3; for (int c = 0; c < nc; c++) ch.push_back(DModChannel{fh.xsize, fh.ysize, 0, 0, 0}); }
-  for (size_t i = 0; i < m.ec.size(); i++) { JXLG_CHECK(fh.ec_upsampling[i] == 1, "upsampling is not supported"); uint32_t s = m.ec[i].dim_shift; ch.push_back(DModChannel{DivCeil(fh.xsize, 1u << s), DivCeil(fh.ysize, 1u << s), s, s, 0}); }
-  JXLG_CHECK(ch.size() <= 8, "too many Modular channels"); h.num_mod_channels = uint32_t(ch.size()); h.num_ops = 0; h.first_group_channel = 0; global_has_data = false; mod_total_ints = 0;
   h.mod_bitdepth = m.bd.bits; { uint32_t mb = m.bd.bits; for (const auto& e : m.ec) mb = std::max(mb, e.bd.bits); h.mod_wide = (mb > 20 || !m.modular_16bit) ? 1 : 0; }
-  const size_t num_image_channels = ch.size();
-  int nb_meta = 0;
-  if (!ch.empty()) {
-    gheader = ReadGroupHeader(br);
-    // ---- the channel list as coded: the forward side of every transform (SURVEY.md A.7; libjxl's MetaApply)
-    for (Transform& t : gheader.transforms) {
-      if (t.id == 0) { JXLG_CHECK(t.begin_c + 3 <= ch.size(), "RCT channel range"); continue; }
-      if (t.id == 1) {
-        const uint32_t end_c = t.begin_c + t.num_c - 1; JXLG_CHECK(t.num_c >= 1 && t.num_c <= 4 && end_c < ch.size(), "palette channel range");
-        for (uint32_t c = t.begin_c + 1; c <= end_c; c++) JXLG_CHECK(ch[c].w == ch[t.begin_c].w && ch[c].h == ch[t.begin_c].h && ch[c].hshift == ch[t.begin_c].hshift && ch[c].vshift == ch[t.begin_c].vshift, "palette channel sizes");
-        if (int(t.begin_c) < nb_meta) { JXLG_CHECK(int(end_c) < nb_meta, "palette across the meta-channel boundary"); nb_meta += 2 - int(t.num_c); } else nb_meta += 1;
-        ch.erase(ch.begin() + t.begin_c + 1, ch.begin() + end_c + 1);
-        ch.insert(ch.begin(), DModChannel{t.nb_colors + t.nb_deltas, t.num_c, 0, 0, 0});   // the palette itself: one row per colour channel, always coded in the global section
-        continue;
-      }
-      // Squeeze: every step halves its channels (average, shift + 1) and appends / inserts the residual channels
-      if (t.squeezes.empty()) {   // default parameters (libjxl's DefaultSqueezeParameters): chroma first when the first two channels match, then alternate until <= 8 x 8
-        const int nb = int(ch.size()) - nb_meta; JXLG_CHECK(nb > 0, "squeeze without channels"); uint32_t w = ch[nb_meta].w, hh = ch[nb_meta].h;
-        if (nb > 2 && ch[nb_meta + 1].w == w && ch[nb_meta + 1].h == hh) { SqueezeParams p; p.horizontal = true; p.in_place = false; p.begin_c = uint32_t(nb_meta + 1); p.num_c = 2; t.squeezes.push_back(p); p.horizontal = false; t.squeezes.push_back(p); }
-        SqueezeParams p; p.begin_c = uint32_t(nb_meta); p.num_c = uint32_t(nb); p.in_place = true;
-        if (!(w > hh)) { if (hh > 8) { p.horizontal = false; t.squeezes.push_back(p); hh = (hh + 1) / 2; } }
-        while (w > 8 || hh > 8) { if (w > 8) { p.horizontal = true; t.squeezes.push_back(p); w = (w + 1) / 2; } if (hh > 8) { p.horizontal = false; t.squeezes.push_back(p); hh = (hh + 1) / 2; } }
-      }
-      for (const SqueezeParams& sq : t.squeezes) {
-        const uint32_t end_c = sq.begin_c + sq.num_c - 1; JXLG_CHECK(sq.num_c >= 1 && end_c < ch.size(), "squeeze channel range"); JXLG_CHECK(int(sq.begin_c) >= nb_meta, "squeeze of meta channels is not supported");
-        const size_t offset = sq.in_place ? size_t(end_c) + 1 : ch.size();
-        for (uint32_t c = sq.begin_c; c <= end_c; c++) {
-          DModChannel a = ch[c], r = a;
-          if (sq.horizontal) { a.w = (ch[c].w + 1) / 2; a.hshift++; r = DModChannel{ch[c].w - a.w, a.h, a.hshift, a.vshift, 0}; }
-          else { a.h = (ch[c].h + 1) / 2; a.vshift++; r = DModChannel{a.w, ch[c].h - a.h, a.hshift, a.vshift, 0}; }
-          JXLG_CHECK(a.hshift < 30 && a.vshift < 30, "squeeze depth"); ch[c] = a; ch.insert(ch.begin() + offset + (c - sq.begin_c), r);
-        }
-      }
-    }
-    JXLG_CHECK(ch.size() <= 255, "too many Modular channels"); h.num_mod_channels = uint32_t(ch.size());
-  }
-  uint64_t off = 0; for (auto& c : ch) { c.plane_off = off; off += uint64_t(c.w) * c.h; }
+  // global Modular image: colour channels (Modular frames) + extra channels
+  GroupHeader gheader; ModPlan plan;
+  if (fh.encoding == 1 || !m.ec.empty()) { gheader = ReadGroupHeader(br); plan = PlanModularImage(m, fh, gheader); }
+  const std::vector<DModChannel>& ch = plan.coded; const size_t nglobal = plan.global_channels;
+  h.num_mod_channels = uint32_t(ch.size()); h.first_group_channel = uint32_t(nglobal); mod_has_lf_level = plan.has_lf_level; mod_total_ints = plan.total_ints; global_has_data = false;
   h.mod_ch_off = 0; if (ch.size() <= 8) { for (size_t i = 0; i < ch.size(); i++) h.mod_ch[i] = ch[i]; } else h.mod_ch_off = blob.Add(ch.data(), ch.size() * sizeof(DModChannel));
-  mod_has_lf_level = false; ops_host.clear(); h.ops_off = 0;
+  for (size_t i = 0; i < plan.out.size(); i++) h.out_ch[i] = plan.out[i];
   if (!ch.empty()) {
-    // ---- which of them the global section holds: meta channels always, then every channel up to the first one larger than a group
-    size_t c = 0; for (; c < ch.size(); c++) if (int(c) >= nb_meta && (ch[c].w > fh.group_dim || ch[c].h > fh.group_dim)) break;
-    global_decoded = c; h.first_group_channel = uint32_t(c);
-    for (size_t i = c; i < ch.size(); i++) if (std::min(ch[i].hshift, ch[i].vshift) >= 3 && ch[i].w && ch[i].h) mod_has_lf_level = true;   // coded in the LF-group sections
-    size_t nonempty = 0; for (size_t i = 0; i < c; i++) if (ch[i].w && ch[i].h) nonempty++;
+    size_t nonempty = 0; for (size_t i = 0; i < nglobal; i++) if (ch[i].w && ch[i].h) nonempty++;
     if (nonempty) {
       global_has_data = true;
-      if (!gheader.use_global_tree) { size_t px = 0; for (size_t i = 0; i < c; i++) px += size_t(ch[i].w) * ch[i].h; global_local = ParseLocalTree(br, px); }   // data starts where this parse stops
+      if (!gheader.use_global_tree) { size_t px = 0; for (size_t i = 0; i < nglobal; i++) px += size_t(ch[i].w) * ch[i].h; global_local = ParseLocalTree(br, px); }   // data starts where this parse stops
       else JXLG_CHECK(has_tree, "the global Modular stream uses the global MA tree, but the frame has none");
     }
     const WPHeader& gw = gheader.wp; h.global_wp.p1 = gw.p1; h.global_wp.p2 = gw.p2; h.global_wp.p3a = gw.p3a; h.global_wp.p3b = gw.p3b; h.global_wp.p3c = gw.p3c; h.global_wp.p3d = gw.p3d; h.global_wp.p3e = gw.p3e;
     for (int i = 0; i < 4; i++) h.global_wp.w[i] = gw.w[i];
-    // ---- the inverse transforms as device ops, last transform first; `cur` follows the channel list back to the image's own channels
-    std::vector<DModChannel> cur = ch;
-    auto new_op = [&]() -> DModOp& { JXLG_CHECK(ops_host.size() < 1024, "too many Modular transform steps"); ops_host.emplace_back(); memset(&ops_host.back(), 0, sizeof(DModOp)); return ops_host.back(); };
-    for (size_t ti = gheader.transforms.size(); ti-- > 0;) {
-      const Transform& t = gheader.transforms[ti];
-      if (t.id == 0) {
-        JXLG_CHECK(t.begin_c + 3 <= cur.size(), "RCT channel range"); const DModChannel& a = cur[t.begin_c];
-        for (int k = 1; k < 3; k++) JXLG_CHECK(cur[t.begin_c + k].w == a.w && cur[t.begin_c + k].h == a.h, "RCT channel sizes");
-        DModOp& op = new_op(); op.kind = 0; op.rct_type = t.rct_type; op.w = a.w; op.h = a.h; for (int k = 0; k < 3; k++) op.p[k] = cur[t.begin_c + k].plane_off;
-      } else if (t.id == 1) {
-        JXLG_CHECK(t.begin_c + 1 < cur.size(), "palette channel range"); const DModChannel pal = cur[0], idx = cur[t.begin_c + 1];
-        JXLG_CHECK(pal.h == t.num_c && pal.w == t.nb_colors + t.nb_deltas, "palette geometry"); JXLG_CHECK(t.nb_deltas == 0 || t.predictor != 6, "delta palettes with the weighted predictor are not supported");
-        DModOp& op = new_op(); op.kind = 1; op.num_c = t.num_c; op.pal_w = pal.w; op.nb_deltas = t.nb_deltas; op.predictor = t.predictor; op.w = idx.w; op.h = idx.h; op.p[0] = idx.plane_off; op.p[1] = pal.plane_off;
-        cur.erase(cur.begin()); std::vector<DModChannel> outs;
-        for (uint32_t k = 0; k < t.num_c; k++) { DModChannel o = idx; o.plane_off = off; off += uint64_t(idx.w) * idx.h; op.out[k] = o.plane_off; outs.push_back(o); }
-        cur.erase(cur.begin() + t.begin_c); cur.insert(cur.begin() + t.begin_c, outs.begin(), outs.end());
-      } else {
-        for (size_t si = t.squeezes.size(); si-- > 0;) {   // steps in reverse; each channel's (average, residual) pair interleaves into a new plane
-          const SqueezeParams& sq = t.squeezes[si]; const uint32_t end_c = sq.begin_c + sq.num_c - 1;
-          JXLG_CHECK(cur.size() >= sq.num_c && size_t(end_c) < cur.size(), "squeeze channel range"); const size_t offset = sq.in_place ? size_t(end_c) + 1 : cur.size() - sq.num_c; JXLG_CHECK(offset + sq.num_c <= cur.size() && offset > end_c, "squeeze channel range");
-          for (uint32_t c = sq.begin_c; c <= end_c; c++) {
-            const DModChannel avg = cur[c], res = cur[offset + (c - sq.begin_c)]; DModChannel o = avg;
-            if (sq.horizontal) { JXLG_CHECK(res.h == avg.h && (res.w == avg.w || res.w + 1 == avg.w) && avg.hshift > 0, "squeeze geometry"); o.w = avg.w + res.w; o.hshift = avg.hshift - 1; }
-            else { JXLG_CHECK(res.w == avg.w && (res.h == avg.h || res.h + 1 == avg.h) && avg.vshift > 0, "squeeze geometry"); o.h = avg.h + res.h; o.vshift = avg.vshift - 1; }
-            o.plane_off = off; off += uint64_t(o.w) * o.h;
-            DModOp& op = new_op(); op.kind = 2; op.rct_type = sq.horizontal ? 1 : 0; op.w = avg.w; op.h = avg.h; op.num_c = res.w; op.pal_w = res.h; op.p[0] = avg.plane_off; op.p[1] = res.plane_off; op.out[0] = o.plane_off;
-            cur[c] = o;
-          }
-          cur.erase(cur.begin() + offset, cur.begin() + offset + sq.num_c);
-        }
-      }
-    }
-    JXLG_CHECK(cur.size() == num_image_channels, "Modular transforms do not restore the channel list");
-    for (size_t i = 0; i < cur.size(); i++) h.out_ch[i] = cur[i];
-    h.num_ops = uint32_t(ops_host.size());
-    if (ops_host.size() <= 4) { for (size_t i = 0; i < ops_host.size(); i++) h.ops[i] = ops_host[i]; } else h.ops_off = blob.Add(ops_host.data(), ops_host.size() * sizeof(DModOp));
   }
-  mod_total_ints = off;
+  ops_host = plan.ops; h.num_ops = uint32_t(ops_host.size()); h.ops_off = 0;
+  if (ops_host.size() <= 4) { for (size_t i = 0; i < ops_host.size(); i++) h.ops[i] = ops_host[i]; } else h.ops_off = blob.Add(ops_host.data(), ops_host.size() * sizeof(DModOp));
 }
 
 void DecodeJob::ParseHfGlobal(BitReader& br) {
@@ -536,24 +539,18 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
   h.local_off = 0;
   { std::vector<DLocalTree> lts(size_t(h.num_groups) + 1 + h.num_lf_groups); memset(lts.data(), 0, lts.size() * sizeof(DLocalTree)); bool any = false;   // [group g | global | LF group g]
     if (global_local.present) { lts[h.num_groups] = global_local; lts[h.num_groups].data_bitpos = after_lfglobal; any = true; }
-    if (fh.encoding == 1 && !single && h.num_passes == 1 && h.num_mod_channels > h.first_group_channel) {
-      for (uint32_t g = 0; g < h.num_groups; g++) {
-        const size_t t = size_t(2) + h.num_lf_groups + g; if (toc.size[t] == 0) continue;
-        BitReader gb(cs.data() + frame_off + toc.offset[t], toc.size[t]); const GroupHeader gh = ReadGroupHeader(gb);
-        bool only_rct = true; for (const Transform& tr : gh.transforms) only_rct = only_rct && tr.id == 0;
-        if (gb.overrun || gh.use_global_tree || !only_rct) continue;   // (palette / squeeze inside a group section: the kernel reports them)
-        lts[g] = ParseLocalTree(gb, size_t(h.group_dim) * h.group_dim * (h.num_mod_channels - h.first_group_channel)); lts[g].data_bitpos = base_bits + uint64_t(toc.offset[t]) * 8 + gb.pos; any = true;
-      }
-    }
-    if (fh.encoding == 1 && !single && mod_has_lf_level) {   // LF-group sections of Modular frames (channels of shift >= 3) start with their Modular header too
-      for (uint32_t g = 0; g < h.num_lf_groups; g++) {
-        const size_t t = size_t(1) + g; if (toc.size[t] == 0) continue;
-        BitReader gb(cs.data() + frame_off + toc.offset[t], toc.size[t]); const GroupHeader gh = ReadGroupHeader(gb);
-        bool only_rct = true; for (const Transform& tr : gh.transforms) only_rct = only_rct && tr.id == 0;
-        if (gb.overrun || gh.use_global_tree || !only_rct) continue;
-        const size_t dim = size_t(h.group_dim); DLocalTree& e = lts[size_t(h.num_groups) + 1 + g]; e = ParseLocalTree(gb, dim * dim * h.num_mod_channels); e.data_bitpos = base_bits + uint64_t(toc.offset[t]) * 8 + gb.pos; any = true;
-      }
-    }
+    auto section_tree = [&](size_t t, size_t slot, size_t pixels) {   // TOC section t, entry lts[slot], at most `pixels` samples
+      if (toc.size[t] == 0) return;
+      BitReader gb(cs.data() + frame_off + toc.offset[t], toc.size[t]); const GroupHeader gh = ReadGroupHeader(gb);
+      bool only_rct = true; for (const Transform& tr : gh.transforms) only_rct = only_rct && tr.id == 0;
+      if (gb.overrun || gh.use_global_tree || !only_rct) return;   // (palette / squeeze inside a section: the kernel reports them)
+      lts[slot] = ParseLocalTree(gb, pixels); lts[slot].data_bitpos = base_bits + uint64_t(toc.offset[t]) * 8 + gb.pos; any = true;
+    };
+    const size_t dim = size_t(h.group_dim);
+    if (fh.encoding == 1 && !single && h.num_passes == 1 && h.num_mod_channels > h.first_group_channel)
+      for (uint32_t g = 0; g < h.num_groups; g++) section_tree(size_t(2) + h.num_lf_groups + g, g, dim * dim * (h.num_mod_channels - h.first_group_channel));
+    if (fh.encoding == 1 && !single && mod_has_lf_level)   // LF-group sections of Modular frames (channels of shift >= 3) start with their Modular header too
+      for (uint32_t g = 0; g < h.num_lf_groups; g++) section_tree(size_t(1) + g, size_t(h.num_groups) + 1 + g, dim * dim * h.num_mod_channels);
     if (any) h.local_off = blob.Add(lts.data(), lts.size() * sizeof(DLocalTree)); }
   std::vector<uint64_t> sec(2 * nlog + 2, 0);
   for (size_t i = 0; i < nlog; i++) { size_t t = single ? 0 : i; sec[i] = base_bits + uint64_t(toc.offset[t]) * 8; sec[nlog + i] = base_bits + uint64_t(toc.offset[t] + toc.size[t]) * 8; }
@@ -564,7 +561,7 @@ void DecodeJob::RunLf(const DecodeRequest& req) {
   const DFrame* d = d_frame.as<DFrame>();
   if (timed) cudaEventRecord(ev[0], stream);
   // global Modular stream
-  if (global_has_data) LaunchModularGlobal(d, h, after_lfglobal, uint32_t(global_decoded), stream);
+  if (global_has_data) LaunchModularGlobal(d, h, after_lfglobal, h.first_group_channel, stream);
   else if (single) { uint64_t* slot = reinterpret_cast<uint64_t*>(h_misc.as<uint8_t>() + 2 * sizeof(DFrame)); slot[0] = after_lfglobal; CUDA_OK(cudaMemcpyAsync(h.end_bitpos, slot, 8, cudaMemcpyHostToDevice, stream)); }
   if (!vardct && !single && mod_has_lf_level) LaunchModLfGroups(h, stream);   // Modular frames: channels of shift >= 3 live in the LF-group sections
   if (vardct) { if (defer_entropy && !single) lf_pending = true; else LaunchLfGroups(d, h, stream); }

@@ -4,6 +4,7 @@ computed from the published XYB constants. The same files are checked against th
 import numpy as np
 import pytest
 
+import jxl_spec_writer as W
 import spec_cases
 from test_spec_writer_cpu import expected_pixels
 
@@ -42,3 +43,24 @@ def test_dc_only_vardct_frame_matches_published_constants(gpu):
     gpu.JpegXLNative.LoadImage(data, image)
     err = np.abs(image.layer_data.interleaved.astype(np.float64) - want).max()
     assert err <= 0.5 + 1e-2, "DC-only VarDCT frame: max |decoded - expected| = %g" % err
+
+
+def _refused(gpu, data, message):
+    with pytest.raises(gpu.FormatException, match=message) as e:
+        gpu.JpegXLNative.LoadImage(data, gpu.DecoderImage())
+    assert e.value.status == "DecodeError"
+
+
+def test_rct_over_channels_of_different_sizes_is_refused(gpu):
+    # R, G, B and an extra channel at half resolution (dim_shift 1); the RCT on channels 1..3 takes B and the extra channel together.
+    # The header is refused before any sample is read, so the extra channel's plane is written at full size.
+    a = spec_cases._img(16, 24, 4, seed=41)
+    data = W.modular_image(spec_cases._planes(a), extra=[dict(type=W.EC_DEPTH, bits=8, dim_shift=1)], rct=(1, 6))
+    _refused(gpu, data, "RCT channel sizes")
+
+
+def test_delta_palette_with_the_weighted_predictor_is_refused(gpu):
+    colors = [(10, 20, 30), (200, 100, 50), (90, 90, 90)]
+    a = np.array(colors)[np.random.default_rng(42).integers(0, 3, size=(16, 24))]
+    data = W.modular_image(spec_cases._planes(a), palette=dict(begin=0, num_c=3, colors=colors, deltas=[(1, 2, 3)], predictor=6))
+    _refused(gpu, data, "delta palettes with the weighted predictor are not supported")
